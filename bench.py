@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- aggregate input MS/s of the SDRReceiver channelizer hot path (25E plan).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = `--blocks` callbacks (default 4 = one second of signal) for each of `--streams`
@@ -15,6 +15,13 @@ ONE JSON line:
             CUDA-event time vs the measured HBM copy peak (MEASURED_PEAKS.json)
   cpu_baseline  the unmodified reference (oracle/_ref) on this box's host cores, bounded sample
 `--impl reference` times the reference's own CPU code instead (same metric/config).
+Every timed loop (kernel leg, end to end, publish leg -- once with n sockets, once with one -- and each of the other
+plans, the kernel legs followed by a second pass with per-launch timing) runs `--steps` steps after `--warmup`, so the
+wall time of a run grows with --steps in every leg.
+`--dump-outputs DIR` writes what the kernel leg's last step computed (rank 0) as DIR/*.npy: the seeded inputs are
+identical from run to run, so two builds can be compared output for output. The bank carries state from step to step
+and the dumped step is the last of the per-launch timing pass (step warmup + 2*steps), so two dumps are comparable when
+--steps, --warmup, --plan, --streams and --blocks agree.
 """
 import argparse
 import ctypes as C
@@ -48,6 +55,9 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-zmq", action="store_true", help="skip the publish-inclusive end-to-end leg")
     ap.add_argument("--no-plans", action="store_true", help="skip the short runs of the other BASELINE configurations")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the kernel leg's last-step int16 records as float32 .npy files; two dumps compare only "
+                         "at equal --steps/--warmup/--plan/--streams/--blocks (the bank carries state across steps)")
     return ap.parse_args()
 
 
@@ -299,6 +309,25 @@ def class_rooflines(plan, per_step_ms, samples_per_step, hbm_peak_gbs, fp32_peak
     return out
 
 
+DUMP_BYTES = 60 << 20        # what --dump-outputs writes at most (float32)
+
+
+def dump_outputs(out_dir, pcm):
+    """pcm [S, NB, pcm_per_block] int16 -- the records a caller of the kernel leg receives for every receiver -- as float32.
+    Receivers beyond the DUMP_BYTES budget are left out: a fixed, seeded choice that always keeps receiver 0 (the canary).
+    pcm.npy is [k, NB, pcm_per_block], pcm_streams.npy the k receiver indices it holds. When one receiver alone is over the
+    budget, k is 1 and pcm.npy is 1-D: the first DUMP_BYTES / 4 samples of receiver 0's records, in memory order."""
+    S = pcm.shape[0]
+    k = max(1, min(S, DUMP_BYTES // (pcm[0].size * 4)))
+    pick = np.sort(np.concatenate([[0], np.random.default_rng(20261020).permutation(np.arange(1, S))[:k - 1]]))
+    sel = pcm[pick]
+    if sel.size * 4 > DUMP_BYTES:          # one receiver alone is over the budget: its first samples
+        sel = sel.reshape(-1)[:DUMP_BYTES // 4]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pcm.npy"), sel.astype(np.float32))
+    np.save(os.path.join(out_dir, "pcm_streams.npy"), pick.astype(np.float64))
+
+
 def canary_check(B, plan, local_rank):
     """Parity verdict of this rank: a fresh one-receiver bank runs the canary's first callback and is compared with
     tests/golden/canary_25E_1block.npz (int16 of the unmodified reference, tools/make_golden.py): +-1 LSB."""
@@ -405,6 +434,8 @@ def b200_arm(args):
     # timings -- the canary digest of every rank, which must agree (identical bytes, identical history on every rank)
     lsb, lsb_what = canary_check(B, plan, local_rank)
     pcm_host = R.d_pcm.cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pcm_host)
     digest = shard.pcm_digest(pcm_host) + shard.pcm_digest(pcm_host[0]) + [-1 if lsb is None else int(lsb)]
     stats_all, digests = shard.gather([dev_ms, e2e_ms if e2e_ms is not None else 0.0, float(samples_per_step)],
                                       digest, device=dev)
@@ -498,7 +529,7 @@ def b200_arm(args):
         "kernel_launches_per_step": launches_per_step,
         "digests": digests,
     }
-    # ---- the other BASELINE.json configurations, short runs (5 steps): value and per-class times ----
+    # ---- the other BASELINE.json configurations, --steps steps each: value and per-class times ----
     if world == 1 and not args.no_plans:
         R.bank.close()
         del R
@@ -508,7 +539,8 @@ def b200_arm(args):
             if name == args.plan:
                 continue
             try:
-                extra[name] = extra_plan(B, torch, shard, name, S, NB, dev, local_rank, peak, fp32_peak, barrier)
+                extra[name] = extra_plan(B, torch, shard, name, S, NB, dev, local_rank, peak, fp32_peak, barrier,
+                                         args.steps, args.warmup)
             except Exception as ex:
                 extra[name] = {"error": str(ex)[:200]}
         line["plans"] = extra
@@ -529,8 +561,8 @@ def b200_arm(args):
 EXTRA_PLANS = ["54W_288K", "54W_all", "CBAND_143E"]
 
 
-def extra_plan(B, torch, shard, name, S, NB, dev, local_rank, peak, fp32_peak, barrier):
-    """Kernel-only leg of another BASELINE.json configuration: same bank size, 3 warm-up + 5 timed steps. CBAND_143E runs with
+def extra_plan(B, torch, shard, name, S, NB, dev, local_rank, peak, fp32_peak, barrier, steps, warmup):
+    """Kernel-only leg of another BASELINE.json configuration: same bank size, `warmup` + `steps` timed steps. CBAND_143E runs with
     the spectrum path fed as the reference's GUI would (fftHandlerSlot): "Main" on every 4th callback and one selected
     sub VFO on every callback, for every receiver of the bank."""
     plan = B.Plan(os.path.join(ROOT, "plans", name + ".ini"))
@@ -552,7 +584,7 @@ def extra_plan(B, torch, shard, name, S, NB, dev, local_rank, peak, fp32_peak, b
                 R.bank.spectrum_feed(spec_sub, 0, cb, None, st)    # vfo.cpp:290-293: the selected VFO, every callback
             ev[1].record(R.stream)
         R.after_step = feed
-    dev_ms, launches, per_step_ms, _ = R.timed(5, 3, barrier)
+    dev_ms, launches, per_step_ms, _ = R.timed(steps, warmup, barrier)
     if name.startswith("CBAND"):
         # the feeds of one step, timed on their own after the run
         torch.cuda.synchronize()
@@ -560,8 +592,8 @@ def extra_plan(B, torch, shard, name, S, NB, dev, local_rank, peak, fp32_peak, b
         torch.cuda.synchronize()
         spec_ms = ev[0].elapsed_time(ev[1])
         spec_main.close(); spec_sub.close()
-    step_ms = dev_ms / 5
-    out = {"value": R.samples_per_step / (step_ms * 1e-3) / 1e6, "unit": "MS/s", "ms_per_step": step_ms, "steps": 5, "warmup": 3,
+    step_ms = dev_ms / steps
+    out = {"value": R.samples_per_step / (step_ms * 1e-3) / 1e6, "unit": "MS/s", "ms_per_step": step_ms, "steps": steps, "warmup": warmup,
            "realtime_x": R.samples_per_step / (step_ms * 1e-3) / plan.fs, "kernels_ms_per_step": per_step_ms,
            "per_class": class_rooflines(plan, per_step_ms, R.samples_per_step, peak, fp32_peak), "gpu_launches": launches}
     if spec_ms is not None:
@@ -629,7 +661,7 @@ def publish_leg(B, plan, bank, host_bufs, row, S, NB, rank, args, n_sockets=8):
         for th in threads:
             th.start()
     time.sleep(0.3)
-    steps = max(2, min(args.steps, 10))
+    steps = args.steps
     sent = 0
     step_no = [0]
 

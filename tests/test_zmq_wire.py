@@ -3,6 +3,9 @@ put on the wire exactly what ZmqPublisher::publish does (zmqpublisher.cpp:82-96)
 [topic, 5 bytes][uint32 LE rate][int16 LE PCM], nothing for an empty payload. A pyzmq SUB
 socket plays JAERO. Host-only: no GPU needed."""
 import ctypes as C
+import pathlib
+import shutil
+import tempfile
 import time
 
 import numpy as np
@@ -14,6 +17,15 @@ from sdrreceiver_b200 import binding as B
 zmq = pytest.importorskip("zmq")
 
 
+@pytest.fixture
+def sock_dir():
+    """Directory for ipc:// endpoints. A Unix socket path holds at most 107 bytes, which a deep tmp_path can exceed, so the
+    sockets live in a fresh directory directly under /tmp."""
+    d = tempfile.mkdtemp(prefix="sdrb-", dir="/tmp")
+    yield pathlib.Path(d)
+    shutil.rmtree(d, ignore_errors=True)
+
+
 def _open(addr, bind):
     h = C.c_void_p()
     rc = B.lib().sdrb_publisher_open(addr.encode(), int(bind), C.byref(h))
@@ -23,8 +35,8 @@ def _open(addr, bind):
     return h
 
 
-def test_three_frame_messages_reach_a_subscriber(tmp_path):
-    addr = "ipc://" + str(tmp_path / "sdrb.sock")
+def test_three_frame_messages_reach_a_subscriber(sock_dir):
+    addr = "ipc://" + str(sock_dir / "sdrb.sock")
     pub = _open(addr, True)
     ctx = zmq.Context()
     sub = ctx.socket(zmq.SUB)
@@ -48,8 +60,8 @@ def test_three_frame_messages_reach_a_subscriber(tmp_path):
     ctx.term()
 
 
-def test_send_block_emits_one_message_per_vfo_in_plan_order(tmp_path):
-    addr = "ipc://" + str(tmp_path / "sdrb2.sock")
+def test_send_block_emits_one_message_per_vfo_in_plan_order(sock_dir):
+    addr = "ipc://" + str(sock_dir / "sdrb2.sock")
     pub = _open(addr, True)
     ctx = zmq.Context()
     sub = ctx.socket(zmq.SUB)
@@ -77,11 +89,11 @@ def test_bad_address_is_an_error_code_not_a_crash():
     assert rc == -5 and not h.value
 
 
-def test_publisher_pool_keeps_format_and_per_receiver_order(tmp_path):
+def test_publisher_pool_keeps_format_and_per_receiver_order(sock_dir):
     """sdrb_publisher_pool_*: n sockets, one sender thread each; receiver s on socket s % n, its callbacks in order, every message
     the reference's three frames (zmqpublisher.cpp:82-96). One SUB socket per pool address plays the decoders."""
     L = B.lib()
-    base = "ipc://" + str(tmp_path / "pool.sock")
+    base = "ipc://" + str(sock_dir / "pool.sock")
     pool = C.c_void_p()
     rc = L.sdrb_publisher_pool_open(base.encode(), 1, 3, C.byref(pool))
     if rc == -5:
@@ -123,9 +135,9 @@ def test_publisher_pool_keeps_format_and_per_receiver_order(tmp_path):
     ctx.term()
 
 
-def test_publisher_pool_address_rules(tmp_path):
+def test_publisher_pool_address_rules(sock_dir):
     L = B.lib()
-    for base, want in (("ipc://" + str(tmp_path / "a%d.sock"), "ipc://" + str(tmp_path / "a1.sock")),
+    for base, want in (("ipc://" + str(sock_dir / "a%d.sock"), "ipc://" + str(sock_dir / "a1.sock")),
                        ("tcp://127.0.0.1:45731", "tcp://127.0.0.1:45732")):
         pool = C.c_void_p()
         rc = L.sdrb_publisher_pool_open(base.encode(), 1, 2, C.byref(pool))
@@ -140,7 +152,7 @@ def test_publisher_pool_address_rules(tmp_path):
     assert L.sdrb_publisher_pool_open(b"ipc:///tmp/x", 1, 0, C.byref(pool)) == -1 and not pool.value
 
 
-def test_pool_delivers_a_whole_call_to_the_counting_sink(tmp_path):
+def test_pool_delivers_a_whole_call_to_the_counting_sink(sock_dir):
     """A call's burst (here 8 receivers x 2 callbacks x 27 messages on 2 sockets, three times) reaches tools/zmq_sink.cpp -- the
     counting subscriber bench.py uses for its publish leg -- completely: message count and payload bytes."""
     import json
@@ -151,7 +163,7 @@ def test_pool_delivers_a_whole_call_to_the_counting_sink(tmp_path):
         pytest.skip("zmq_sink not built (make -C sdrreceiver_b200/csrc)")
     L = B.lib()
     pool = C.c_void_p()
-    rc = L.sdrb_publisher_pool_open(("ipc://" + str(tmp_path / "sink%d.sock")).encode(), 1, 2, C.byref(pool))
+    rc = L.sdrb_publisher_pool_open(("ipc://" + str(sock_dir / "sink%d.sock")).encode(), 1, 2, C.byref(pool))
     if rc == -5:
         pytest.skip("libzmq not loadable here")
     assert rc == 0, L.sdrb_last_error()

@@ -2,7 +2,8 @@
 """Generate tests/golden/* from the UNMODIFIED reference (oracle/_ref, needs /root/reference to
 have been built). The fixtures let a box without oracle/_ref still pin the C restatement and
 the CUDA path to reference outputs. Inputs are regenerated from sdrreceiver_b200.synth (seeded,
-library-RNG free), so only outputs/digests are stored."""
+library-RNG free), so only outputs/digests are stored. `make_golden.py runs` writes only what
+write_reference_runs() writes, from sdr_ref_i16 and sdr_ref_f32."""
 import ctypes as C
 import hashlib
 import json
@@ -39,7 +40,55 @@ def write_canaries(names=("25E", "54W_288K", "54W_all", "CBAND_143E")):
                             **{"pcm_" + k: v for k, v in outs.items()})
 
 
+RUN_STRIDE = 257      # prime, so the sample does not lock onto a callback or half-band period
+
+
+def digest(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def write_reference_runs():
+    """Whole runs of the reference binaries alone (sdr_ref_i16 / sdr_ref_f32, no libref_prims.so needed):
+    ref_runs.json  -- SHA-256 of every sub VFO's int16 and float tap (IQ forwarders: their payload bytes) and of every
+                      main-VFO tap, and the wire frames, for the runs tests/test_oracle_vs_ref.py and
+                      tests/test_forwarder.py hold the restatement to bit for bit;
+    ref_<plan>_16blocks.npz -- every RUN_STRIDE-th int16 and float-tap sample of every sub VFO over 16 callbacks, what
+                      tests/test_parity_gpu.py holds the CUDA path to."""
+    runs = {}
+    for name, n_blocks in [(p, 2) for p in PLANS] + [("25E", 16), ("CBAND_143E", 13), ("54W_all", 9), ("54W_288K", 12),
+                                                     ("FWD_test", 3)]:
+        op, iq = plan_input(name, n_blocks)
+        ini = os.path.join(ROOT, "plans", name + ".ini")
+        outs, frames, mains = O.run_ref(ini, iq, main_tap=True)
+        taps, _, _ = O.run_ref(ini, iq, float_tap=True)
+        runs["%s/%d" % (name, n_blocks)] = {
+            "input_sha256": digest(iq),
+            "pcm_sha256": {k: digest(v) for k, v in outs.items()},
+            "tap_sha256": {k: digest(v) for k, v in taps.items()},
+            "main_sha256": {str(k): digest(v) for k, v in mains.items()},
+            "frames": [[t.hex(), r, n, p] for t, r, n, p in frames],
+        }
+    with open(os.path.join(GOLD, "ref_runs.json"), "w") as f:
+        json.dump(runs, f, sort_keys=True, separators=(",", ":"))
+    for name in ("25E", "CBAND_143E"):
+        op, iq = plan_input(name, 16)
+        ini = os.path.join(ROOT, "plans", name + ".ini")
+        outs, _, _ = O.run_ref(ini, iq)
+        taps, _, _ = O.run_ref(ini, iq, float_tap=True)
+        np.savez_compressed(os.path.join(GOLD, "ref_%s_16blocks.npz" % name),
+                            input_sha256=np.frombuffer(hashlib.sha256(iq.tobytes()).digest(), np.uint8),
+                            stride=np.int64(RUN_STRIDE),
+                            **{"pcm_" + k: v[::RUN_STRIDE].copy() for k, v in outs.items()},
+                            **{"tap_" + k: v[::RUN_STRIDE].copy() for k, v in taps.items()},
+                            **{"n_" + k: np.int64(v.size) for k, v in outs.items()})
+
+
 def main():
+    if sys.argv[1:] == ["runs"]:
+        assert all(os.path.exists(os.path.join(O.REF_DIR, f)) for f in ("sdr_ref_i16", "sdr_ref_f32")), \
+            "build oracle/_ref/sdr_ref_i16 and sdr_ref_f32 first (make -C oracle)"
+        write_reference_runs()
+        return
     assert O.have_ref(), "build oracle/_ref first (make -C oracle)"
     os.makedirs(GOLD, exist_ok=True)
     R = O.ref_prims()
@@ -96,6 +145,7 @@ def main():
         }
     # ---- the bench's canaries: first callback of stream 0 of a plan from a reset receiver, full int16 (bench.py canary_check) ----
     write_canaries()
+    write_reference_runs()
     with open(os.path.join(GOLD, "plan_digests.json"), "w") as f:
         json.dump(dig, f, indent=1, sort_keys=True)
     print("golden written to", GOLD)
