@@ -265,9 +265,6 @@ struct sdrb_bank {
     int k3_cta_warps2 = 0;                        // ... of the groups with at most 3 stages (SDRB_K3_CTA_WARPS2=1..12; 0 = the size with the most resident warps): their 160-register warps fit
                                                   // three to a scheduler, shared memory per CTA (the rotation table is per CTA) decides
     int k3_regs5 = 200;                           // register cap of the 5-stage k2a_v3 instantiation (SDRB_K3_REGS=168|200|232|255; 200..255 all hold two warps per scheduler)
-    int dc_run = 4;                               // blocks per integer solve of k0_dc_walk: 4, 2 or 1 (SDRB_DC_RUN; 1 = round-1 behaviour)
-    bool dcw_bulk = false;                        // k0_dc_walk: one bulk copy per batch instead of per-lane cp.async (SDRB_DCW_BULK=1; measured neutral)
-    int dcw_ring = 2;                             // shared-memory ring depth of k0_dc_walk (SDRB_DCW_RING=4: the round-1 size)
     int dbg_only = 0;                             // SDRB_DEBUG_ONLY=dc|filters: profiling aid, device-resident calls skip the other half (results are then meaningless)
     DevBuf cascdev, rfdev, latedev, usbdev, carry;
     std::vector<SubGroup> groups;
@@ -447,12 +444,9 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
 
     // ---- descriptors ----
     K1Params &k1 = b->k1;
-    k1.tail = (const uint8_t *)b->raw_tail.p;
     k1.cf_in = nullptr; k1.cf_stride = 0; k1.cf_tail = (const float2 *)b->cf_tail.p;
-    k1.dc_table = (const uint2 *)b->dc_table.p;
-    k1.dc_anchor = (const DcAnchor *)b->dc_anchor.p;
     k1.blocks_done = (const long long *)b->blocks_done.p;
-    k1.dc_stride = b->dc_stride + DC_HALO_BLKS; k1.block = h.block; k1.correct_dc = h.correct_dc; k1.n_main = (int)h.mains.size();
+    k1.block = h.block; k1.n_main = (int)h.mains.size();
     for (size_t i = 0; i < h.mains.size(); i++) {
         MainDev &M = k1.mains[i];
         M.lut = (const float2 *)b->luts.p + main_lut_off[i];
@@ -666,12 +660,7 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
     b->uv_warp_floats = std::max(UV_IN_FLOATS, 2 * b->uv_eo_rows * UV_ROW);
     b->uv_smem = sizeof(float) * (2 * (size_t)(64 + b->uv_np_max) + (size_t)UV_WARPS * b->uv_warp_floats);
     BANK_CU(cudaFuncSetAttribute(k2b_v2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->uv_smem));
-    BANK_CU(cudaFuncSetAttribute(k0_dc_walk<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dcw_smem<2>()));
-    BANK_CU(cudaFuncSetAttribute(k0_dc_walk<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dcw_smem<2>()));
-    BANK_CU(cudaFuncSetAttribute(k0_dc_walk<4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dcw_smem<4>()));
-    if (const char *e = getenv("SDRB_DCW_RING")) b->dcw_ring = atoi(e) == 4 ? 4 : 2;
-    if (const char *e = getenv("SDRB_DCW_BULK")) b->dcw_bulk = atoi(e) != 0;
-    if (const char *e = getenv("SDRB_DC_RUN")) b->dc_run = atoi(e) >= 4 ? 4 : (atoi(e) >= 2 ? 2 : 1);
+    BANK_CU(cudaFuncSetAttribute(k0_dc_walk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DCW_SMEM));
     BANK_CU((cudaFuncSetAttribute(k2_late_v2<5, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lv_smem<5>())));
     BANK_CU((cudaFuncSetAttribute(k2_late_v2<6, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lv_smem<6>())));
     BANK_CU((cudaFuncSetAttribute(k2_late_v2<5, 10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lv_smem<5>())));
@@ -788,18 +777,9 @@ static int enqueue_dc_cb(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaStr
     }
     {
         TimedScope t(b, sd, 0);
-        if (b->dcw_ring == 4)
-            k0_dc_walk<4, false><<<(unsigned)ns, 64, dcw_smem<4>(), sd>>>(c.d_iq, c.iq_stride, (const DcStats *)b->dc_stats.p, b->dc_stride,
-                                                                  b->anchor_buf(c.par), b->qtab_buf(c.par), (float2 *)b->dc_state.p, b->table_buf(c.par),
-                                                                  b->dc_stride + DC_HALO_BLKS, cb * per_cb, per_cb, s0, b->dc_run);
-        else if (b->dcw_bulk)
-            k0_dc_walk<2, true><<<(unsigned)ns, 64, dcw_smem<2>(), sd>>>(c.d_iq, c.iq_stride, (const DcStats *)b->dc_stats.p, b->dc_stride,
-                                                                        b->anchor_buf(c.par), b->qtab_buf(c.par), (float2 *)b->dc_state.p, b->table_buf(c.par),
-                                                                        b->dc_stride + DC_HALO_BLKS, cb * per_cb, per_cb, s0, b->dc_run);
-        else
-            k0_dc_walk<2, false><<<(unsigned)ns, 64, dcw_smem<2>(), sd>>>(c.d_iq, c.iq_stride, (const DcStats *)b->dc_stats.p, b->dc_stride,
-                                                                         b->anchor_buf(c.par), b->qtab_buf(c.par), (float2 *)b->dc_state.p, b->table_buf(c.par),
-                                                                         b->dc_stride + DC_HALO_BLKS, cb * per_cb, per_cb, s0, b->dc_run);
+        k0_dc_walk<<<(unsigned)ns, 64, DCW_SMEM, sd>>>(c.d_iq, c.iq_stride, (const DcStats *)b->dc_stats.p, b->dc_stride,
+                                                      b->anchor_buf(c.par), b->qtab_buf(c.par), (float2 *)b->dc_state.p, b->table_buf(c.par),
+                                                      b->dc_stride + DC_HALO_BLKS, cb * per_cb, per_cb, s0);
     }
     (*nl) += 2;
     CU_TRY(cudaEventRecord(done, sd));
@@ -811,9 +791,8 @@ static int enqueue_ingest_cb(sdrb_bank *b, const CallCtx &c, int s0, int ns, cud
     const HostPlan &h = b->plan->h;
     if (wait) CU_TRY(cudaStreamWaitEvent(st, wait, 0));
     K1Params k1 = b->k1;
-    k1.iq = c.d_iq; k1.iq_stride = c.iq_stride; k1.n_blocks = c.n_blocks; k1.stream0 = s0; k1.b0 = cb;
+    k1.stream0 = s0; k1.b0 = cb;
     k1.cf_in = c.d_cf; k1.cf_stride = c.cf_stride;
-    k1.dc_table = b->table_buf(c.par); k1.dc_anchor = b->anchor_buf(c.par);
     if (c.d_cf) {
         const int k1_tiles = (h.block + K1_TILE - 1) / K1_TILE;
         TimedScope t(b, st, 1);

@@ -422,7 +422,7 @@ constexpr int K1_TPC = SDRB_K1_TPC;
 
 // ---- bulk-copy (TMA engine, cp.async.bulk + mbarrier) variant of the tile prefetch: one elected thread moves the whole
 // tile's raw bytes and DC block states with two or three bulk copies; everybody waits on the buffer's mbarrier ----
-// (mbar_init / mbar_expect_tx / mbar_wait / bulk_g2s live in kernels.cuh: the DC walk uses them too)
+// (mbar_init / mbar_expect_tx / mbar_wait / bulk_g2s live in kernels.cuh)
 template <int NT> constexpr int k1_bulk_raw_bytes() { return NT * 64 + 32; }                 // samples v0(0)-16 .. v0(NT-1)+31
 template <int NT> constexpr int k1_bulk_buf_bytes() { return k1_bulk_raw_bytes<NT>() + (NT / 4) * 16 + 16; }
 template <int NT> constexpr size_t k1v2_smem_bulk() { return V2L<NT>::SMEM + 2 * (size_t)k1_bulk_buf_bytes<NT>(); }

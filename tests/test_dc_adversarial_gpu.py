@@ -8,8 +8,7 @@ lock-in fixed points, and through the largest excursion one block can make. Each
 
   * the block-start DC states and the DC-corrected input of every callback equal the plain-C restatement bit for bit;
   * whole-plan outputs of three of the scenarios agree with the restatement (+-1 LSB, 1e-4 rel-L2);
-  * how the callbacks are grouped into calls, the input-ready overlap of process_device_ex and every walk variant
-    selectable through the environment give identical bits;
+  * how the callbacks are grouped into calls and the input-ready overlap of process_device_ex give identical bits;
   * the walk's per-block mode bytes show that every path was taken (translations below and above T, integer solves,
     also in the ragged last batch of a callback, float steps), and that every block whose states leave the anchor's
     window was stepped in float -- a necessary condition of the algorithm, checked from the restatement's own trace."""
@@ -296,15 +295,6 @@ def test_call_shape_does_not_matter(case):
     same_bits(case.main, run_bank(case.plan, case.iq, [case.n_cb], want_tap=True), "one call")
     same_bits(case.main, run_bank(case.plan, case.iq, [1] * case.n_cb, want_tap=True), "single-callback calls")
     same_bits(case.main, run_bank_overlapped(case.plan, case.iq, case.split), "process_device_ex, overlapped")
-
-
-@pytest.mark.parametrize("env", [{"SDRB_DC_RUN": "1"}, {"SDRB_DC_RUN": "2"}, {"SDRB_DC_RUN": "4"},
-                                 {"SDRB_DCW_RING": "4"}, {"SDRB_DCW_BULK": "1"}], ids=lambda e: "-".join(map("=".join, e.items())))
-def test_walk_variants(case, env, monkeypatch):
-    """Every walk variant the environment selects (read in sdrb_bank_create) gives the same bits."""
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
-    same_bits(case.main, run_bank(case.plan, case.iq, case.split, want_tap=True), str(env))
 
 
 # ---- the scenarios do what they say --------------------------------------------------------------------------------------

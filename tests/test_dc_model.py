@@ -10,12 +10,12 @@ recursion to with a usable ("ok") anchor:
   1. inside the anchor's window (lo, hi) the rounded product removes r0 ulps below T and r0 + 1 from T on, and T is the
      true first mantissa of r0 + 1 wherever the walk can see it;
   2. one real step from a state in the window moves its bit pattern by exactly Q(byte) - r0 - [bits >= T];
-  3. no byte is a rounding tie (DC_QTIE) for an ok anchor, so the tie branches of the walk are unreachable with uint8
-     input -- while ties do exist for states below 2^-6, where no anchor is ok;
+  3. no byte is a rounding tie for an ok anchor, which is why k0_dc_qtab, k0_dc_blocks and the walk have no tie
+     handling -- while ties do exist for states below 2^-6, where no anchor is ok;
   4. the largest dip one block can make from the window's low edge keeps r in {r0, r0 + 1}: the low side needs no
      per-block check (only the high side has one, DcStats::tb_hi).
 
-Restated: kernels.cuh dc_step / dc_incr (lines 255-266), k0_dc_anchor (268-320), k0_dc_qtab (328-340)."""
+Restated: kernels.cuh dc_step / dc_incr (lines 250-258), k0_dc_anchor (260-312), k0_dc_qtab (320-326)."""
 import math
 
 import numpy as np
@@ -26,7 +26,6 @@ DC_A = F32(1.0) - F32(0.000001)          # kernels.cuh:48, folded in float like 
 DC_C = F32(0.000001)
 DC_MAGIC = F32(12582912.0)
 DC_BLK = 128
-DC_QTIE = 0x40000000
 STEP = 16777216.0 / 17.0                   # mantissa distance between steps of r
 EF_LO, EF_HI = 127 - 8, 127 + 7            # binades 2^-8 .. 2^7: |avept| <= 128 for uint8 input, and the binade above
 EF_OK_MIN = 127 - 3                        # anchors are ok from 2^-3 up
@@ -41,13 +40,13 @@ def bits_of(x):
 
 
 def dc_step(s, x):
-    """kernels.cuh:255-257, elementwise in float32."""
+    """kernels.cuh:250-252, elementwise in float32."""
     s, x = np.asarray(s, F32), np.asarray(x, F32)
     return (s * DC_A) + (DC_C * x)
 
 
 def anchor(s0):
-    """k0_dc_anchor (kernels.cuh:268-320) for one state; float32 operations in the kernel's order, doubles where it
+    """k0_dc_anchor (kernels.cuh:260-312) for one state; float32 operations in the kernel's order, doubles where it
     uses doubles. Returns a dict with the DcAnchor fields."""
     s0 = F32(s0)
     A = dict(sgn=-1.0 if s0 < 0 else 1.0, inv_u=F32(0), r0=0, ok=0, T=0, lo=0, hi=0, pinned=True)
@@ -94,14 +93,15 @@ def anchor(s0):
 
 
 def qtab(A):
-    """k0_dc_qtab (kernels.cuh:328-340) with dc_incr (261-266): increment d = Q - r0 of each byte, or DC_QTIE."""
+    """k0_dc_qtab (kernels.cuh:320-326) with dc_incr (255-258): increment d = Q - r0 of each byte. Also returns
+    which bytes are rounding ties, fl(c * x) / ulp an exact half: the kernel assumes there are none."""
     x = (np.arange(256) - 127).astype(F32)
     y = F32(DC_C) * (F32(A["sgn"]) * x)
     y = (y * F32(A["inv_u"])).astype(F32)
     q = ((y + DC_MAGIC).astype(F32) - DC_MAGIC).astype(F32)
     tie = np.abs((y - q).astype(F32)) == F32(0.5)
     d = q.astype(np.int64) - A["r0"]
-    return np.where(tie, DC_QTIE, d if A["ok"] else 0), tie
+    return (d if A["ok"] else np.zeros_like(d)), tie
 
 
 def r_of_binade(ef):
@@ -218,9 +218,9 @@ def test_increment_model_sampled(ok_anchors):
 
 
 def test_no_rounding_tie_is_reachable(binades, ok_anchors):
-    """fl(c * x) / ulp is never an exact half for an ok anchor, whatever the byte and sign: the DC_QTIE branches of
-    k0_dc_blocks, dc_solve_run and the one-block solve cannot be taken with uint8 input. They exist because ties do
-    occur for |avept| < 2^-6 (where the anchor is never ok): removing them needs this test to keep passing."""
+    """fl(c * x) / ulp is never an exact half for an ok anchor, whatever the byte and sign: this is why k0_dc_qtab
+    stores Q - r0 without marking ties, and k0_dc_blocks and the walk's integer solves have no tie branch. Ties do occur
+    for |avept| < 2^-6, where the anchor is never ok and every block is stepped in float."""
     for A in ok_anchors:
         for sg in (1.0, -1.0):
             _, tie = qtab(dict(A, sgn=sg))

@@ -344,15 +344,14 @@ def test_dc_state_is_bit_identical(dc, sigma, n_blocks, splits):
 @pytest.mark.gpu
 @pytest.mark.parametrize("k1_threads,k2a_threads,extra", [(128, 64, {}), (96, 96, {"SDRB_K2A_V3": "0"}), (64, 128, {"SDRB_K1_BULK": "0"}),
                                                           (64, 64, {"SDRB_K2A_V3": "0", "SDRB_FUSE_LATE": "0", "SDRB_PER_CB": "1"}),
-                                                          (64, 64, {"SDRB_K3_REGS": "168", "SDRB_K3_CTA_WARPS": "4", "SDRB_DCW_RING": "4"}),
-                                                          (64, 64, {"SDRB_LATE_GENERIC": "1", "SDRB_DC_RUN": "1", "SDRB_DCW_BULK": "1",
-                                                                    "SDRB_K3_CTA_WARPS2": "3", "SDRB_K3_WAVES": "3"})])
+                                                          (64, 64, {"SDRB_K3_REGS": "168", "SDRB_K3_CTA_WARPS": "4"}),
+                                                          (64, 64, {"SDRB_LATE_GENERIC": "1", "SDRB_K3_CTA_WARPS2": "3", "SDRB_K3_WAVES": "3"})])
 def test_every_cta_size_of_the_cascade_kernels(k1_threads, k2a_threads, extra):
     """k1_v2 / k2a_v2 exist for 64-, 96- and 128-thread CTAs and the host picks one per launch
     (api.cu: v2_pick_threads). SDRB_K1_THREADS / SDRB_K2A_THREADS force a size: every instantiation
     must pass the same oracle comparison as the default (smoke(): 54W_288K and 25E, 1e-4 rel-L2, +-1 LSB).
     The other switches select the kernels the defaults replaced (k2a_v2 instead of k2a_v3, per-thread cp.async instead of
-    the bulk-copy prefetch, unfused /late mixer, per-callback launches, other register caps / CTA sizes / ring depths): they
+    the bulk-copy prefetch, unfused /late mixer, per-callback launches, other register caps / CTA sizes): they
     stay selectable for A/B measurements and must stay correct."""
     import subprocess
     import sys
