@@ -201,6 +201,7 @@ struct SubGroup {           // sub VFOs of one main VFO (at most V2_MAX_VFO) -> 
     // whole number of 128-sample tiles; otherwise the group stays on k2a_v2
     bool v3 = false;
     int v3_maxs = 5, v3_nsw = 1;
+    bool ragged = false;    // callback not a whole number of 32-sample chunks: k2a_v2's masked instantiation
 };
 
 // Rf[j] = (rot/|rot|)^j, j = -10..31 (index j + 10), rot = the float rotation the Oscillator table is
@@ -281,6 +282,11 @@ struct sdrb_bank {
     size_t z_stride = 0;                    // float2 per stream in zbuf
     std::vector<size_t> sub_z_off;          // per sub VFO: offset of its slice inside a stream's zbuf row
     std::vector<int> sub_z_hist;            // ... and the history samples in front of the body
+    // VFOs deeper than their mixing kernel's cascade (main VFOs with 4..8 stages, sub VFOs with 6..8): the mixing kernel writes
+    // a staging slice (k1_v2 / k1_ingest_main: 3 stages, k2a_v3 / k2a_v2: 5) inside the same per-stream row as the real outputs
+    // (main_out, zbuf), and k_hb_tail runs the remaining stages into the real output. Empty for plans without such VFOs.
+    DevBuf main_tails, sub_tails;           // TailDev per deep main / sub VFO
+    int n_main_tails = 0, n_sub_tails = 0, main_tail_tiles = 0, sub_tail_tiles = 0;   // channels and the longest channel's tiles
     // what the last process call consumed (inspection entry points: spectrum of the raw input)
     const uint8_t *last_iq = nullptr; size_t last_iq_stride = 0;
     const float2 *last_cf = nullptr; size_t last_cf_stride = 0;
@@ -317,6 +323,7 @@ extern "C" void sdrb_bank_destroy(sdrb_bank *b) {
     cudaDeviceSynchronize();                                 // asynchronous host calls may still be in flight
     DevBuf *all[] = {&b->luts, &b->taps, &b->blocks_done, &b->dc_state, &b->raw_tail, &b->cf_tail, &b->dc_anchor, &b->dc_stats, &b->dc_table, &b->dc_qtab,
                      &b->main_out, &b->zbuf, &b->dbuf, &b->cascdev, &b->rfdev, &b->latedev, &b->usbdev, &b->carry,
+                     &b->main_tails, &b->sub_tails,
                      &b->d_iq, &b->d_pcm, &b->d_tap, &b->d_cf, &b->d_fwd, &b->k3_rrel};
     for (DevBuf *d : all) d->release();
     for (cudaEvent_t e : b->ev_in) cudaEventDestroy(e);
@@ -414,12 +421,21 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
     BANK_TRY(b->dc_qtab.alloc(2 * sizeof(int) * 512 * (size_t)n_streams));
     BANK_TRY(b->dc_stats.alloc(h.correct_dc ? sizeof(DcStats) * 2 * (size_t)n_streams * (size_t)b->dc_stride + 1024 : 16));
     BANK_TRY(b->dc_table.alloc(h.correct_dc ? 2 * sizeof(uint2) * 2 * (size_t)n_streams * (size_t)(b->dc_stride + DC_HALO_BLKS) : 64));
+    // staging slices of the deep VFOs: first stage count a mixing kernel runs, and the rest for k_hb_tail
+    static_assert(TAIL_HIST == MAIN_HIST, "k1_ingest_main writes every main output, staged or not, behind MAIN_HIST samples");
+    constexpr int kMainStaged = 3, kSubStaged = 5;
+    std::vector<size_t> main_stage_off(h.mains.size(), 0), sub_stage_off(h.subs.size(), 0);
     {
         size_t at = 0;
         for (const MainVfo &m : h.mains) {
             b->main_off.push_back(at);
             at += round_up((size_t)MAIN_HIST + (size_t)max_blocks * m.block_out, 2);
         }
+        for (size_t i = 0; i < h.mains.size(); i++)
+            if (h.mains[i].decim > kMainStaged) {
+                main_stage_off[i] = at;
+                at += round_up((size_t)TAIL_HIST + (size_t)max_blocks * (h.block >> kMainStaged), 2);
+            }
         b->main_stride = at;
     }
     BANK_TRY(b->main_out.alloc(sizeof(float2) * b->main_stride * (size_t)n_streams));
@@ -439,6 +455,11 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
         d_off.push_back(d_stride);
         if (s.late > 0) d_stride += round_up((size_t)dh + (size_t)max_blocks * s.samples_out, 2);
     }
+    for (size_t i = 0; i < h.subs.size(); i++)
+        if (h.subs[i].decim > kSubStaged) {
+            sub_stage_off[i] = z_stride;
+            z_stride += round_up((size_t)TAIL_HIST + (size_t)max_blocks * (h.subs[i].block_in >> kSubStaged), 2);
+        }
     BANK_TRY(b->zbuf.alloc(sizeof(float2) * z_stride * (size_t)n_streams));
     BANK_TRY(b->dbuf.alloc(sizeof(float2) * d_stride * (size_t)n_streams));
 
@@ -453,6 +474,10 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
         M.out = (float2 *)b->main_out.p + b->main_off[i];
         M.out_stride = (long long)b->main_stride;
         M.lut_len = (int)h.mains[i].lut.size(); M.decim = h.mains[i].decim; M.block_out = h.mains[i].block_out;
+        if (h.mains[i].decim > kMainStaged) {
+            M.out = (float2 *)b->main_out.p + main_stage_off[i];
+            M.decim = kMainStaged; M.block_out = h.block >> kMainStaged;
+        }
     }
     // sub VFOs grouped by parent main VFO: one k2a_v2 launch per group, the parent's output is
     // read once per thread and kept in registers for all sub VFOs of the group
@@ -479,7 +504,7 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
             if (h.subs[i].main_idx != (int)mi || b->sub_fused[i]) continue;
             if (g.count == V2_MAX_VFO) { b->groups.push_back(g); g.first = (int)order.size(); g.count = 0; g.halo = 0; }
             order.push_back((int)i); g.count++;
-            g.halo = std::max(g.halo, kHalo[h.subs[i].decim]);
+            g.halo = std::max(g.halo, kHalo[std::min(h.subs[i].decim, kSubStaged)]);
         }
         if (g.count) b->groups.push_back(g);
     }
@@ -489,21 +514,31 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
         const SubVfo &s0v = h.subs[(size_t)order[(size_t)g.first]];
         g.lut_len = (int)s0v.lut.size(); g.block_in = s0v.block_in;
         g.tiles = (g.block_in + adv - 1) / adv;
+        g.ragged = g.block_in % V2_CHUNK != 0;
     }
     std::vector<CascVfo> cascdev;
     std::vector<float2> rfhost((h.mains.size() + h.subs.size()) * RF_LEN);
     std::vector<LateDev> latedev;
     std::vector<UsbDev> usbdev;
     std::vector<CarryItem> carry;
+    // the mixing cascade of sub VFO i: z itself, or the staging slice of a sub VFO with more than 5 stages
+    auto sub_cascade = [&](size_t i) {
+        const SubVfo &s = h.subs[i];
+        CascVfo D;
+        D.lut = (const float2 *)b->luts.p + sub_lut_off[i];
+        D.out = (float2 *)b->zbuf.p + z_off[i];
+        D.S = s.decim; D.block_out = s.block_z; D.hist = z_hist[i]; D.pad = 0;
+        if (s.decim > kSubStaged) {
+            D.out = (float2 *)b->zbuf.p + sub_stage_off[i];
+            D.S = kSubStaged; D.block_out = s.block_in >> kSubStaged; D.hist = TAIL_HIST;
+        }
+        return D;
+    };
     for (size_t i = 0; i < h.mains.size(); i++) rf_table((double)h.fs, h.mains[i].mixer, &rfhost[i * RF_LEN]);
     for (size_t k = 0; k < order.size(); k++) {
         const int i = order[k];
         const SubVfo &s = h.subs[(size_t)i];
-        CascVfo D;
-        D.lut = (const float2 *)b->luts.p + sub_lut_off[(size_t)i];
-        D.out = (float2 *)b->zbuf.p + z_off[(size_t)i];
-        D.S = s.decim; D.block_out = s.block_z; D.hist = z_hist[(size_t)i]; D.pad = 0;
-        cascdev.push_back(D);
+        cascdev.push_back(sub_cascade((size_t)i));
         rf_table((double)s.fs, s.mixer, &rfhost[(h.mains.size() + k) * RF_LEN]);
     }
     b->z_stride = z_stride;
@@ -512,10 +547,7 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
     b->sub_casc.resize(h.subs.size()); b->sub_rf.resize(h.subs.size());
     for (size_t i = 0; i < h.subs.size(); i++) {
         const SubVfo &s = h.subs[i];
-        CascVfo &D = b->sub_casc[i];
-        D.lut = (const float2 *)b->luts.p + sub_lut_off[i];
-        D.out = (float2 *)b->zbuf.p + z_off[i];
-        D.S = s.decim; D.block_out = s.block_z; D.hist = z_hist[i]; D.pad = 0;
+        b->sub_casc[i] = sub_cascade(i);
         rf_tab((double)s.fs, s.mixer, &b->sub_rf[i]);
     }
     for (size_t i = 0; i < h.subs.size(); i++) {
@@ -564,6 +596,35 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
         c.hist_bytes = MAIN_HIST * (int)sizeof(float2); c.block_bytes = h.mains[i].block_out * (int)sizeof(float2);
         carry.push_back(c);
     }
+    // deep VFOs: the tail kernels' descriptors, and the staging slices' histories among the carry items
+    std::vector<TailDev> main_tails, sub_tails;
+    auto add_tail = [&](std::vector<TailDev> &list, float2 *in, float2 *out, size_t stride, int out_hist, int block_in, int S) {
+        TailDev T;
+        T.in = in; T.out = out; T.in_stride = T.out_stride = (long long)stride;
+        T.in_hist = TAIL_HIST; T.out_hist = out_hist; T.block_in = block_in; T.S = S;
+        T.HT = kHalo[S];
+        T.tiles = (block_in + (TAIL_NT - T.HT) * V2_CHUNK - 1) / ((TAIL_NT - T.HT) * V2_CHUNK);
+        list.push_back(T);
+        CarryItem c; c.base = in; c.stride = (long long)(stride * sizeof(float2));
+        c.hist_bytes = TAIL_HIST * (int)sizeof(float2); c.block_bytes = block_in * (int)sizeof(float2);
+        carry.push_back(c);
+        return T.tiles;
+    };
+    for (size_t i = 0; i < h.mains.size(); i++)
+        if (h.mains[i].decim > kMainStaged)
+            b->main_tail_tiles = std::max(b->main_tail_tiles,
+                                          add_tail(main_tails, (float2 *)b->main_out.p + main_stage_off[i], (float2 *)b->main_out.p + b->main_off[i],
+                                                   b->main_stride, MAIN_HIST, h.block >> kMainStaged, h.mains[i].decim - kMainStaged));
+    for (size_t i = 0; i < h.subs.size(); i++)
+        if (h.subs[i].decim > kSubStaged)
+            b->sub_tail_tiles = std::max(b->sub_tail_tiles,
+                                         add_tail(sub_tails, (float2 *)b->zbuf.p + sub_stage_off[i], (float2 *)b->zbuf.p + z_off[i], z_stride,
+                                                  z_hist[i], h.subs[i].block_in >> kSubStaged, h.subs[i].decim - kSubStaged));
+    b->n_main_tails = (int)main_tails.size(); b->n_sub_tails = (int)sub_tails.size();
+    BANK_TRY(b->main_tails.alloc(sizeof(TailDev) * std::max<size_t>(main_tails.size(), 1)));
+    BANK_TRY(b->sub_tails.alloc(sizeof(TailDev) * std::max<size_t>(sub_tails.size(), 1)));
+    if (!main_tails.empty()) BANK_CU(cudaMemcpy(b->main_tails.p, main_tails.data(), sizeof(TailDev) * main_tails.size(), cudaMemcpyHostToDevice));
+    if (!sub_tails.empty()) BANK_CU(cudaMemcpy(b->sub_tails.p, sub_tails.data(), sizeof(TailDev) * sub_tails.size(), cudaMemcpyHostToDevice));
     b->n_late = (int)latedev.size(); b->n_usb = (int)usbdev.size(); b->n_carry = (int)carry.size();
     BANK_TRY(b->cascdev.alloc(sizeof(CascVfo) * std::max<size_t>(cascdev.size(), 1)));
     BANK_TRY(b->rfdev.alloc(sizeof(float2) * rfhost.size()));
@@ -587,6 +648,10 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
             M.lut = (const float2 *)b->luts.p + main_lut_off[i];
             M.out = (float2 *)b->main_out.p + b->main_off[i];
             M.S = h.mains[i].decim; M.block_out = h.mains[i].block_out; M.hist = MAIN_HIST; M.pad = 0;
+            if (h.mains[i].decim > kMainStaged) {           // k1_v2 runs 3 stages (cascade_loop<3>); k_hb_tail the rest
+                M.out = (float2 *)b->main_out.p + main_stage_off[i];
+                M.S = kMainStaged; M.block_out = h.block >> kMainStaged; M.hist = TAIL_HIST;
+            }
         }
     }
     b->k2v2.assign(b->groups.size(), K2V2Params{});
@@ -620,10 +685,11 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
             int maxs = 0;
             for (int v = 0; v < g.count; v++) {
                 const SubVfo &sv = h.subs[(size_t)order[(size_t)(g.first + v)]];
-                if (sv.decim < 1 || sv.decim > 5) ok = false;
-                maxs = std::max(maxs, sv.decim);
+                const int staged = cascdev[(size_t)(g.first + v)].S;   // a deep sub VFO's first 5 stages; its 2^-S factor is that of the 5
+                if (staged < 1) ok = false;
+                maxs = std::max(maxs, staged);
                 K3Vfo &V = kp.v[v];
-                k3_fill_vfo((double)sv.fs, sv.mixer, std::max(sv.decim, 1), V, &rrel[(size_t)(g.first + v) * K3_OUT1]);
+                k3_fill_vfo((double)sv.fs, sv.mixer, std::max(staged, 1), V, &rrel[(size_t)(g.first + v) * K3_OUT1]);
                 V.lut = cascdev[(size_t)(g.first + v)].lut; V.out = cascdev[(size_t)(g.first + v)].out;
                 V.block_out = cascdev[(size_t)(g.first + v)].block_out; V.hist = cascdev[(size_t)(g.first + v)].hist; V.pad = 0;
             }
@@ -668,6 +734,9 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
     BANK_CU(cudaFuncSetAttribute(k2a_v2<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<64>::SMEM));
     BANK_CU(cudaFuncSetAttribute(k2a_v2<96>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<96>::SMEM));
     BANK_CU(cudaFuncSetAttribute(k2a_v2<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<128>::SMEM));
+    BANK_CU((cudaFuncSetAttribute(k2a_v2<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<64>::SMEM)));
+    BANK_CU((cudaFuncSetAttribute(k2a_v2<96, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<96>::SMEM)));
+    BANK_CU((cudaFuncSetAttribute(k2a_v2<128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<128>::SMEM)));
     BANK_CU((cudaFuncSetAttribute(k1_v2<true, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1v2_smem<64>())));
     BANK_CU((cudaFuncSetAttribute(k1_v2<false, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1v2_smem<64>())));
     BANK_CU((cudaFuncSetAttribute(k1_v2<true, 96>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1v2_smem<96>())));
@@ -836,7 +905,19 @@ static int k3_slots(K kernel, int threads, size_t smem) {
     return per_sm * sms;
 }
 
-// Sub-VFO cascades of callbacks cb0 .. cb0+ncb-1.
+// The half-band stages of the deep main VFOs (subs = false, timed with the ingest class) or sub VFOs (timed with the cascades)
+// that their mixing kernel does not run, for callbacks cb0 .. cb0+ncb-1: one k_hb_tail launch, nothing for a plan without them.
+static int enqueue_tails(sdrb_bank *b, bool subs, int s0, int ns, cudaStream_t st, int cb0, int ncb, int *nl) {
+    const int n = subs ? b->n_sub_tails : b->n_main_tails, tiles = subs ? b->sub_tail_tiles : b->main_tail_tiles;
+    if (n == 0) return SDRB_OK;
+    TimedScope t(b, st, subs ? 2 : 1);
+    k_hb_tail<<<dim3((unsigned)ns, (unsigned)(n * tiles), (unsigned)ncb), TAIL_NT, V2L<TAIL_NT>::SMEM, st>>>(
+        (const TailDev *)(subs ? b->sub_tails.p : b->main_tails.p), tiles, s0, cb0);
+    (*nl)++;
+    return SDRB_OK;
+}
+
+// Sub-VFO cascades of callbacks cb0 .. cb0+ncb-1 (and the tails of the deep ones).
 static int enqueue_subs(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaStream_t st, int cb0, int ncb, int *nl) {
     for (const SubGroup &g : b->groups) {
         const size_t gi = (size_t)(&g - b->groups.data());
@@ -902,12 +983,16 @@ static int enqueue_subs(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaStre
         kp.stream0 = s0; kp.b0 = cb0;
         TimedScope t(b, st, 2);
         const dim3 grid((unsigned)ns, (unsigned)g.tiles, (unsigned)ncb);
-        if (g.threads == 64) k2a_v2<64><<<grid, 64, V2L<64>::SMEM, st>>>(kp);
+        if (g.ragged) {
+            if (g.threads == 64) k2a_v2<64, true><<<grid, 64, V2L<64>::SMEM, st>>>(kp);
+            else if (g.threads == 96) k2a_v2<96, true><<<grid, 96, V2L<96>::SMEM, st>>>(kp);
+            else k2a_v2<128, true><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
+        } else if (g.threads == 64) k2a_v2<64><<<grid, 64, V2L<64>::SMEM, st>>>(kp);
         else if (g.threads == 96) k2a_v2<96><<<grid, 96, V2L<96>::SMEM, st>>>(kp);
         else k2a_v2<128><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
         (*nl)++;
     }
-    return SDRB_OK;
+    return enqueue_tails(b, true, s0, ns, st, cb0, ncb, nl);
 }
 
 // /late FIR and USB audio of callbacks cb0 .. cb0+ncb-1. `out_done` (optional) is recorded at the end.
@@ -959,6 +1044,7 @@ static int enqueue_main_cb(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaS
                            cudaEvent_t out_done, int *nl) {
     int rc;
     if ((rc = enqueue_ingest_cb(b, c, s0, ns, st, cb, wait, nl)) != SDRB_OK) return rc;
+    if ((rc = enqueue_tails(b, false, s0, ns, st, cb, 1, nl)) != SDRB_OK) return rc;
     if ((rc = enqueue_subs(b, c, s0, ns, st, cb, 1, nl)) != SDRB_OK) return rc;
     return enqueue_audio(b, c, s0, ns, st, cb, 1, out_done, nl);
 }
@@ -1018,6 +1104,7 @@ static int enqueue_all(sdrb_bank *b, CallCtx &c, cudaStream_t st, int *launches,
         // (their warm-up tiles amortise), and the DC walk of the next call has the whole cascade/audio phase to hide in
         for (int cb = 0; cb < c.n_blocks; cb++)
             if ((rc = enqueue_ingest_cb(b, c, 0, ns, st, cb, dc ? b->ev_dc[0][(size_t)cb] : nullptr, launches)) != SDRB_OK) return rc;
+        if ((rc = enqueue_tails(b, false, 0, ns, st, 0, c.n_blocks, launches)) != SDRB_OK) return rc;
         if ((rc = enqueue_subs(b, c, 0, ns, st, 0, c.n_blocks, launches)) != SDRB_OK) return rc;
         if ((rc = enqueue_audio(b, c, 0, ns, st, 0, c.n_blocks, nullptr, launches)) != SDRB_OK) return rc;
     }
@@ -1217,7 +1304,9 @@ static int ensure_sub_z(sdrb_bank *b, int sub_idx, cudaStream_t st) {
     kp.count = 1; kp.lut_len = (int)s.lut.size(); kp.block_in = s.block_in; kp.HT = 0; kp.stream0 = 0; kp.b0 = 0;
     kp.blk_off = -b->last_blocks;
     const int tiles = (s.block_in + 128 * V2_CHUNK - 1) / (128 * V2_CHUNK);
-    k2a_v2<128><<<dim3((unsigned)b->n_streams, (unsigned)tiles, (unsigned)b->last_blocks), 128, V2L<128>::SMEM, st>>>(kp);
+    const dim3 grid((unsigned)b->n_streams, (unsigned)tiles, (unsigned)b->last_blocks);
+    if (s.block_in % V2_CHUNK != 0) k2a_v2<128, true><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
+    else k2a_v2<128><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
     CU_TRY(cudaGetLastError());
     return SDRB_OK;
 }

@@ -151,6 +151,19 @@ __device__ __forceinline__ void st_store(const float2 (&v)[N], float2 *__restric
     }
 }
 
+// st_store of the first n of the N outputs (a chunk that runs past the end of its callback: the filters are causal, so the outputs
+// inside the callback are complete and the rest belong to nobody). Every stored length is even, so n is even for N >= 2.
+template <int N>
+__device__ __forceinline__ void st_store_n(const float2 (&v)[N], float2 *__restrict__ dst, int n) {
+    if (n >= N) {
+        st_store<N>(v, dst);
+    } else {
+#pragma unroll
+        for (int k = 0; k < N; ++k)
+            if (k < n) dst[k] = v[k];
+    }
+}
+
 // Exact first stage for the few chunks the rotating-frame shortcut does not cover (table start-up
 // transient and wrap, stream sample 0, first chunk of a callback): every rotation is read from
 // the Oscillator table. Deliberately not inlined and not unrolled: it runs for ~1 % of the chunks
@@ -185,10 +198,12 @@ __device__ __noinline__ void stage1_exact(const float2 *xc, const float2 *__rest
 //   n_abs     absolute stream index of sample v0 (negative: before the stream began)
 //   k0        n_abs mod L
 //   P         the kernel's parameter struct (__grid_constant__): P::vfos[], P::rf[]
-template <int MAXS, int NT, class P>
+// RAGGED: the callback is not a whole number of 32-sample chunks; `nin` = samples of the callback from v0 on, and outputs
+// past the callback end are not stored (they would overwrite the next callback's first outputs).
+template <int MAXS, int NT, class P, bool RAGGED = false>
 __device__ __forceinline__ void cascade_loop(const float2 (&x)[44], const P &p, int count,
                                              float2 *__restrict__ sm, int t, int v0, long long n_abs, int k0, int L,
-                                             bool store, size_t out_off /* stream*out_stride */, int b) {
+                                             bool store, size_t out_off /* stream*out_stride */, int b, int nin = V2_CHUNK) {
     float2 *sB = sm + V2L<NT>::SB, *sC = sm + V2L<NT>::SC, *sD = sm + V2L<NT>::SD;
     int prevS = 1, flip = 0;
     const bool head = (v0 == 0);
@@ -214,7 +229,7 @@ __device__ __forceinline__ void cascade_loop(const float2 (&x)[44], const P &p, 
                 for (int q = 0; q < V2_CHUNK / 2; ++q) {
                     const float2 a = rotF(Fc, Fs, rot2(p.rf[v].q[2 * q + 10], x[12 + 2 * q]));      // Rf[2q]
                     const float2 c = rotF(Fc, Fs, rot2(p.rf[v].q[2 * q + 11], x[13 + 2 * q]));      // Rf[2q+1]
-                    *reinterpret_cast<float4 *>(outp + v0 + 2 * q) = make_float4(a.x, a.y, c.x, c.y);
+                    if (!RAGGED || 2 * q < nin) *reinterpret_cast<float4 *>(outp + v0 + 2 * q) = make_float4(a.x, a.y, c.x, c.y);
                 }
             } else if (store) {
 #pragma unroll
@@ -224,7 +239,7 @@ __device__ __forceinline__ void cascade_loop(const float2 (&x)[44], const P &p, 
                     if (i1 >= L) i1 -= L;
                     if (n_abs + j == 0) i0 = L - 1;       // oscillator.cpp:26-30
                     const float2 a = cmul(__ldg(V.lut + i0), x[12 + j]), c = cmul(__ldg(V.lut + i1), x[13 + j]);
-                    *reinterpret_cast<float4 *>(outp + v0 + j) = make_float4(a.x, a.y, c.x, c.y);
+                    if (!RAGGED || j < nin) *reinterpret_cast<float4 *>(outp + v0 + j) = make_float4(a.x, a.y, c.x, c.y);
                 }
             }
             continue;
@@ -258,7 +273,8 @@ __device__ __forceinline__ void cascade_loop(const float2 (&x)[44], const P &p, 
             if (store) {
                 float4 *o4 = reinterpret_cast<float4 *>(outp + (v0 >> 1));
 #pragma unroll
-                for (int k = 0; k < 8; ++k) o4[k] = pa[k];
+                for (int k = 0; k < 8; ++k)
+                    if (!RAGGED || 4 * k < nin) o4[k] = pa[k];
             }
             continue;
         }
@@ -266,7 +282,10 @@ __device__ __forceinline__ void cascade_loop(const float2 (&x)[44], const P &p, 
         float2 o2[8];
         st_run<16, false>(nullptr, o2, sA, t, v0 >> 1);
         if (V.S == 2) {
-            if (store) st_store<8>(o2, outp + (v0 >> 2));
+            if (store) {
+                if (RAGGED) st_store_n<8>(o2, outp + (v0 >> 2), nin >> 2);
+                else st_store<8>(o2, outp + (v0 >> 2));
+            }
             continue;
         }
         st_publish<8>(o2, sB, t);
@@ -274,7 +293,10 @@ __device__ __forceinline__ void cascade_loop(const float2 (&x)[44], const P &p, 
         float2 o3[4];
         st_run<8, true>(o2, o3, sB, t, v0 >> 2);
         if (MAXS == 3 || V.S == 3) {
-            if (store) st_store<4>(o3, outp + (v0 >> 3));
+            if (store) {
+                if (RAGGED) st_store_n<4>(o3, outp + (v0 >> 3), nin >> 3);
+                else st_store<4>(o3, outp + (v0 >> 3));
+            }
             continue;
         }
         if constexpr (MAXS > 3) {
@@ -283,14 +305,20 @@ __device__ __forceinline__ void cascade_loop(const float2 (&x)[44], const P &p, 
             float2 o4[2];
             st_run<4, true>(o3, o4, sC, t, v0 >> 3);
             if (V.S == 4) {
-                if (store) st_store<2>(o4, outp + (v0 >> 4));
+                if (store) {
+                    if (RAGGED) st_store_n<2>(o4, outp + (v0 >> 4), nin >> 4);
+                    else st_store<2>(o4, outp + (v0 >> 4));
+                }
                 continue;
             }
             st_publish<2>(o4, sD, t);
             __syncthreads();
             float2 o5[1];
             st_run<2, true>(o4, o5, sD, t, v0 >> 4);
-            if (store) st_store<1>(o5, outp + (v0 >> 5));
+            if (store) {
+                if (RAGGED) st_store_n<1>(o5, outp + (v0 >> 5), nin >> 5);
+                else st_store<1>(o5, outp + (v0 >> 5));
+            }
         }
     }
 }
@@ -309,7 +337,9 @@ struct K2V2Params {
     int blk_off, pad;               // added to the callback counter: -n for a replay of the last call's callbacks after the carry
 };
 
-template <int NT>
+// RAGGED: callbacks that are not a whole number of 32-sample chunks (a 30 000- or 3 600-sample parent): loads stop at the end of
+// the callback, stores at the end of each VFO's callback (cascade_loop).
+template <int NT, bool RAGGED = false>
 __global__ void __launch_bounds__(NT, v2_minb<NT>()) k2a_v2(const __grid_constant__ K2V2Params p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2 *sm = reinterpret_cast<float2 *>(smem_raw);
@@ -329,7 +359,7 @@ __global__ void __launch_bounds__(NT, v2_minb<NT>()) k2a_v2(const __grid_constan
         const float4 *xp = reinterpret_cast<const float4 *>(p.in + (size_t)stream * p.in_stride + MAIN_HIST + (size_t)b * B + (v0 - 12));
 #pragma unroll
         for (int q = 0; q < 22; ++q) {
-            const float4 v = __ldg(xp + q);
+            const float4 v = (!RAGGED || v0 - 12 + 2 * q < B) ? __ldg(xp + q) : make_float4(0.f, 0.f, 0.f, 0.f);
             x[2 * q] = make_float2(v.x, v.y);
             x[2 * q + 1] = make_float2(v.z, v.w);
         }
@@ -341,8 +371,103 @@ __global__ void __launch_bounds__(NT, v2_minb<NT>()) k2a_v2(const __grid_constan
     int k0 = sBase[0] + v0;
     if (k0 < 0) k0 += L;
     if (k0 >= L) k0 -= L;
-    cascade_loop<5, NT>(x, p, p.count, sm, t, v0, blk * (long long)B + v0, k0, L, in_block && t >= p.HT,
-                    (size_t)stream * p.out_stride, b);
+    cascade_loop<5, NT, K2V2Params, RAGGED>(x, p, p.count, sm, t, v0, blk * (long long)B + v0, k0, L, in_block && t >= p.HT,
+                                            (size_t)stream * p.out_stride, b, B - v0);
+}
+
+// ------------------------------------------------------------------------------------
+// k_hb_tail: the half-band stages of a VFO beyond what its mixing kernel runs (a main VFO's stages 4..8 after k1_v2's three, a
+// sub VFO's stages 6..8 after the five of k2a_v3 / k2a_v2). No NCO: the input is already mixed and partly decimated, staged
+// per callback with a carried history in front. The machine is k2a_v2's without the mixer: a thread owns 32 input samples (+ 12
+// in front) in registers and runs the first stage on them, later stages exchange 10 trailing samples through shared memory
+// (st_run), HT halo threads per tile recompute what the stages need from in front of the tile. Every stage applies the
+// FIRQueueBackToFront rule in its own callback coordinates (st_run's head path; for the first stage here: window slots at negative
+// coordinates hold the staged sample one further back, i.e. the previous callback's staged outputs).
+// Grid = (stream, channel x tile, callback): all channels of a plan class (mains or subs) and all callbacks of a call in one launch.
+// ------------------------------------------------------------------------------------
+constexpr int TAIL_NT = 64;
+constexpr int TAIL_MAX_STAGES = 5;
+constexpr int TAIL_HIST = 512;         // staged samples kept in front of each call (>= the 11 halo chunks + 12 of a 5-stage tail)
+struct TailDev {
+    const float2 *in;               // staged input: [n_streams][in_stride], in_hist + n_blocks*block_in
+    float2 *out;                    // [n_streams][out_stride], out_hist + n_blocks*(block_in >> S)
+    long long in_stride, out_stride;
+    int in_hist, out_hist, block_in, S, HT, tiles;   // HT halo threads per tile, tiles per callback
+};
+
+__global__ void __launch_bounds__(TAIL_NT) k_hb_tail(const TailDev *__restrict__ devs, int max_tiles, int stream0, int b0) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float2 *sm = reinterpret_cast<float2 *>(smem_raw);
+    const TailDev D = devs[blockIdx.y / max_tiles];
+    const int tile = blockIdx.y % max_tiles;
+    if (tile >= D.tiles) return;                              // uniform per CTA: a shorter channel of the launch
+    const int stream = stream0 + blockIdx.x, b = b0 + blockIdx.z;
+    const int t = threadIdx.x;
+    const int B = D.block_in, S = D.S;
+    const int v0 = tile * ((TAIL_NT - D.HT) * V2_CHUNK) - D.HT * V2_CHUNK + t * V2_CHUNK;
+    const bool in_block = v0 < B;
+    float2 x[44];                                             // x[i] = staged sample v0 - 12 + i
+    {
+        // halo chunks reach at most 11 * 32 + 12 samples in front of the callback: the previous callback or the carried history
+        const float4 *xp = reinterpret_cast<const float4 *>(D.in + (size_t)stream * D.in_stride + D.in_hist + (size_t)b * B + (v0 - 12));
+#pragma unroll
+        for (int q = 0; q < 22; ++q) {
+            const float4 v = (in_block && v0 - 12 + 2 * q < B) ? __ldg(xp + q) : make_float4(0.f, 0.f, 0.f, 0.f);
+            x[2 * q] = make_float2(v.x, v.y);
+            x[2 * q + 1] = make_float2(v.z, v.w);
+        }
+    }
+    // first stage on the thread's registers: output r has the window x[2r+2 .. 2r+12] (newest = sample v0 + 2r); at the head of
+    // a callback the slots at negative coordinates (x[0..11]) hold the sample one further back
+    const int head = (v0 == 0) ? 1 : 0;
+    float2 o1[16];
+#pragma unroll
+    for (int r = 0; r < 16; ++r) {
+        float2 w[11];
+#pragma unroll
+        for (int k = 0; k < 11; ++k) {
+            const int i = 2 * r + 2 + k;
+            w[k] = (i < 12 && head) ? x[i - 1] : x[i];
+        }
+        o1[r] = hb11(w[0], w[2], w[4], w[5], w[6], w[8], w[10]);
+    }
+    const bool store = in_block && t >= D.HT;
+    const int nin = B - v0;
+    float2 *outp = D.out + (size_t)stream * D.out_stride + D.out_hist + (size_t)b * (B >> S);
+    if (S == 1) {
+        if (store) st_store_n<16>(o1, outp + (v0 >> 1), nin >> 1);
+        return;
+    }
+    float2 *sA = sm + V2L<TAIL_NT>::SA, *sB = sm + V2L<TAIL_NT>::SB, *sC = sm + V2L<TAIL_NT>::SC, *sD = sm + V2L<TAIL_NT>::SD;
+    st_publish<16>(o1, sA, t);
+    __syncthreads();
+    float2 o2[8];
+    st_run<16, true>(o1, o2, sA, t, v0 >> 1);
+    if (S == 2) {
+        if (store) st_store_n<8>(o2, outp + (v0 >> 2), nin >> 2);
+        return;
+    }
+    st_publish<8>(o2, sB, t);
+    __syncthreads();
+    float2 o3[4];
+    st_run<8, true>(o2, o3, sB, t, v0 >> 2);
+    if (S == 3) {
+        if (store) st_store_n<4>(o3, outp + (v0 >> 3), nin >> 3);
+        return;
+    }
+    st_publish<4>(o3, sC, t);
+    __syncthreads();
+    float2 o4[2];
+    st_run<4, true>(o3, o4, sC, t, v0 >> 3);
+    if (S == 4) {
+        if (store) st_store_n<2>(o4, outp + (v0 >> 4), nin >> 4);
+        return;
+    }
+    st_publish<2>(o4, sD, t);
+    __syncthreads();
+    float2 o5[1];
+    st_run<2, true>(o4, o5, sD, t, v0 >> 4);
+    if (store) st_store_n<1>(o5, outp + (v0 >> 5), nin >> 5);
 }
 
 // ------------------------------------------------------------------------------------

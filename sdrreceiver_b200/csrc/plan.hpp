@@ -12,6 +12,9 @@ namespace sdrb {
 
 struct cf32 { float re, im; };
 
+constexpr int MAX_DECIM = 8;            // half-band stages of a VFO: vfo::decimate is decimate[9] (vfo.h:39)
+constexpr int MAIN_STAGE_MIN = 512;     // samples per callback after the third stage of a main VFO with more than 3 stages
+
 struct MainVfo {
     int frequency = 0;
     double mixer = 0;

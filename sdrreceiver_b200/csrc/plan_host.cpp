@@ -141,6 +141,29 @@ static int ilog2_floor_of_ratio(int num, int den) {
     return (int)std::log2((double)(num / den));
 }
 
+static std::string vfo_name(const char *kind, int idx, const std::string &topic) {
+    std::string n = std::string(kind) + " " + std::to_string(idx + 1);
+    if (!topic.empty()) n += " ('" + topic + "')";
+    return n;
+}
+
+// A half-band stage writes in.size()/2 outputs and needs an even input (HalfBandDecimator::decimate; the reference is undefined
+// otherwise), and every length the library stores per callback is moved in 16-byte pieces (k3_carry, float4 loads and stores),
+// so it must be even too: the n per-callback lengths len, len/2, .., len/2^stages must all be even.
+static bool even_cascade(int len, int stages, const std::string &name) {
+    for (int a = 0; a < stages; a++, len /= 2)
+        if (len % 2 != 0) {
+            set_error("plan: " + name + ": half-band stage " + std::to_string(a + 1) + " would get " + std::to_string(len) +
+                      " samples per callback, an odd count");
+            return false;
+        }
+    if (len % 2 != 0) {
+        set_error("plan: " + name + " would store " + std::to_string(len) + " samples per callback; stored lengths must be even");
+        return false;
+    }
+    return true;
+}
+
 // Shared tail of both constructors: derive rates/sizes, build tables, validate.
 static int finish_plan(HostPlan &p) {
     if (p.fs <= 0 || p.block <= 0 || p.mains.empty()) {
@@ -156,8 +179,18 @@ static int finish_plan(HostPlan &p) {
         return SDRB_E_INVALID;
     }
     for (MainVfo &m : p.mains) {
-        if (m.decim < 0 || m.decim > 3) {
-            set_error("plan: main VFO needs 0..3 half-band stages (out_rate >= sample_rate/8)");
+        const std::string name = vfo_name("main VFO", (int)(&m - p.mains.data()), m.topic);
+        if (m.decim < 0 || m.decim > MAX_DECIM) {                  // vfo::decimate[9] (vfo.h:39)
+            set_error("plan: " + name + " needs 0..8 half-band stages (out_rate >= sample_rate/256), not " +
+                      std::to_string(m.decim));
+            return SDRB_E_INVALID;
+        }
+        if (!even_cascade(p.block, m.decim, name)) return SDRB_E_INVALID;
+        // stages 4.. run on k1_v2's third-stage output; its tail kernel reaches up to 364 staged samples back, which must lie in the
+        // previous callback's body, not across that callback's own head
+        if (m.decim > 3 && (p.block >> 3) < MAIN_STAGE_MIN) {
+            set_error("plan: " + name + " with more than 3 half-band stages needs at least " + std::to_string(MAIN_STAGE_MIN * 8) +
+                      " samples per callback");
             return SDRB_E_INVALID;
         }
         m.out_rate = (int)(p.fs / std::pow(2, m.decim));               // vfo::getOutRate
@@ -186,14 +219,12 @@ static int finish_plan(HostPlan &p) {
                       std::to_string(s.block_in) + " samples per callback, its main VFO writes " + std::to_string(m.block_out) + ")");
             return SDRB_E_INVALID;
         }
-        if (s.decim < 0 || s.decim > 5 || (s.late != 0 && s.late != 5 && s.late != 6)) {
-            set_error("plan: sub VFO '" + s.topic + "' needs 0..5 half-band stages and late in {0,5,6}");
+        if (s.decim < 0 || s.decim > MAX_DECIM || (s.late != 0 && s.late != 5 && s.late != 6)) {
+            set_error("plan: sub VFO '" + s.topic + "' needs 0..8 half-band stages and late in {0,5,6} (it has " +
+                      std::to_string(s.decim) + " stages, late " + std::to_string(s.late) + ")");
             return SDRB_E_INVALID;
         }
-        if (s.block_in % 32 != 0 || ((s.block_in >> s.decim) << s.decim) != s.block_in) {
-            set_error("plan: sub VFO callback size must be a multiple of 32");
-            return SDRB_E_INVALID;
-        }
+        if (!even_cascade(s.block_in, s.decim, "sub VFO '" + s.topic + "'")) return SDRB_E_INVALID;
         int rate = (int)(s.fs / std::pow(2, s.decim));                  // vfo.cpp:65-66
         s.block_z = (int)(s.block_in / std::pow(2, s.decim));
         s.samples_out = s.block_z;
@@ -204,6 +235,11 @@ static int finish_plan(HostPlan &p) {
                 return SDRB_E_INVALID;
             }
             s.samples_out = s.block_z / s.late;
+            if (s.samples_out % 2 != 0) {
+                set_error("plan: sub VFO '" + s.topic + "' would store " + std::to_string(s.samples_out) +
+                          " samples per callback after its /late FIR; stored lengths must be even");
+                return SDRB_E_INVALID;
+            }
             const int rc = low_pass_hamming(2, rate * s.late, rate / 2, (double)rate / (s.late - 1), s.dec_taps);
             if (rc < 0) return rc;
         }
