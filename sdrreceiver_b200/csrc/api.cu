@@ -260,12 +260,6 @@ struct sdrb_bank {
     DevBuf k3_rrel;
     bool per_cb = false;                          // SDRB_PER_CB=1: device-resident calls launch every kernel class per callback
     bool k1_bulk = true;                          // k1_v2 (64-thread CTAs) prefetches tiles with cp.async.bulk + mbarrier; SDRB_K1_BULK=0: per-thread cp.async records
-    bool k3_xs200 = false;                        // SDRB_K3_XS200=1: staged input also at the 200-register cap
-    int k3_ws = 0;                                // SDRB_K3_WS=1|2: warp-specialised k2a_v3ws (producer + consumer warp per CTA)
-    int k3_cta_warps = K3_WARPS;                  // warps per k2a_v3 CTA (SDRB_K3_CTA_WARPS=1..4)
-    int k3_cta_warps2 = 0;                        // ... of the groups with at most 3 stages (SDRB_K3_CTA_WARPS2=1..12; 0 = the size with the most resident warps): their 160-register warps fit
-                                                  // three to a scheduler, shared memory per CTA (the rotation table is per CTA) decides
-    int k3_regs5 = 200;                           // register cap of the 5-stage k2a_v3 instantiation (SDRB_K3_REGS=168|200|232|255; 200..255 all hold two warps per scheduler)
     int dbg_only = 0;                             // SDRB_DEBUG_ONLY=dc|filters: profiling aid, device-resident calls skip the other half (results are then meaningless)
     DevBuf cascdev, rfdev, latedev, usbdev, carry;
     std::vector<SubGroup> groups;
@@ -706,17 +700,9 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
             kp.nsw = g.v3_nsw;
         }
         BANK_CU(cudaMemcpy(b->k3_rrel.p, rrel.data(), sizeof(float2) * rrel.size(), cudaMemcpyHostToDevice));
-#define K3_ATTR(S_, R_, X_) BANK_CU((cudaFuncSetAttribute(k2a_v3<S_, R_, X_>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)))
-        K3_ATTR(2, 168, false); K3_ATTR(3, 168, false); K3_ATTR(5, 168, false); K3_ATTR(5, 200, false); K3_ATTR(5, 200, true); K3_ATTR(5, 232, true); K3_ATTR(5, 255, false);
-#undef K3_ATTR
-#define K3W_ATTR(S_, R_, X_) BANK_CU((cudaFuncSetAttribute(k2a_v3ws<S_, R_, X_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k3ws_cta_smem_bytes(K3_MAX_VFO, 32, 8))))
-        K3W_ATTR(2, 168, false); K3W_ATTR(3, 168, false); K3W_ATTR(5, 168, false); K3W_ATTR(5, 168, true);
-#undef K3W_ATTR
-        if (const char *e = getenv("SDRB_K3_WS")) b->k3_ws = atoi(e);
-        b->k3_xs200 = getenv("SDRB_K3_XS200") && atoi(getenv("SDRB_K3_XS200")) != 0;
-        if (const char *e = getenv("SDRB_K3_CTA_WARPS")) { const int v = atoi(e); if (v >= 1 && v <= 4) b->k3_cta_warps = v; }
-        if (const char *e = getenv("SDRB_K3_CTA_WARPS2")) { const int v = atoi(e); if (v >= 1 && v <= 12) b->k3_cta_warps2 = v; }
-        if (const char *e = getenv("SDRB_K3_REGS")) { const int v = atoi(e); if (v == 168 || v == 200 || v == 232 || v == 255) b->k3_regs5 = v; }
+        BANK_CU(cudaFuncSetAttribute(k2a_v3<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        BANK_CU(cudaFuncSetAttribute(k2a_v3<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        BANK_CU(cudaFuncSetAttribute(k2a_v3<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     }
     if (!latedev.empty()) BANK_CU(cudaMemcpy(b->latedev.p, latedev.data(), sizeof(LateDev) * latedev.size(), cudaMemcpyHostToDevice));
     if (!usbdev.empty()) BANK_CU(cudaMemcpy(b->usbdev.p, usbdev.data(), sizeof(UsbDev) * usbdev.size(), cudaMemcpyHostToDevice));
@@ -880,15 +866,13 @@ static int enqueue_ingest_cb(sdrb_bank *b, const CallCtx &c, int s0, int ns, cud
 }
 
 // k2a_v3 launch geometry: one warp per (stream group, span, callback). `slots` = CTAs of this kernel the device holds at once
-// (occupancy x SM count): the spans are chosen so that the grid is just under SDRB_K3_WAVES (default 2) full waves of it -- the
+// (occupancy x SM count): the spans are chosen so that the grid is just under two full waves of it -- the
 // 5-stage kernel holds 4 CTAs per SM (two 200-register warps per scheduler), and a grid of 2.4 waves left the last third of its run
 // 60 % empty (profiles/r02_experiments.md section 1). Never shorter than 16 tiles: 3 warm-up tiles are recomputed per span.
 static void k3_geometry(const SubGroup &g, K3Params &kp, int ns, int ncb, int cta_warps, int slots, dim3 *grid) {
     const int sgroups = (ns + g.v3_nsw - 1) / g.v3_nsw;
     const int ctas_x = (sgroups + cta_warps - 1) / cta_warps;
-    static const int waves = [] { const char *e = getenv("SDRB_K3_WAVES"); const int v = e ? atoi(e) : 0; return v > 0 ? v : 2; }();
-    int target_ctas = slots > 0 ? waves * slots : 148 * 10;
-    if (const char *e = getenv("SDRB_K3_WARPS")) { const int v = atoi(e); if (v > 0) target_ctas = v / cta_warps; }
+    const int target_ctas = slots > 0 ? 2 * slots : 148 * 10;
     int spans = std::max(1, target_ctas / std::max(1, ctas_x * ncb));
     int tps = std::max(16, (kp.n_tiles + spans - 1) / spans);
     tps = std::min(tps, kp.n_tiles);
@@ -903,6 +887,33 @@ static int k3_slots(K kernel, int threads, size_t smem) {
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem) != cudaSuccess) return 0;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     return per_sm * sms;
+}
+
+// One k2a_v3 launch for sub-VFO group gi. First launch of the group: CTA size and resident CTAs. The 5-stage kernel holds two warps
+// per scheduler whatever the CTA size (registers); the shorter cascades fit three, and how many CTAs fit is a matter of shared memory
+// (the rotation table is per CTA, a ring per warp): take the CTA size with the most resident warps (25E's 15 two-stage VFOs: 6 warps,
+// 12 per SM).
+template <int MAXS>
+static void launch_k3(sdrb_bank *b, size_t gi, int ns, int ncb, cudaStream_t st) {
+    const SubGroup &g = b->groups[gi];
+    K3Params &kp = b->k3[gi];
+    int &slots = b->k3_slots[gi], &cw = b->k3_cw[gi];
+    const int rows = g.v3_nsw * g.count;
+    if (slots < 0) {
+        cw = K3_WARPS;
+        if (MAXS <= 3) {
+            int best = 0;
+            for (int c : {2, 3, 4, 6}) {
+                const int w = c * k3_slots(k2a_v3<MAXS>, c * 32, k3_cta_smem_bytes(g.count, c, rows));
+                if (w > best) { best = w; cw = c; }
+            }
+        }
+        slots = k3_slots(k2a_v3<MAXS>, cw * 32, k3_cta_smem_bytes(g.count, cw, rows));
+    }
+    dim3 grid;
+    k3_geometry(g, kp, ns, ncb, cw, slots, &grid);
+    TimedScope t(b, st, 2);
+    k2a_v3<MAXS><<<grid, cw * 32, k3_cta_smem_bytes(g.count, cw, rows), st>>>(kp);
 }
 
 // The half-band stages of the deep main VFOs (subs = false, timed with the ingest class) or sub VFOs (timed with the cascades)
@@ -924,58 +935,10 @@ static int enqueue_subs(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaStre
         if (g.v3) {
             K3Params &kp = b->k3[gi];
             kp.stream0 = s0; kp.stream_end = s0 + ns; kp.b0 = cb0;
-            if (b->k3_ws) {
-                // warp-specialised pair per CTA (kernels_v3.cuh: k2a_v3ws); SDRB_K3_WS=2: with staged input for the 5-stage groups
-                dim3 grid;
-                k3_geometry(g, kp, ns, ncb, 1, 0, &grid);
-                const bool xs = b->k3_ws == 2 && g.v3_maxs == 5;
-                const size_t smem = k3ws_cta_smem_bytes(g.count, g.v3_nsw * g.count, xs ? g.v3_nsw : 0);
-                TimedScope t(b, st, 2);
-                if (g.v3_maxs == 2) k2a_v3ws<2, 168, false><<<grid, 64, smem, st>>>(kp);
-                else if (g.v3_maxs == 3) k2a_v3ws<3, 168, false><<<grid, 64, smem, st>>>(kp);
-                else if (xs) k2a_v3ws<5, 168, true><<<grid, 64, smem, st>>>(kp);
-                else k2a_v3ws<5, 168, false><<<grid, 64, smem, st>>>(kp);
-                (*nl)++;
-                continue;
-            }
-            dim3 grid;
-            // staged input (bulk copies) only where registers, not shared memory, set the number of resident CTAs
-            const bool xs = g.v3_maxs == 5 && (b->k3_regs5 == 232 || b->k3_xs200);
             if (b->k3_slots.size() <= gi) { b->k3_slots.resize(gi + 1, -1); b->k3_cw.resize(gi + 1, 0); }
-            int &slots = b->k3_slots[gi];
-            int &cw = b->k3_cw[gi];
-            size_t smem = 0;
-            // First launch of the group: CTA size and resident CTAs. The 5-stage kernels hold two warps per scheduler whatever the CTA
-            // size (registers); the shorter cascades fit three, and how many CTAs fit is a matter of shared memory (the rotation table is
-            // per CTA, a ring per warp): take the CTA size with the most resident warps (25E's 15 two-stage VFOs: 6 warps, 12 per SM).
-#define K3_GO(S_, R_, X_)                                                                                   \
-    do {                                                                                                    \
-        if (slots < 0) {                                                                                    \
-            cw = g.v3_maxs <= 3 ? b->k3_cta_warps2 : b->k3_cta_warps;                                       \
-            if (cw == 0) {                                                                                  \
-                int best = 0;                                                                               \
-                for (int c : {2, 3, 4, 6}) {                                                                \
-                    const int w = c * k3_slots(k2a_v3<S_, R_, X_>, c * 32,                                  \
-                                               k3_cta_smem_bytes(g.count, c, g.v3_nsw * g.count, xs ? g.v3_nsw : 0)); \
-                    if (w > best) { best = w; cw = c; }                                                     \
-                }                                                                                           \
-                if (cw == 0) cw = K3_WARPS;                                                                 \
-            }                                                                                               \
-            slots = k3_slots(k2a_v3<S_, R_, X_>, cw * 32, k3_cta_smem_bytes(g.count, cw, g.v3_nsw * g.count, xs ? g.v3_nsw : 0)); \
-        }                                                                                                   \
-        smem = k3_cta_smem_bytes(g.count, cw, g.v3_nsw * g.count, xs ? g.v3_nsw : 0);                       \
-        k3_geometry(g, kp, ns, ncb, cw, slots, &grid);                                                      \
-        TimedScope t(b, st, 2);                                                                             \
-        k2a_v3<S_, R_, X_><<<grid, cw * 32, smem, st>>>(kp);                                                \
-    } while (0)
-            if (g.v3_maxs == 2) K3_GO(2, 168, false);
-            else if (g.v3_maxs == 3) K3_GO(3, 168, false);
-            else if (b->k3_regs5 == 232) K3_GO(5, 232, true);
-            else if (b->k3_regs5 == 255) K3_GO(5, 255, false);
-            else if (b->k3_regs5 == 200 && b->k3_xs200) K3_GO(5, 200, true);
-            else if (b->k3_regs5 == 200) K3_GO(5, 200, false);
-            else K3_GO(5, 168, false);
-#undef K3_GO
+            if (g.v3_maxs == 2) launch_k3<2>(b, gi, ns, ncb, st);
+            else if (g.v3_maxs == 3) launch_k3<3>(b, gi, ns, ncb, st);
+            else launch_k3<5>(b, gi, ns, ncb, st);
             (*nl)++;
             continue;
         }

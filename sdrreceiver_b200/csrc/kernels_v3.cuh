@@ -43,7 +43,6 @@ constexpr int K3_WARM = 3;              // warm-up tiles in front of a span (>= 
 constexpr int K3_MAX_VFO = 16;
 constexpr int K3_LUT_STEADY = 512;      // table entries of the start-up transient (94 measured)
 constexpr int K3_MAX_SLOTS = K3_MAX_VFO * 32;
-constexpr int K3_XS = K3_TILE + 16;     // staged input samples per stream and tile: 16 in front (the windows reach back 12), then the tile
 
 #ifndef HB_P0
 #define HB_P0 0.0060431029837374152f
@@ -53,18 +52,6 @@ constexpr int K3_XS = K3_TILE + 16;     // staged input samples per stream and t
 #endif
 
 #define K3_HD __host__ __device__ __forceinline__
-// tuning switches of the VFO loop of role A (tools/k3_variants.sh builds the alternatives)
-#ifndef K3_PIPE
-#define K3_PIPE 1            /* 1: rotation-table pair and anchors of VFO v+1 are read while VFO v is computed */
-#endif
-#ifndef K3_PACKED_CMUL
-#define K3_PACKED_CMUL 1
-#endif
-#ifndef K3_VFO_UNROLL
-#define K3_VFO_UNROLL 4
-#endif
-#define K3_STR2(x) #x
-#define K3_STR(x) K3_STR2(x)
 
 struct K3Vfo {
     const float2 *lut;          // Oscillator table
@@ -135,7 +122,7 @@ K3_HD float2 k3_splat(float v) { return make_float2(v, v); }
 // complex product a * b. Device: two packed operations -- b * (a.x, a.x), then (-b.y, b.x) * (a.y, a.y) added: ptxas folds the
 // half swap, the per-half sign and the broadcast of the scalar into the operands of FMUL2 / FFMA2 (no extra registers or moves)
 K3_HD float2 k3_cmul(float2 a, float2 b) {
-#if defined(__CUDA_ARCH__) && K3_PACKED_CMUL
+#ifdef __CUDA_ARCH__
     unsigned long long r, bx = *reinterpret_cast<unsigned long long *>(&b);
     float2 sx = make_float2(a.x, a.x), sy = make_float2(a.y, a.y), bs = make_float2(-b.y, b.x);
     asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(bx), "l"(*reinterpret_cast<unsigned long long *>(&sx)));
@@ -196,14 +183,12 @@ struct K3Hist {
 };
 
 // Shared memory of a CTA: [rrel: count*64 float2][slot table: K3_MAX_SLOTS ushort][per warp: ring of `rows` rows,
-// 32 dst pointers, 2 x 32 table anchors (float2), 32 per-stream table bases (int2), nsw staged input tiles of K3_XS samples,
-// one mbarrier]
-K3_HD size_t k3_warp_smem_bytes(int rows, int nsw) {          // nsw = 0: no staged input
-    return (size_t)rows * K3_ROW * sizeof(float2) + 32 * sizeof(float2 *) + 64 * sizeof(float2) + 32 * sizeof(int2) +
-           (size_t)nsw * K3_XS * sizeof(float2) + 16;
+// 32 dst pointers, 2 x 32 table anchors (float2), 32 per-stream table bases (int2)]
+K3_HD size_t k3_warp_smem_bytes(int rows) {
+    return (size_t)rows * K3_ROW * sizeof(float2) + 32 * sizeof(float2 *) + 64 * sizeof(float2) + 32 * sizeof(int2);
 }
-K3_HD size_t k3_cta_smem_bytes(int count, int warps, int rows, int nsw) {
-    return (size_t)count * K3_OUT1 * sizeof(float2) + K3_MAX_SLOTS * sizeof(unsigned short) + (size_t)warps * k3_warp_smem_bytes(rows, nsw);
+K3_HD size_t k3_cta_smem_bytes(int count, int warps, int rows) {
+    return (size_t)count * K3_OUT1 * sizeof(float2) + K3_MAX_SLOTS * sizeof(unsigned short) + (size_t)warps * k3_warp_smem_bytes(rows);
 }
 // 8 bytes global -> shared without passing through a register (LDGSTS); k3_async_wait() makes them visible to the issuing thread
 K3_HD void k3_async_copy8(void *smem, const void *gmem) {
@@ -239,16 +224,11 @@ K3_HD void k3_prefetch_l1(const void *p) {
 //   ring    32 rows of K3_ROW float2, private to the warp
 //   sdst    32 pointers, private to the warp
 //   srrel   the CTA's copy of p.rrel;  stab: slot table (v << 8 | 16-byte chunk), n_slots entries per stream
-// XS: the input tiles are staged in shared memory by the bulk-copy engine (worth it when the extra 1.2 KB per stream do not
-// cost a resident CTA: the 5-stage instantiation, which registers limit to 8 warps per SM); otherwise the lanes load their
-// windows from global memory, the lines prefetched into L1 one tile ahead.
-// ROLE: 0 = one warp plays both roles in turn (role A, warp barrier, role B); 1 / 2 = warp-specialised pair: this warp is the
-// producer (role A only, writes tile i into ring buffer i & 1) or the consumer (role B and the output copy only); the two hand the
-// buffers over with env.signal_/wait_ full/empty (named barriers of the CTA). A warp then holds only its role's registers
-// (the histories live in the consumer, the sums and differences in the producer) and tile i+1 is produced while tile i is filtered.
-template <int MAXS, bool XS, int ROLE, class Env>
+// The warp plays both roles in turn (role A, warp barrier, role B). The lanes load their windows from global memory, the lines
+// prefetched into L1 one tile ahead.
+template <int MAXS, class Env>
 K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 *ring, float2 **sdst, float2 *sF, int2 *sK,
-                   float2 *sX, const float2 *srrel, const unsigned short *stab, int n_slots) {
+                   const float2 *srrel, const unsigned short *stab, int n_slots) {
     const int lane = env.lane;
     const int nv = p.count, nsw = p.nsw, B = p.block_in, L = p.lut_len;
     const int sbase = p.stream0 + sg * nsw;
@@ -269,9 +249,8 @@ K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 
         H.h4[i] = make_float2(0.f, 0.f); H.h5[i] = make_float2(0.f, 0.f);
     }
     const int SBw = rowB ? SB : 0;
-    const int ring_buf = nsw * nv * K3_ROW;                       // float2 per ring buffer (ROLE 1/2: two buffers)
     // per stream of the warp: table index of callback coordinate 0 and "this callback starts the stream" (oscillator.cpp:26-30)
-    if (ROLE != 2 && lane < nsw) {
+    if (lane < nsw) {
         int kb = 0, zero = 0;
         if (sbase + lane < p.stream_end) {
             const long long blk = k3_ldg(p.blocks_done + sbase + lane) + b;
@@ -282,29 +261,17 @@ K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 
     }
     env.sync();
     const float2 *lutB = p.v[rowB ? vB : 0].lut;
-    const int kbB = ROLE != 2 ? sK[rowB ? sB : 0].x : 0;
+    const int kbB = sK[rowB ? sB : 0].x;
     auto wrapL = [L](int k) { if (k < 0) k += L; if (k >= L) k -= L; return k; };
     // the table entry of this row's (stream, VFO) at the first sample of a tile travels global -> shared one tile ahead
     // (sF is two buffers of 32 entries): no register holds it while the previous tile is being worked on
-    if (ROLE != 2) k3_async_copy8(sF + lane, lutB + wrapL(kbB + (t_begin - K3_WARM) * K3_TILE));
+    k3_async_copy8(sF + lane, lutB + wrapL(kbB + (t_begin - K3_WARM) * K3_TILE));
     int fpar = 0;
     const float2 *in0 = p.in + (size_t)sbase * (size_t)p.in_stride + p.hist_in + (long long)b * B;         // sample 0 of stream sbase
-    // The input of a tile (K3_XS samples per stream: 16 in front of the tile, then the tile) is staged in shared memory by the
-    // bulk-copy engine one tile ahead: one lane issues one copy per stream when role A has consumed the previous tile, the
-    // bytes land while role B runs, everybody waits on the warp's mbarrier at the next tile head.
     int n_str = 0;
     for (int s = 0; s < nsw && sbase + s < p.stream_end; ++s) n_str++;
-    auto stage_x = [&](int c_first) {
-        if (XS && ROLE != 2 && lane == 0) {
-            env.x_expect((unsigned)(n_str * K3_XS * sizeof(float2)));
-            for (int s = 0; s < n_str; ++s)
-                env.x_copy(sX + s * K3_XS, in0 + (size_t)s * (size_t)p.in_stride + c_first - 16, (unsigned)(K3_XS * sizeof(float2)));
-        }
-    };
-    stage_x((t_begin - K3_WARM) * K3_TILE);
-    unsigned xpar = 0;
-    const float2 *in_pf = in0 + K3_TILE - 16 + 16 * lane;                                                  // !XS: this lane's line of the next tile
-    const float2 *in_ln = in0 + 4 * lane;                                                                  // !XS: this lane's chunk of a tile
+    const float2 *in_pf = in0 + K3_TILE - 16 + 16 * lane;                                                  // this lane's line of the next tile
+    const float2 *in_ln = in0 + 4 * lane;                                                                  // this lane's chunk of a tile
     // Output copy, common case (at most 32 sixteen-byte chunks per stream and tile): this lane's chunk is the same for every
     // tile and stream, so its source offset and destination are kept in registers instead of being looked up per tile.
     const bool cp_fast = n_slots <= 32;
@@ -320,26 +287,18 @@ K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 
 
     for (int t = t_begin - K3_WARM; t < t_end; ++t) {
         const int c0 = t * K3_TILE;                          // callback coordinate of the tile's first sample (may be negative)
-        const int ti = t - (t_begin - K3_WARM);              // tile counter of this unit
-        float2 *rbuf = ring + (ROLE == 0 ? 0 : (ti & 1) * ring_buf);
         const float2 *sFt = sF + 32 * fpar;                  // this tile's anchors
-        if (ROLE != 2) {
         k3_async_wait();
-        if (XS) {
-            env.x_wait(xpar);
-            xpar ^= 1u;
-        }
         env.sync();
         fpar ^= 1;
         k3_async_copy8(sF + 32 * fpar + lane, lutB + wrapL(kbB + c0 + K3_TILE));
         // The coming tile's lines into L1 (10 x 128 bytes cover 128 + 14 samples). Measured and not kept (profiles/r02_experiments.md
         // section 1): a request per 32-byte sector, real "touch" loads instead of the prefetch instruction, the first stream's loads
         // hoisted above the barrier, staged input -- none of them moves the kernel's time.
-        if (!XS && t + 1 < t_end && lane < 10) {
+        if (t + 1 < t_end && lane < 10) {
             const float2 *pf = in_pf + c0;
             for (int s = 0; s < n_str; ++s, pf += p.in_stride) k3_prefetch_l1(pf);
         }
-        if (ROLE == 1 && ti >= 2) env.wait_empty(ti & 1);    // the consumer is done with the tile that used this buffer
         // =============================== role A ===============================
         for (int s0 = 0; s0 < nsw; s0 += 2) {
             const int strA = sbase + s0, strB = sbase + s0 + 1;
@@ -348,10 +307,9 @@ K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 
             const int kaA = wrapL(baseA.x + c0), kaB = wrapL(baseB.x + c0);      // table index of sample c0
             const bool fastA = c0 != 0 && kaA >= K3_LUT_STEADY + 16 && kaA + K3_TILE + 8 <= L;
             const bool fastB = c0 != 0 && kaB >= K3_LUT_STEADY + 16 && kaB + K3_TILE + 8 <= L;
-            // staged samples of the two streams: index i of a stream's buffer is sample c0 - 16 + i
-            const float2 *inA = XS ? sX + s0 * K3_XS + 16 + 4 * lane : in_ln + (size_t)s0 * (size_t)p.in_stride + c0;
-            const float2 *inB = XS ? sX + (hasB ? s0 + 1 : s0) * K3_XS + 16 + 4 * lane
-                                   : in_ln + (size_t)(hasB ? s0 + 1 : s0) * (size_t)p.in_stride + c0;
+            // sample c0 + 4l of the two streams
+            const float2 *inA = in_ln + (size_t)s0 * (size_t)p.in_stride + c0;
+            const float2 *inB = in_ln + (size_t)(hasB ? s0 + 1 : s0) * (size_t)p.in_stride + c0;
             if (env.all(fastA && fastB)) {              // a vote: the compiler then knows the branch (and the VFO loop in it) is warp-uniform
                 // ---- sums and differences, once for all VFOs ----
                 // x[i] = sample c0 + 4l - 10 + i; outputs m' = 0, 1 have centres i = 5, 7
@@ -363,7 +321,7 @@ K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 
                     const bool has = q ? hasB : hasA;
 #pragma unroll
                     for (int i = 0; i < 7; ++i) {
-                        const float4 v = has ? (XS ? xp[i] : k3_ldg(xp + i)) : make_float4(0.f, 0.f, 0.f, 0.f);
+                        const float4 v = has ? k3_ldg(xp + i) : make_float4(0.f, 0.f, 0.f, 0.f);
                         x[2 * i] = make_float2(v.x, v.y);
                         x[2 * i + 1] = make_float2(v.z, v.w);
                     }
@@ -384,16 +342,11 @@ K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 
                 // software pipeline: the rotation-table pair and the anchors of VFO v+1 are fetched while VFO v is computed
                 float4 rr_n = *reinterpret_cast<const float4 *>(srrel + 2 * lane);
                 float2 FA_n = sFt[s0 * nv], FB_n = sFt[(hasB ? s0 + 1 : s0) * nv];
-_Pragma(K3_STR(unroll K3_VFO_UNROLL))
+#pragma unroll 4
                 for (int v = 0; v < nv; ++v) {
-#if K3_PIPE
                     const float4 rr = rr_n;
                     const float2 FA = FA_n, FB = FB_n;
-#else
-                    const float4 rr = *reinterpret_cast<const float4 *>(srrel + v * K3_OUT1 + 2 * lane);
-                    const float2 FA = sFt[s0 * nv + v], FB = sFt[(hasB ? s0 + 1 : s0) * nv + v];
-#endif
-                    if (K3_PIPE && v + 1 < nv) {
+                    if (v + 1 < nv) {
                         rr_n = *reinterpret_cast<const float4 *>(srrel + (v + 1) * K3_OUT1 + 2 * lane);
                         FA_n = sFt[s0 * nv + v + 1];
                         FB_n = sFt[(hasB ? s0 + 1 : s0) * nv + v + 1];
@@ -435,7 +388,7 @@ _Pragma(K3_STR(unroll K3_VFO_UNROLL))
                     for (int q = 0; q < 2; ++q) {
                         const float2 o0 = k3_cmul(G[q][0], acc[q][0]), o1 = k3_cmul(G[q][1], acc[q][1]);
                         if (q ? hasB : hasA)
-                            *reinterpret_cast<float4 *>(rbuf + ((s0 + q) * nv + v) * K3_ROW + 2 * lane) = make_float4(o0.x, o0.y, o1.x, o1.y);
+                            *reinterpret_cast<float4 *>(ring + ((s0 + q) * nv + v) * K3_ROW + 2 * lane) = make_float4(o0.x, o0.y, o1.x, o1.y);
                     }
                 }
             } else {
@@ -449,7 +402,7 @@ _Pragma(K3_STR(unroll K3_VFO_UNROLL))
                     float2 xe[16];                                           // xe[i] = sample c0 + 4l - 12 + i
 #pragma unroll
                     for (int i = 0; i < 8; ++i) {
-                        const float4 v = XS ? xp[i] : k3_ldg(xp + i);
+                        const float4 v = k3_ldg(xp + i);
                         xe[2 * i] = make_float2(v.x, v.y);
                         xe[2 * i + 1] = make_float2(v.z, v.w);
                     }
@@ -471,21 +424,16 @@ _Pragma(K3_STR(unroll K3_VFO_UNROLL))
                         float2 o1 = k3_hb(u[2], u[4], u[6], u[7], u[8], u[10], u[12]);
                         o0 = make_float2(o0.x * sc, o0.y * sc);
                         o1 = make_float2(o1.x * sc, o1.y * sc);
-                        *reinterpret_cast<float4 *>(rbuf + ((s0 + q) * nv + v) * K3_ROW + 2 * lane) = make_float4(o0.x, o0.y, o1.x, o1.y);
+                        *reinterpret_cast<float4 *>(ring + ((s0 + q) * nv + v) * K3_ROW + 2 * lane) = make_float4(o0.x, o0.y, o1.x, o1.y);
                     }
                 }
             }
         }
         env.sync();
-        if (XS && t + 1 < t_end) stage_x(c0 + K3_TILE);      // role A has read this tile's samples: the next tile's may land
-        if (ROLE == 1) env.signal_full(ti & 1);
-        }                                                    // ROLE != 2
         // =============================== role B ===============================
-        if (ROLE != 1) {
-        if (ROLE == 2) env.wait_full(ti & 1);
         // lanes without a row store nothing and read the (read-only, >= 64 entries) rotation table instead of somebody's row: a row is
         // rewritten in place by its owner while it is read, and a second reader would be a data race (compute-sanitizer racecheck)
-        const float2 *myrow = rowB ? rbuf + lane * K3_ROW : srrel;
+        const float2 *myrow = rowB ? ring + lane * K3_ROW : srrel;
         if (c0 == 0) {
             k3_head_shift(H.h2);
             if (MAXS > 2) k3_head_shift(H.h3);
@@ -495,7 +443,7 @@ _Pragma(K3_STR(unroll K3_VFO_UNROLL))
 #pragma unroll
         for (int sub = 0; sub < K3_OUT1 / 16; ++sub) {
             const float4 *rp = reinterpret_cast<const float4 *>(myrow + 16 * sub);
-            float2 *wr = rbuf + (rowB ? lane : 0) * K3_ROW;  // outputs go to the front of the row (always behind the read position)
+            float2 *wr = ring + (rowB ? lane : 0) * K3_ROW;  // outputs go to the front of the row (always behind the read position)
             if (MAXS >= 2) {
                 // stage 2 in two halves of 8 inputs: only half of the 16 first-stage samples is in registers at any time
                 float2 o2[8];
@@ -545,7 +493,7 @@ _Pragma(K3_STR(unroll K3_VFO_UNROLL))
                 if (lane < n_slots) {
                     const long long adv = ((long long)t * K3_OUT1) >> cp_shift;      // out1 index 64 t -> index of the VFO's own output
                     for (int s = 0; s < nsw && sbase + s < p.stream_end; ++s) {
-                        const float4 v = *reinterpret_cast<const float4 *>(rbuf + s * nv * K3_ROW + cp_src);
+                        const float4 v = *reinterpret_cast<const float4 *>(ring + s * nv * K3_ROW + cp_src);
                         k3_store_global16(cp_dst + (size_t)s * (size_t)p.out_stride + adv, v);
                     }
                 }
@@ -569,7 +517,7 @@ _Pragma(K3_STR(unroll K3_VFO_UNROLL))
 #pragma unroll
                         for (int u = 0; u < 4; ++u) {
                             const int r = s * nv + (e[u] >= 0 ? (e[u] >> 8) : 0), ch = e[u] >= 0 ? (e[u] & 0xff) : 0;
-                            v[u] = *reinterpret_cast<const float4 *>(rbuf + r * K3_ROW + 2 * ch);
+                            v[u] = *reinterpret_cast<const float4 *>(ring + r * K3_ROW + 2 * ch);
                             d[u] = sdst[r] + 2 * ch;
                         }
 #pragma unroll
@@ -579,57 +527,25 @@ _Pragma(K3_STR(unroll K3_VFO_UNROLL))
                 }
             }
         }
-        if (ROLE == 2) {
-            env.sync();
-            env.signal_empty(ti & 1);
-        }
-        }                                                    // ROLE != 1
-        if (ROLE == 0) env.sync();
+        env.sync();
     }
 }
 
 #ifdef __CUDACC__
 struct K3DevEnv {
     int lane;
-    unsigned long long *xbar;                              // the warp's mbarrier of the staged input
     __device__ __forceinline__ void sync() { __syncwarp(); }
     __device__ __forceinline__ bool all(bool v) { return __all_sync(0xffffffffu, v) != 0; }
-    // producer/consumer hand-over of the two ring buffers (ROLE 1/2): named barriers 1..4 of the 64-thread CTA, the signalling warp
-    // arrives, the waiting warp syncs (64 = both warps)
-    __device__ __forceinline__ void signal_full(int buf) { asm volatile("bar.arrive %0, 64;\n" ::"r"(1 + buf) : "memory"); }
-    __device__ __forceinline__ void wait_full(int buf) { asm volatile("bar.sync %0, 64;\n" ::"r"(1 + buf) : "memory"); }
-    __device__ __forceinline__ void signal_empty(int buf) { asm volatile("bar.arrive %0, 64;\n" ::"r"(3 + buf) : "memory"); }
-    __device__ __forceinline__ void wait_empty(int buf) { asm volatile("bar.sync %0, 64;\n" ::"r"(3 + buf) : "memory"); }
-    __device__ __forceinline__ void x_expect(unsigned bytes) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"((unsigned)__cvta_generic_to_shared(xbar)), "r"(bytes) : "memory");
-    }
-    __device__ __forceinline__ void x_copy(void *smem, const void *gmem, unsigned bytes) {
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n" ::"r"(
-                         (unsigned)__cvta_generic_to_shared(smem)),
-                     "l"(gmem), "r"(bytes), "r"((unsigned)__cvta_generic_to_shared(xbar))
-                     : "memory");
-    }
-    __device__ __forceinline__ void x_wait(unsigned parity) {
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "K3WAIT_%=:\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-            "@p bra K3DONE_%=;\n"
-            "bra K3WAIT_%=;\n"
-            "K3DONE_%=:\n"
-            "}\n" ::"r"((unsigned)__cvta_generic_to_shared(xbar)), "r"(parity) : "memory");
-    }
 };
 
 constexpr int K3_WARPS = 2;                                 // default warps per CTA; the kernel works with any CTA size (independent warps that
                                                             // only share the read-only tables)
 
-// grid: x = ceil(stream groups / K3_WARPS), y = spans, z = callbacks
-// RC = register cap: 168 (three warps per scheduler = 12 per SM, the deep cascades then spill a history array); 200, 232 and 255 all hold two
-// warps per scheduler = 8 per SM (the register file is per scheduler: 16384 registers), without spills
-template <int MAXS, int RC, bool XS>
-__global__ void __maxnreg__(RC) k2a_v3(const __grid_constant__ K3Params p) {
+// grid: x = ceil(stream groups / warps per CTA), y = spans, z = callbacks
+// Register cap: 168 for 2 and 3 stages (three warps per scheduler = 12 per SM). At 168 the 5-stage cascade spills a history array; at 200
+// it holds two warps per scheduler = 8 per SM (the register file is per scheduler: 16384 registers), without spills.
+template <int MAXS>
+__global__ void __maxnreg__(MAXS == 5 ? 200 : 168) k2a_v3(const __grid_constant__ K3Params p) {
     extern __shared__ __align__(16) unsigned char k3_smem[];
     float2 *srrel = reinterpret_cast<float2 *>(k3_smem);
     unsigned short *stab = reinterpret_cast<unsigned short *>(srrel + p.count * K3_OUT1);
@@ -645,58 +561,14 @@ __global__ void __maxnreg__(RC) k2a_v3(const __grid_constant__ K3Params p) {
     }
     __syncthreads();
     const int rows = p.nsw * p.count;
-    float2 *ring = reinterpret_cast<float2 *>(wbase + (size_t)warp * k3_warp_smem_bytes(rows, XS ? p.nsw : 0));
+    float2 *ring = reinterpret_cast<float2 *>(wbase + (size_t)warp * k3_warp_smem_bytes(rows));
     float2 **sdst = reinterpret_cast<float2 **>(ring + rows * K3_ROW);
     float2 *sF = reinterpret_cast<float2 *>(sdst + 32);
     int2 *sK = reinterpret_cast<int2 *>(sF + 64);
-    float2 *sX = reinterpret_cast<float2 *>(sK + 32);
-    unsigned long long *xbar = reinterpret_cast<unsigned long long *>(sX + (XS ? p.nsw : 0) * K3_XS);
-    if (lane == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;\n" ::"r"((unsigned)__cvta_generic_to_shared(xbar)));
-        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-    }
-    __syncwarp();
     const int sg = blockIdx.x * (int)(blockDim.x >> 5) + warp;
     if (p.stream0 + sg * p.nsw >= p.stream_end) return;
-    K3DevEnv env{lane, xbar};
-    k3_unit<MAXS, XS, 0>(env, p, sg, (int)blockIdx.y, p.b0 + (int)blockIdx.z, ring, sdst, sF, sK, sX, srrel, stab, n_slots);
-}
-// Warp-specialised form: a CTA is ONE unit of work handled by a producer warp (role A) and a consumer warp (role B) that hand two
-// ring buffers back and forth. grid: x = stream groups, y = spans, z = callbacks; 64 threads.
-K3_HD size_t k3ws_cta_smem_bytes(int count, int rows, int nsw) {
-    return (size_t)count * K3_OUT1 * sizeof(float2) + K3_MAX_SLOTS * sizeof(unsigned short) + (size_t)rows * K3_ROW * sizeof(float2) +
-           k3_warp_smem_bytes(rows, nsw);
-}
-template <int MAXS, int RC, bool XS>
-__global__ void __maxnreg__(RC) k2a_v3ws(const __grid_constant__ K3Params p) {
-    extern __shared__ __align__(16) unsigned char k3_smem[];
-    float2 *srrel = reinterpret_cast<float2 *>(k3_smem);
-    unsigned short *stab = reinterpret_cast<unsigned short *>(srrel + p.count * K3_OUT1);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    for (int e = threadIdx.x; e < p.count * K3_OUT1; e += blockDim.x) srrel[e] = p.rrel[e];
-    int n_slots = 0;
-    for (int v = 0; v < p.count; ++v) {
-        const int n = 32 >> (p.v[v].S - 1);
-        for (int c = threadIdx.x; c < n; c += blockDim.x) stab[n_slots + c] = (unsigned short)((v << 8) | c);
-        n_slots += n;
-    }
-    const int rows = p.nsw * p.count;
-    float2 *ring = reinterpret_cast<float2 *>(stab + K3_MAX_SLOTS);                // two buffers of `rows` rows
-    float2 **sdst = reinterpret_cast<float2 **>(ring + 2 * rows * K3_ROW);
-    float2 *sF = reinterpret_cast<float2 *>(sdst + 32);
-    int2 *sK = reinterpret_cast<int2 *>(sF + 64);
-    float2 *sX = reinterpret_cast<float2 *>(sK + 32);
-    unsigned long long *xbar = reinterpret_cast<unsigned long long *>(sX + (XS ? p.nsw : 0) * K3_XS);
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;\n" ::"r"((unsigned)__cvta_generic_to_shared(xbar)));
-        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-    }
-    __syncthreads();
-    const int sg = blockIdx.x;
-    if (p.stream0 + sg * p.nsw >= p.stream_end) return;
-    K3DevEnv env{lane, xbar};
-    if (warp == 0) k3_unit<MAXS, XS, 1>(env, p, sg, (int)blockIdx.y, p.b0 + (int)blockIdx.z, ring, sdst, sF, sK, sX, srrel, stab, n_slots);
-    else k3_unit<MAXS, XS, 2>(env, p, sg, (int)blockIdx.y, p.b0 + (int)blockIdx.z, ring, sdst, sF, sK, sX, srrel, stab, n_slots);
+    K3DevEnv env{lane};
+    k3_unit<MAXS>(env, p, sg, (int)blockIdx.y, p.b0 + (int)blockIdx.z, ring, sdst, sF, sK, srrel, stab, n_slots);
 }
 #endif
 

@@ -4,7 +4,6 @@
 // HalfBandDecimator stages with FIRQueueBackToFront's shifted history (dsp.cpp:163-173), callback by
 // callback. Built and run by tests/test_k3_sim.py (nvcc host compile; no GPU involved).
 #include <barrier>
-#include <semaphore>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -17,27 +16,11 @@
 
 using namespace sdrb;
 
-struct HandOver {                                  // the four named barriers of the warp-specialised kernel
-    std::counting_semaphore<4> full[2] = {std::counting_semaphore<4>(0), std::counting_semaphore<4>(0)};
-    std::counting_semaphore<4> empty[2] = {std::counting_semaphore<4>(0), std::counting_semaphore<4>(0)};
-};
-
 struct HostEnv {
     int lane;
     std::barrier<> *bar;
-    HandOver *ho = nullptr;
-    // one lane talks to the other warp, the warp barrier spreads the news (on the GPU all 32 lanes arrive / sync)
-    void signal_full(int b) { bar->arrive_and_wait(); if (lane == 0) ho->full[b].release(); }
-    void wait_full(int b) { if (lane == 0) ho->full[b].acquire(); bar->arrive_and_wait(); }
-    void signal_empty(int b) { bar->arrive_and_wait(); if (lane == 0) ho->empty[b].release(); }
-    void wait_empty(int b) { if (lane == 0) ho->empty[b].acquire(); bar->arrive_and_wait(); }
     void sync() { bar->arrive_and_wait(); }
     bool all(bool v) { return v; }                 // every lane evaluates the same warp-uniform condition
-    // the bulk-copy engine: on the CPU the copy is done on the spot by the issuing lane; the barrier that follows every
-    // x_wait() in k3_unit orders it against the readers
-    void x_expect(unsigned) {}
-    void x_copy(void *smem, const void *gmem, unsigned bytes) { memcpy(smem, gmem, bytes); }
-    void x_wait(unsigned) {}
 };
 
 // ---- reference: one sub VFO front end over n_cb callbacks of B samples, state carried across ----
@@ -85,7 +68,7 @@ static float frand() {
     return (float)((double)(rng >> 11) / 9007199254740992.0 * 2.0 - 1.0);
 }
 
-template <int MAXS, bool XS>
+template <int MAXS>
 static void run_units(const K3Params &p, int n_cb, int n_spans) {
     const int n_groups = (p.stream_end - p.stream0 + p.nsw - 1) / p.nsw;
     // slot table and rrel as the kernel builds them
@@ -103,47 +86,12 @@ static void run_units(const K3Params &p, int n_cb, int n_spans) {
                 std::vector<float2 *> sdst(32, nullptr);
                 std::vector<float2> sF(64, make_float2(NAN, NAN));
                 std::vector<int2> sK(32, make_int2(0, 0));
-                std::vector<float2> sX((size_t)p.nsw * K3_XS, make_float2(NAN, NAN));
                 std::barrier<> bar(32);
                 std::vector<std::thread> th;
                 for (int lane = 0; lane < 32; ++lane)
                     th.emplace_back([&, lane]() {
                         HostEnv env{lane, &bar};
-                        k3_unit<MAXS, XS, 0>(env, p, sg, span, p.b0 + cb, ring.data(), sdst.data(), sF.data(), sK.data(), sX.data(), p.rrel, stab.data(), n_slots);
-                    });
-                for (auto &t : th) t.join();
-            }
-}
-
-// the warp-specialised pair: 32 producer lanes + 32 consumer lanes, two ring buffers
-template <int MAXS, bool XS>
-static void run_units_ws(const K3Params &p, int n_cb, int n_spans) {
-    const int n_groups = (p.stream_end - p.stream0 + p.nsw - 1) / p.nsw;
-    std::vector<unsigned short> stab((size_t)K3_MAX_SLOTS);
-    int n_slots = 0;
-    for (int v = 0; v < p.count; ++v) {
-        const int n = 32 >> (p.v[v].S - 1);
-        for (int c = 0; c < n; ++c) stab[(size_t)(n_slots + c)] = (unsigned short)((v << 8) | c);
-        n_slots += n;
-    }
-    for (int cb = 0; cb < n_cb; ++cb)
-        for (int span = 0; span < n_spans; ++span)
-            for (int sg = 0; sg < n_groups; ++sg) {
-                std::vector<float2> ring((size_t)2 * p.nsw * p.count * K3_ROW, make_float2(NAN, NAN));
-                std::vector<float2 *> sdst(32, nullptr);
-                std::vector<float2> sF(64, make_float2(NAN, NAN));
-                std::vector<int2> sK(32, make_int2(0, 0));
-                std::vector<float2> sX((size_t)p.nsw * K3_XS, make_float2(NAN, NAN));
-                std::barrier<> barA(32), barB(32);
-                HandOver ho;
-                std::vector<std::thread> th;
-                for (int lane = 0; lane < 64; ++lane)
-                    th.emplace_back([&, lane]() {
-                        HostEnv env{lane & 31, lane < 32 ? &barA : &barB, &ho};
-                        if (lane < 32)
-                            k3_unit<MAXS, XS, 1>(env, p, sg, span, p.b0 + cb, ring.data(), sdst.data(), sF.data(), sK.data(), sX.data(), p.rrel, stab.data(), n_slots);
-                        else
-                            k3_unit<MAXS, XS, 2>(env, p, sg, span, p.b0 + cb, ring.data(), sdst.data(), sF.data(), sK.data(), sX.data(), p.rrel, stab.data(), n_slots);
+                        k3_unit<MAXS>(env, p, sg, span, p.b0 + cb, ring.data(), sdst.data(), sF.data(), sK.data(), p.rrel, stab.data(), n_slots);
                     });
                 for (auto &t : th) t.join();
             }
@@ -203,12 +151,7 @@ int main(int argc, char **argv) {
             for (int cb = 0; cb < cb_per_call; ++cb)
                 for (int v = 0; v < nv; ++v) ref[(size_t)s][(size_t)v].process(body + (size_t)cb * B, B, ref_out[(size_t)s][(size_t)v]);
         }
-        const bool ws = argc > 7 && atoi(argv[7]) != 0;                  // 7th argument: the warp-specialised pair
-        if (ws) {
-            if (call & 1) run_units_ws<5, false>(p, cb_per_call, n_spans);
-            else run_units_ws<5, true>(p, cb_per_call, n_spans);
-        } else if (call & 1) run_units<5, false>(p, cb_per_call, n_spans);   // both input paths, alternating from call to call
-        else run_units<5, true>(p, cb_per_call, n_spans);
+        run_units<5>(p, cb_per_call, n_spans);
         for (int s = 0; s < n_streams; ++s) {
             for (int v = 0; v < nv; ++v) {
                 const float2 *z = zbuf[(size_t)v].data() + (size_t)s * out_stride + OHIST;

@@ -35,10 +35,10 @@ def sim(built):
     (30720, 7680, 4, 2, 7, 16),      # 16 sub VFOs, ragged last span
     (30720, 7680, 3, 8, 3, 4),       # eight streams per warp
     (30720, 7680, 2, 1, 5, 16),      # one stream per warp
-    (30720, 7680, 3, 2, 4, 6, 1),    # the warp-specialised producer / consumer pair, two ring buffers
-    (30720, 7680, 4, 2, 7, 16, 1),
-    (30720, 7680, 5, 3, 1, 6, 1),
-])
+    (30720, 7680, 4, 2, 3, 15),      # 15 sub VFOs, two lanes without a row (25E's two-stage group)
+    (30720, 7680, 9, 8, 2, 1),       # one sub VFO, eight streams per warp, a second group with one stream
+    (30000, 6144, 3, 2, 3, 6),       # the table wraps inside a tile (sample 30000 of 36864)
+], ids=lambda a: "-".join(str(x) for x in a))
 def test_k3_unit_matches_the_plain_cascade(sim, args):
     r = subprocess.run([sim] + [str(a) for a in args], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0 and r.stdout.strip().endswith("OK"), r.stdout[-3000:]
