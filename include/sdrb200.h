@@ -137,6 +137,56 @@ int sdrb_bank_reset(sdrb_bank *bank, int stream);
 int sdrb_bank_blocks_done(sdrb_bank *bank, int stream, int64_t *blocks);
 
 /*
+ * Receiver state records: one receiver's carried state (NCO sample counter, DC recursion, every filter history) as one
+ * fixed-size byte record, to move a receiver into another bank of the same plan -- a larger or smaller bank, another GPU,
+ * a new process -- and continue it as if it had never moved: bit for bit when the other streams of the bank it lands in
+ * have consumed as many callbacks as it has (a bank rebuilt from one bank's records); next to streams at another count the
+ * sub-VFO audio of it and its neighbours may differ in the last bits, within +-1 LSB (DESIGN.md section 3).
+ *
+ * sdrb_plan_fingerprint: 64-bit hash of everything in the compiled plan that can change an output sample (fs, block,
+ * bufsplit, correct_dc; per main VFO mixer, decimation, compress parameters; per sub VFO parent, mixer, decimation, /late
+ * factor, gain, /late and low-pass taps). Topics, addresses, center_frequency and operational ini keys do not enter it.
+ * Host only, needs no GPU.
+ *
+ * sdrb_bank_state_bytes: size of one record. It depends on the plan only, never on n_streams, max_blocks or the device.
+ * Layout, little endian, every section on a 16-byte boundary:
+ *     0  u32 magic 0x54534253 ("SBST"), u32 format version (1)
+ *     8  u64 record_bytes
+ *    16  u64 plan fingerprint
+ *    24  i64 blocks_done (callbacks consumed)
+ *    32  float32 x2 DC recursion state (I, Q)
+ *    40  u32 flags: bit 0 correct_dc, bit 1 the bank fuses the NCO mix of mix-only /late sub VFOs into the /late FIR
+ *        (SDRB_FUSE_LATE, on by default); 20 reserved bytes, zero
+ *    64  DC table halo: 2 x 2 entries of 8 bytes, the anchor-free block-start states the next call starts from
+ *        (zero while blocks_done == 0 or without correct_dc)
+ *    96  raw uint8 tail, 512 bytes;  608  cf32 tail, 256 samples
+ *  2656  the history of every carried filter buffer, in the bank's order: per sub VFO its /late output history (late VFOs)
+ *        and its cascade output history, per main VFO its output history, then the staging histories of main VFOs with
+ *        more than 3 and sub VFOs with more than 5 half-band stages. Histories no kernel reads are zero: the cascade
+ *        output of a sub VFO whose mix is fused, the output of a main VFO without sub VFOs.
+ * A record depends on the receiver's state alone: saving one state twice gives identical bytes, and a fresh receiver's
+ * record equals its record after sdrb_bank_reset.
+ *
+ * streams: host array of n distinct indices in [0, n_streams), free for reuse when the call returns; record k belongs to
+ * streams[k]. Streams not listed are not touched.
+ * save_state / load_state: d_records is device memory of n * state_bytes bytes on the bank's device; both only enqueue on
+ * cuda_stream (NULL = default stream), after the last process call whatever stream it ran on; the next process call waits
+ * for them. load_state reads the headers first and therefore synchronises cuda_stream.
+ * read_state / write_state: the same with host memory; they return when the records are read or written.
+ * A load is all or nothing: every record's magic, version, record_bytes, fingerprint and flags are checked before anything
+ * is written, and a mismatch returns SDRB_E_INVALID with the record and field named in sdrb_last_error(), the bank unchanged.
+ * After a load, the inspection entry points (copy_main / read_main, copy_sub / read_sub, copy_forward / read_forward,
+ * copy_input / read_input, copy_dc_trace, sdrb_bank_spectrum_feed) are undefined for the loaded streams until the next
+ * process call. Spectrum display state (sdrb_spectrum) is not part of a record.
+ */
+int sdrb_plan_fingerprint(const sdrb_plan *plan, uint64_t *out);
+size_t sdrb_bank_state_bytes(const sdrb_bank *bank);
+int sdrb_bank_save_state(sdrb_bank *bank, const int32_t *streams, int n, void *d_records, void *cuda_stream);
+int sdrb_bank_load_state(sdrb_bank *bank, const int32_t *streams, int n, const void *d_records, void *cuda_stream);
+int sdrb_bank_read_state(sdrb_bank *bank, const int32_t *streams, int n, void *h_records);
+int sdrb_bank_write_state(sdrb_bank *bank, const int32_t *streams, int n, const void *h_records);
+
+/*
  * n_blocks callbacks for every stream of the bank, everything resident on the device.
  * Stands in for n_blocks x { sdr::rtlsdr_callback (jonti/sdr.cpp:100-145) -> sdrj::demodData
  * (sdrj.cpp:266-305) -> vfo::process tree (vfo.cpp:235-296) } per stream.

@@ -84,6 +84,12 @@ def lib():
         "sdrb_bank_destroy": (None, [vp]),
         "sdrb_bank_reset": (i, [vp, i]),
         "sdrb_bank_blocks_done": (i, [vp, i, P(C.c_int64)]),
+        "sdrb_plan_fingerprint": (i, [vp, P(C.c_uint64)]),
+        "sdrb_bank_state_bytes": (sz, [vp]),
+        "sdrb_bank_save_state": (i, [vp, vp, i, vp, vp]),
+        "sdrb_bank_load_state": (i, [vp, vp, i, vp, vp]),
+        "sdrb_bank_read_state": (i, [vp, vp, i, vp]),
+        "sdrb_bank_write_state": (i, [vp, vp, i, vp]),
         "sdrb_bank_process_device": (i, [vp, vp, sz, i, vp, vp, vp]),
         "sdrb_bank_process_device_ex": (i, [vp, vp, sz, i, vp, vp, vp, vp]),
         "sdrb_bank_copy_main": (i, [vp, i, i, vp, vp]),
@@ -217,6 +223,13 @@ class Plan:
             d.subs[k].filter_bw, d.subs[k].gain = s.get("filterbw", 0), s.get("gain", 0.01)
         return cls(desc=d)
 
+    @property
+    def fingerprint(self):
+        """64-bit hash of everything in the plan that can change an output sample (sdrb_plan_fingerprint)."""
+        v = C.c_uint64()
+        _check(lib().sdrb_plan_fingerprint(self.h, C.byref(v)), "sdrb_plan_fingerprint")
+        return v.value
+
     def setting(self, key, default=None):
         """Value of an ini key as QSettings names it, or `default`."""
         buf = C.create_string_buffer(512)
@@ -261,6 +274,41 @@ class Bank:
         v = C.c_int64()
         _check(lib().sdrb_bank_blocks_done(self.h, stream, C.byref(v)), "sdrb_bank_blocks_done")
         return v.value
+
+    @property
+    def state_bytes(self):
+        """Size of one receiver state record; the same for every bank of this plan."""
+        return lib().sdrb_bank_state_bytes(self.h)
+
+    @staticmethod
+    def _streams(streams):
+        s = np.ascontiguousarray(streams, dtype=np.int32).reshape(-1)
+        return s, s.ctypes.data_as(C.c_void_p)
+
+    def read_state(self, streams):
+        """State records of the listed streams: uint8 [len(streams), state_bytes] (sdrb_bank_read_state)."""
+        s, sp = self._streams(streams)
+        out = np.zeros((s.size, self.state_bytes), dtype=np.uint8)
+        _check(lib().sdrb_bank_read_state(self.h, sp, s.size, out.ctypes.data_as(C.c_void_p)), "sdrb_bank_read_state")
+        return out
+
+    def write_state(self, streams, records):
+        """Load records (uint8 [len(streams), state_bytes]) into the listed streams; all or nothing (sdrb_bank_write_state)."""
+        s, sp = self._streams(streams)
+        rec = np.ascontiguousarray(records, dtype=np.uint8)
+        if rec.size != s.size * self.state_bytes:
+            raise SdrbError("write_state: expected %d records of %d bytes" % (s.size, self.state_bytes))
+        _check(lib().sdrb_bank_write_state(self.h, sp, s.size, rec.ctypes.data_as(C.c_void_p)), "sdrb_bank_write_state")
+
+    def save_state(self, streams, d_records_ptr, cuda_stream=None):
+        """Enqueue the records of the listed streams into device memory (len(streams) * state_bytes bytes)."""
+        s, sp = self._streams(streams)
+        _check(lib().sdrb_bank_save_state(self.h, sp, s.size, d_records_ptr, cuda_stream), "sdrb_bank_save_state")
+
+    def load_state(self, streams, d_records_ptr, cuda_stream=None):
+        """Load device-resident records into the listed streams (synchronises cuda_stream to check the headers)."""
+        s, sp = self._streams(streams)
+        _check(lib().sdrb_bank_load_state(self.h, sp, s.size, d_records_ptr, cuda_stream), "sdrb_bank_load_state")
 
     def process_device(self, d_iq_ptr, iq_stride, n_blocks, d_pcm_ptr, d_tap_ptr=None, cuda_stream=None,
                        input_ready_event=None):

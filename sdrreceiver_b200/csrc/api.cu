@@ -141,6 +141,38 @@ extern "C" long sdrb_plan_copy_table(const sdrb_plan *plan, int kind, int idx, f
     return n;
 }
 
+// FNV-1a over a canonical serialisation (little-endian 64-bit integers, IEEE bits of doubles and floats) of what can change
+// an output sample. The NCO tables follow from (fs, mixer) and the Hilbert points from the rates; topics, addresses, the
+// centre frequency and operational ini keys stay out, so renaming a topic keeps the fingerprint.
+static uint64_t plan_fingerprint(const HostPlan &h) {
+    uint64_t x = 0xcbf29ce484222325ull;
+    auto bytes = [&](const void *p, size_t n) {
+        for (size_t k = 0; k < n; k++) { x ^= ((const unsigned char *)p)[k]; x *= 0x100000001b3ull; }
+    };
+    auto i64 = [&](int64_t v) { uint64_t u = (uint64_t)v; unsigned char b[8]; for (int k = 0; k < 8; k++) b[k] = (unsigned char)(u >> (8 * k)); bytes(b, 8); };
+    auto f64 = [&](double v) { int64_t u; memcpy(&u, &v, 8); i64(u); };
+    auto f32 = [&](float v) { uint32_t u; memcpy(&u, &v, 4); i64(u); };
+    bytes("sdrb-plan-1", 11);
+    i64(h.fs); i64(h.block); i64(h.bufsplit); i64(h.correct_dc);
+    i64((int64_t)h.mains.size());
+    for (const MainVfo &m : h.mains) { f64(m.mixer); i64(m.decim); i64(m.compress_scale); i64(m.compress_style); }
+    i64((int64_t)h.subs.size());
+    for (const SubVfo &s : h.subs) {
+        i64(s.main_idx); f64(s.mixer); i64(s.decim); i64(s.late); f32(s.gain);
+        i64((int64_t)s.dec_taps.size());
+        for (float v : s.dec_taps) f32(v);
+        i64((int64_t)s.lpf_taps.size());
+        for (float v : s.lpf_taps) f32(v);
+    }
+    return x;
+}
+
+extern "C" int sdrb_plan_fingerprint(const sdrb_plan *plan, uint64_t *out) {
+    if (!plan || !out) { set_error("sdrb_plan_fingerprint: NULL argument"); return SDRB_E_INVALID; }
+    *out = plan_fingerprint(plan->h);
+    return SDRB_OK;
+}
+
 // ------------------------------------------------------------------------------------
 // bank
 // ------------------------------------------------------------------------------------
@@ -281,6 +313,15 @@ struct sdrb_bank {
     // (main_out, zbuf), and k_hb_tail runs the remaining stages into the real output. Empty for plans without such VFOs.
     DevBuf main_tails, sub_tails;           // TailDev per deep main / sub VFO
     int n_main_tails = 0, n_sub_tails = 0, main_tail_tiles = 0, sub_tail_tiles = 0;   // channels and the longest channel's tiles
+    // receiver state records (k_state_io): where each carry item sits in a record, the record's size and the header fields
+    // of this bank; the stream list of a save / load, and the host variants' staging
+    DevBuf state_items, state_streams, d_state;
+    size_t state_bytes = 0;
+    StateHeader state_hdr{};
+    // end of the last save / load (recorded on the caller's stream): the next call's DC pre-pass waits for it, it may
+    // otherwise run as soon as that call's input is ready
+    cudaEvent_t ev_state = nullptr;
+    bool state_pending = false;
     // what the last process call consumed (inspection entry points: spectrum of the raw input)
     const uint8_t *last_iq = nullptr; size_t last_iq_stride = 0;
     const float2 *last_cf = nullptr; size_t last_cf_stride = 0;
@@ -317,9 +358,10 @@ extern "C" void sdrb_bank_destroy(sdrb_bank *b) {
     cudaDeviceSynchronize();                                 // asynchronous host calls may still be in flight
     DevBuf *all[] = {&b->luts, &b->taps, &b->blocks_done, &b->dc_state, &b->raw_tail, &b->cf_tail, &b->dc_anchor, &b->dc_stats, &b->dc_table, &b->dc_qtab,
                      &b->main_out, &b->zbuf, &b->dbuf, &b->cascdev, &b->rfdev, &b->latedev, &b->usbdev, &b->carry,
-                     &b->main_tails, &b->sub_tails,
+                     &b->main_tails, &b->sub_tails, &b->state_items, &b->state_streams, &b->d_state,
                      &b->d_iq, &b->d_pcm, &b->d_tap, &b->d_cf, &b->d_fwd, &b->k3_rrel};
     for (DevBuf *d : all) d->release();
+    if (b->ev_state) cudaEventDestroy(b->ev_state);
     for (cudaEvent_t e : b->ev_in) cudaEventDestroy(e);
     for (cudaEvent_t e : b->ev_free) cudaEventDestroy(e);
     for (cudaEvent_t e : b->ev_out) cudaEventDestroy(e);
@@ -415,6 +457,8 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
     BANK_TRY(b->dc_qtab.alloc(2 * sizeof(int) * 512 * (size_t)n_streams));
     BANK_TRY(b->dc_stats.alloc(h.correct_dc ? sizeof(DcStats) * 2 * (size_t)n_streams * (size_t)b->dc_stride + 1024 : 16));
     BANK_TRY(b->dc_table.alloc(h.correct_dc ? 2 * sizeof(uint2) * 2 * (size_t)n_streams * (size_t)(b->dc_stride + DC_HALO_BLKS) : 64));
+    // the halo entries a state record saves exist before any u8 call writes them (a bank fed only cf32 input): start them at zero
+    BANK_CU(cudaMemset(b->dc_table.p, 0, b->dc_table.bytes));
     // staging slices of the deep VFOs: first stage count a mixing kernel runs, and the rest for k_hb_tail
     static_assert(TAIL_HIST == MAIN_HIST, "k1_ingest_main writes every main output, staged or not, behind MAIN_HIST samples");
     constexpr int kMainStaged = 3, kSubStaged = 5;
@@ -515,6 +559,10 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
     std::vector<LateDev> latedev;
     std::vector<UsbDev> usbdev;
     std::vector<CarryItem> carry;
+    // per carry item: 1 if a kernel reads its history in the next call. A state record holds the others as zeros: the z of a
+    // sub VFO whose mix is fused into the /late FIR (that kernel reads the parent's output instead) and the output of a main
+    // VFO without sub VFOs (the forwarder and copy_main read only the body)
+    std::vector<int> carry_read;
     // the mixing cascade of sub VFO i: z itself, or the staging slice of a sub VFO with more than 5 stages
     auto sub_cascade = [&](size_t i) {
         const SubVfo &s = h.subs[i];
@@ -566,7 +614,7 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
             U.src = L.d; U.src_stride = L.d_stride; U.src_hist = L.d_hist;
             CarryItem c; c.base = L.d; c.stride = (long long)(d_stride * sizeof(float2));
             c.hist_bytes = L.d_hist * (int)sizeof(float2); c.block_bytes = s.samples_out * (int)sizeof(float2);
-            carry.push_back(c);
+            carry.push_back(c); carry_read.push_back(1);
         } else {
             U.src = (const float2 *)b->zbuf.p + z_off[i]; U.src_stride = (long long)z_stride; U.src_hist = z_hist[i];
         }
@@ -582,13 +630,13 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
         b->uv_vfo_out.push_back(s.samples_out); b->uv_vfo_np.push_back(U.np);
         CarryItem c; c.base = (float2 *)b->zbuf.p + z_off[i]; c.stride = (long long)(z_stride * sizeof(float2));
         c.hist_bytes = z_hist[i] * (int)sizeof(float2); c.block_bytes = s.block_z * (int)sizeof(float2);
-        carry.push_back(c);
+        carry.push_back(c); carry_read.push_back(b->sub_fused[i] ? 0 : 1);
     }
     for (size_t i = 0; i < h.mains.size(); i++) {
         CarryItem c; c.base = (float2 *)b->main_out.p + b->main_off[i];
         c.stride = (long long)(b->main_stride * sizeof(float2));
         c.hist_bytes = MAIN_HIST * (int)sizeof(float2); c.block_bytes = h.mains[i].block_out * (int)sizeof(float2);
-        carry.push_back(c);
+        carry.push_back(c); carry_read.push_back(h.mains[i].n_subs > 0 ? 1 : 0);
     }
     // deep VFOs: the tail kernels' descriptors, and the staging slices' histories among the carry items
     std::vector<TailDev> main_tails, sub_tails;
@@ -601,7 +649,7 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
         list.push_back(T);
         CarryItem c; c.base = in; c.stride = (long long)(stride * sizeof(float2));
         c.hist_bytes = TAIL_HIST * (int)sizeof(float2); c.block_bytes = block_in * (int)sizeof(float2);
-        carry.push_back(c);
+        carry.push_back(c); carry_read.push_back(1);
         return T.tiles;
     };
     for (size_t i = 0; i < h.mains.size(); i++)
@@ -707,6 +755,23 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
     if (!latedev.empty()) BANK_CU(cudaMemcpy(b->latedev.p, latedev.data(), sizeof(LateDev) * latedev.size(), cudaMemcpyHostToDevice));
     if (!usbdev.empty()) BANK_CU(cudaMemcpy(b->usbdev.p, usbdev.data(), sizeof(UsbDev) * usbdev.size(), cudaMemcpyHostToDevice));
     BANK_CU(cudaMemcpy(b->carry.p, carry.data(), sizeof(CarryItem) * carry.size(), cudaMemcpyHostToDevice));
+    {
+        // receiver state records: the carry items' histories in bank order behind the fixed sections (kernels.cuh, k_state_io)
+        std::vector<int2> rec(carry.size());
+        size_t at = STATE_ITEMS_OFF;
+        for (size_t k = 0; k < carry.size(); k++) {
+            rec[k] = make_int2((int)at, carry_read[k]);
+            at += (size_t)carry[k].hist_bytes;
+        }
+        b->state_bytes = at;
+        BANK_TRY(b->state_items.alloc(sizeof(int2) * std::max<size_t>(rec.size(), 1)));
+        if (!rec.empty()) BANK_CU(cudaMemcpy(b->state_items.p, rec.data(), sizeof(int2) * rec.size(), cudaMemcpyHostToDevice));
+        BANK_TRY(b->state_streams.alloc(sizeof(int) * (size_t)n_streams));
+        StateHeader &sh = b->state_hdr;
+        sh.magic = STATE_MAGIC; sh.version = STATE_VERSION; sh.record_bytes = at; sh.fingerprint = plan_fingerprint(h);
+        sh.flags = (h.correct_dc ? STATE_FLAG_DC : 0u) |
+                   (std::find(b->sub_fused.begin(), b->sub_fused.end(), true) != b->sub_fused.end() ? STATE_FLAG_FUSED_LATE : 0u);
+    }
 
     b->uv_eo_rows = 34 + b->uv_np_max / 32;
     b->uv_warp_floats = std::max(UV_IN_FLOATS, 2 * b->uv_eo_rows * UV_ROW);
@@ -1039,6 +1104,11 @@ static int enqueue_all(sdrb_bank *b, CallCtx &c, cudaStream_t st, int *launches,
     c.par = b->dc_par;
     b->last_iq = c.d_iq; b->last_iq_stride = c.iq_stride; b->last_cf = c.d_cf; b->last_cf_stride = c.cf_stride;
     b->last_blocks = c.n_blocks; b->last_par = c.par;
+    if (b->state_pending) {             // a save or load since the last call: the DC pre-pass and the filters come after it
+        CU_TRY(cudaStreamWaitEvent(st, b->ev_state, 0));
+        if (dc) CU_TRY(cudaStreamWaitEvent(b->s_dc[0], b->ev_state, 0));
+        b->state_pending = false;
+    }
     if (dc) {
         cudaStream_t sd = b->s_dc[0];
         if (input_ready) {
@@ -1560,6 +1630,129 @@ extern "C" int sdrb_bank_read_main(sdrb_bank *b, int main_idx, int n_blocks, flo
 }
 
 extern "C" int sdrb_bank_last_launches(const sdrb_bank *b) { return b ? b->last_launches : 0; }
+
+// ---- receiver state records (layout: include/sdrb200.h, kernels.cuh k_state_io) ----
+extern "C" size_t sdrb_bank_state_bytes(const sdrb_bank *b) { return b ? b->state_bytes : 0; }
+
+static int check_state_args(const sdrb_bank *b, const int32_t *streams, int n, const void *records, const char *who) {
+    if (!b || !streams || !records) { set_error(std::string(who) + ": NULL argument"); return SDRB_E_INVALID; }
+    if (n <= 0 || n > b->n_streams) { set_error(std::string(who) + ": n must be 1..n_streams"); return SDRB_E_INVALID; }
+    std::vector<char> seen((size_t)b->n_streams, 0);
+    for (int k = 0; k < n; k++) {
+        const int s = streams[k];
+        const char *bad = (s < 0 || s >= b->n_streams) ? "is outside 0..n_streams-1" : (seen[(size_t)s] ? "is listed twice" : nullptr);
+        if (bad) { set_error(std::string(who) + ": streams[" + std::to_string(k) + "] = " + std::to_string(s) + " " + bad); return SDRB_E_INVALID; }
+        seen[(size_t)s] = 1;
+    }
+    return SDRB_OK;
+}
+
+// Every header of a batch against this bank, before anything is written: a load is all or nothing.
+static int check_state_headers(const sdrb_bank *b, const int32_t *streams, int n, const unsigned char *h, size_t pitch, const char *who) {
+    const StateHeader &w = b->state_hdr;
+    for (int k = 0; k < n; k++) {
+        StateHeader r;
+        memcpy(&r, h + (size_t)k * pitch, sizeof(r));
+        const char *field = nullptr;
+        unsigned long long got = 0, want = 0;
+        if (r.magic != w.magic) { field = "magic"; got = r.magic; want = w.magic; }
+        else if (r.version != w.version) { field = "version"; got = r.version; want = w.version; }
+        else if (r.record_bytes != w.record_bytes) { field = "record_bytes"; got = r.record_bytes; want = w.record_bytes; }
+        else if (r.fingerprint != w.fingerprint) { field = "plan fingerprint"; got = r.fingerprint; want = w.fingerprint; }
+        else if (r.flags != w.flags) { field = "flags (correct_dc, fused /late VFOs)"; got = r.flags; want = w.flags; }
+        if (field) {
+            char msg[320];
+            snprintf(msg, sizeof(msg), "%s: record %d (for stream %d): %s is 0x%llx, this bank needs 0x%llx; nothing was loaded", who, k,
+                     (int)streams[k], field, got, want);
+            set_error(msg);
+            return SDRB_E_INVALID;
+        }
+    }
+    return SDRB_OK;
+}
+
+// One k_state_io launch on `st` between records at d_records and the listed streams. Ordered after the last device-resident call
+// and the last save / load, whatever stream those ran on; the next process call waits for it (ev_state, ev_device_tail).
+static int state_enqueue(sdrb_bank *b, const int32_t *streams, int n, void *d_records, cudaStream_t st, bool save) {
+    if (b->device_tail_pending) CU_TRY(cudaStreamWaitEvent(st, b->ev_device_tail, 0));
+    if (b->state_pending) CU_TRY(cudaStreamWaitEvent(st, b->ev_state, 0));          // the last save / load still reads state_streams
+    const std::vector<int> list(streams, streams + n);      // pageable: staged before cudaMemcpyAsync returns, the caller may reuse `streams`
+    CU_TRY(cudaMemcpyAsync(b->state_streams.p, list.data(), sizeof(int) * (size_t)n, cudaMemcpyHostToDevice, st));
+    StateIoParams p;
+    p.items = (const CarryItem *)b->carry.p; p.item_rec = (const int2 *)b->state_items.p; p.n_items = b->n_carry;
+    p.streams = (const int *)b->state_streams.p; p.rec = (unsigned char *)d_records; p.rec_bytes = b->state_bytes;
+    p.blocks_done = (long long *)b->blocks_done.p; p.dc_state = (float2 *)b->dc_state.p;
+    p.raw_tail = (uint8_t *)b->raw_tail.p; p.cf_tail = (float2 *)b->cf_tail.p;
+    p.dc_table = b->plan->h.correct_dc ? b->table_buf(b->dc_par) : nullptr;   // the buffer the next call reads its halo from
+    p.dc_table_stride = b->dc_stride + DC_HALO_BLKS;
+    p.hdr = b->state_hdr;
+    const dim3 grid((unsigned)n, (unsigned)(b->n_carry + 1));
+    if (save) k_state_io<true><<<grid, 128, 0, st>>>(p);
+    else k_state_io<false><<<grid, 128, 0, st>>>(p);
+    CU_TRY(cudaGetLastError());
+    if (!b->ev_state) CU_TRY(cudaEventCreateWithFlags(&b->ev_state, cudaEventDisableTiming));
+    CU_TRY(cudaEventRecord(b->ev_state, st));
+    b->state_pending = true;
+    if (!b->ev_device_tail) CU_TRY(cudaEventCreateWithFlags(&b->ev_device_tail, cudaEventDisableTiming));
+    CU_TRY(cudaEventRecord(b->ev_device_tail, st));       // a following host call waits for it like for a device call
+    b->device_tail_pending = true;
+    return SDRB_OK;
+}
+
+extern "C" int sdrb_bank_save_state(sdrb_bank *b, const int32_t *streams, int n, void *d_records, void *cuda_stream) {
+    int rc = check_state_args(b, streams, n, d_records, "sdrb_bank_save_state");
+    if (rc != SDRB_OK) return rc;
+    CU_TRY(cudaSetDevice(b->device));
+    if ((rc = host_drain(b)) != SDRB_OK) return rc;
+    return state_enqueue(b, streams, n, d_records, (cudaStream_t)cuda_stream, true);
+}
+
+extern "C" int sdrb_bank_load_state(sdrb_bank *b, const int32_t *streams, int n, const void *d_records, void *cuda_stream) {
+    int rc = check_state_args(b, streams, n, d_records, "sdrb_bank_load_state");
+    if (rc != SDRB_OK) return rc;
+    CU_TRY(cudaSetDevice(b->device));
+    if ((rc = host_drain(b)) != SDRB_OK) return rc;
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    std::vector<unsigned char> hdr((size_t)n * sizeof(StateHeader));
+    CU_TRY(cudaMemcpy2DAsync(hdr.data(), sizeof(StateHeader), d_records, b->state_bytes, sizeof(StateHeader), (size_t)n,
+                             cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    if ((rc = check_state_headers(b, streams, n, hdr.data(), sizeof(StateHeader), "sdrb_bank_load_state")) != SDRB_OK) return rc;
+    return state_enqueue(b, streams, n, const_cast<void *>(d_records), st, false);
+}
+
+static int state_staging(sdrb_bank *b, int n) {
+    const size_t need = (size_t)n * b->state_bytes;
+    if (b->d_state.bytes >= need && b->d_state.p) return SDRB_OK;
+    b->d_state.release();
+    return b->d_state.alloc((size_t)b->n_streams * b->state_bytes);
+}
+
+extern "C" int sdrb_bank_read_state(sdrb_bank *b, const int32_t *streams, int n, void *h_records) {
+    int rc = check_state_args(b, streams, n, h_records, "sdrb_bank_read_state");
+    if (rc != SDRB_OK) return rc;
+    CU_TRY(cudaSetDevice(b->device));
+    if ((rc = host_drain(b)) != SDRB_OK || (rc = state_staging(b, n)) != SDRB_OK) return rc;
+    cudaStream_t st = b->s_compute;
+    if ((rc = state_enqueue(b, streams, n, b->d_state.p, st, true)) != SDRB_OK) return rc;
+    CU_TRY(cudaMemcpyAsync(h_records, b->d_state.p, (size_t)n * b->state_bytes, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    return SDRB_OK;
+}
+
+extern "C" int sdrb_bank_write_state(sdrb_bank *b, const int32_t *streams, int n, const void *h_records) {
+    int rc = check_state_args(b, streams, n, h_records, "sdrb_bank_write_state");
+    if (rc != SDRB_OK) return rc;
+    if ((rc = check_state_headers(b, streams, n, (const unsigned char *)h_records, b->state_bytes, "sdrb_bank_write_state")) != SDRB_OK)
+        return rc;
+    CU_TRY(cudaSetDevice(b->device));
+    if ((rc = host_drain(b)) != SDRB_OK || (rc = state_staging(b, n)) != SDRB_OK) return rc;
+    cudaStream_t st = b->s_compute;
+    CU_TRY(cudaMemcpyAsync(b->d_state.p, h_records, (size_t)n * b->state_bytes, cudaMemcpyHostToDevice, st));
+    if ((rc = state_enqueue(b, streams, n, b->d_state.p, st, false)) != SDRB_OK) return rc;
+    CU_TRY(cudaStreamSynchronize(st));
+    return SDRB_OK;
+}
 
 // ---- FP32 peak probe ----
 namespace sdrb {

@@ -12,6 +12,7 @@
 //   k2b_v2 (v2)                             delay62 - Hilbert125 (vfo.cpp:316-324), optional low-pass, gain, int16
 //                                           (vfo.cpp:328)
 //   k3_carry                                filter tails / raw tail / counters for the next call
+//   k_state_io                              the same carried state to / from per-receiver records (outside the call)
 //
 // Reference quirks reproduced on purpose (SURVEY.md section 0):
 //   * FIRQueueBackToFront copies one slot early (dsp.cpp:169): at every callback edge, at
@@ -867,6 +868,85 @@ __global__ void __launch_bounds__(128) k3_carry(const CarryItem *__restrict__ it
             dc_table_next[(size_t)stream * dc_table_stride * 2 + threadIdx.x] = e;   // the next call owns the other buffer
         }
     }
+}
+
+// ------------------------------------------------------------------------------------
+// Receiver state records (sdrb_bank_save_state / load_state, layout in include/sdrb200.h): everything k3_carry leaves
+// for the next call, for a list of streams, as one fixed-size record per stream. The record holds the carry items'
+// history regions (never bank rows, whose strides depend on max_blocks), so banks of one plan exchange records.
+// ------------------------------------------------------------------------------------
+struct StateHeader {
+    unsigned magic, version;
+    unsigned long long record_bytes, fingerprint;
+    long long blocks_done;
+    float2 dc_state;
+    unsigned flags, reserved[5];
+};
+static_assert(sizeof(StateHeader) == 64, "the record header is 64 bytes");
+constexpr unsigned STATE_MAGIC = 0x54534253u;                   // "SBST", little endian
+constexpr unsigned STATE_VERSION = 1u;
+constexpr unsigned STATE_FLAG_DC = 1u, STATE_FLAG_FUSED_LATE = 2u;
+constexpr int STATE_HALO_OFF = (int)sizeof(StateHeader);                        // 2*DC_HALO_BLKS uint2
+constexpr int STATE_RAW_OFF = STATE_HALO_OFF + 2 * DC_HALO_BLKS * 8;            // 2*RAW_TAIL bytes
+constexpr int STATE_CF_OFF = STATE_RAW_OFF + 2 * RAW_TAIL;                      // RAW_TAIL float2
+constexpr int STATE_ITEMS_OFF = STATE_CF_OFF + RAW_TAIL * 8;                    // carry items, in bank order
+static_assert(STATE_RAW_OFF % 16 == 0 && STATE_CF_OFF % 16 == 0 && STATE_ITEMS_OFF % 16 == 0, "sections start on 16 bytes");
+
+struct StateIoParams {
+    const CarryItem *items;         // the bank's carry items (the list k3_carry runs)
+    const int2 *item_rec;           // per item: (offset in the record, 1 = some kernel reads it / 0 = saved as zeros)
+    int n_items;
+    const int *streams;             // record k <-> stream streams[k]
+    unsigned char *rec;             // n records of rec_bytes
+    size_t rec_bytes;
+    long long *blocks_done;
+    float2 *dc_state;
+    uint8_t *raw_tail;              // [n_streams][2*RAW_TAIL]
+    float2 *cf_tail;                // [n_streams][RAW_TAIL]
+    uint2 *dc_table;                // table_buf(dc_par): the buffer the next call reads its halo from; nullptr without DC
+    int dc_table_stride;
+    StateHeader hdr;                // SAVE: magic .. flags of this bank; blocks_done and dc_state are filled per stream
+};
+
+// grid (listed streams, n_items + 1): y < n_items copies one carry item's history, the last y-block the header scalars, the DC
+// halo and the raw / cf32 tails (as k3_carry splits its work). Every section is a whole number of 16-byte chunks.
+template <bool SAVE>
+__global__ void __launch_bounds__(128) k_state_io(const __grid_constant__ StateIoParams p) {
+    const int stream = p.streams[blockIdx.x];
+    unsigned char *rec = p.rec + (size_t)blockIdx.x * p.rec_bytes;
+    auto copy16 = [&](void *bank, int rec_off, int bytes, bool live) {
+        uint4 *b = reinterpret_cast<uint4 *>(bank);
+        uint4 *r = reinterpret_cast<uint4 *>(rec + rec_off);
+        for (int e = threadIdx.x; e < bytes / 16; e += 128) {
+            if (SAVE) r[e] = live ? b[e] : make_uint4(0u, 0u, 0u, 0u);
+            else b[e] = r[e];
+        }
+    };
+    if ((int)blockIdx.y < p.n_items) {
+        const CarryItem it = p.items[blockIdx.y];
+        const int2 ir = p.item_rec[blockIdx.y];
+        copy16(reinterpret_cast<unsigned char *>(it.base) + (size_t)stream * it.stride, ir.x, it.hist_bytes, ir.y != 0);
+        return;
+    }
+    StateHeader *h = reinterpret_cast<StateHeader *>(rec);
+    long long done;
+    if (SAVE) {
+        done = p.blocks_done[stream];
+        if (threadIdx.x == 0) {
+            StateHeader o = p.hdr;
+            o.blocks_done = done;
+            o.dc_state = p.dc_state[stream];
+            *h = o;
+        }
+    } else {
+        done = h->blocks_done;
+        if (threadIdx.x == 0) { p.blocks_done[stream] = done; p.dc_state[stream] = h->dc_state; }
+    }
+    // the halo entries only exist once a call has run: a fresh stream's record holds zeros
+    if (SAVE || p.dc_table)
+        copy16(p.dc_table + (size_t)stream * p.dc_table_stride * 2, STATE_HALO_OFF, 2 * DC_HALO_BLKS * 8, p.dc_table && done != 0);
+    copy16(p.raw_tail + (size_t)stream * (2 * RAW_TAIL), STATE_RAW_OFF, 2 * RAW_TAIL, true);
+    copy16(p.cf_tail + (size_t)stream * RAW_TAIL, STATE_CF_OFF, RAW_TAIL * 8, true);
 }
 
 // ------------------------------------------------------------------------------------
