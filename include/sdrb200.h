@@ -175,10 +175,19 @@ int sdrb_bank_blocks_done(sdrb_bank *bank, int stream, int64_t *blocks);
  * read_state / write_state: the same with host memory; they return when the records are read or written.
  * A load is all or nothing: every record's magic, version, record_bytes, fingerprint and flags are checked before anything
  * is written, and a mismatch returns SDRB_E_INVALID with the record and field named in sdrb_last_error(), the bank unchanged.
+ * The same check refuses a record whose state no kernel can run from, so a corrupt or hand-edited record is an error, never
+ * an out-of-bounds table read or a poisoned DC recursion:
+ *   - blocks_done outside 0 .. SDRB_STATE_MAX_BLOCKS_DONE(block) = floor(2^62 / block). Every kernel forms its table
+ *     indices from (blocks_done + b) * block in 64 bits; the bound leaves more than 2^62 samples of headroom (about
+ *     95 000 years at 1.536 MS/s). A receiver that runs past it keeps running; only its records are refused.
+ *   - a DC state component that is NaN, infinite or larger in magnitude than SDRB_STATE_MAX_DC = 128. The recursion's
+ *     inputs x - 127 lie in [-127, 128] and it starts at 0; full-scale input (all 255 or all 0) settles at +-124.2353.
  * After a load, the inspection entry points (copy_main / read_main, copy_sub / read_sub, copy_forward / read_forward,
  * copy_input / read_input, copy_dc_trace, sdrb_bank_spectrum_feed) are undefined for the loaded streams until the next
  * process call. Spectrum display state (sdrb_spectrum) is not part of a record.
  */
+#define SDRB_STATE_MAX_BLOCKS_DONE(block) ((int64_t)(((int64_t)1 << 62) / (int64_t)(block)))
+#define SDRB_STATE_MAX_DC 128.0f
 int sdrb_plan_fingerprint(const sdrb_plan *plan, uint64_t *out);
 size_t sdrb_bank_state_bytes(const sdrb_bank *bank);
 int sdrb_bank_save_state(sdrb_bank *bank, const int32_t *streams, int n, void *d_records, void *cuda_stream);

@@ -1660,13 +1660,30 @@ static int check_state_headers(const sdrb_bank *b, const int32_t *streams, int n
         else if (r.record_bytes != w.record_bytes) { field = "record_bytes"; got = r.record_bytes; want = w.record_bytes; }
         else if (r.fingerprint != w.fingerprint) { field = "plan fingerprint"; got = r.fingerprint; want = w.fingerprint; }
         else if (r.flags != w.flags) { field = "flags (correct_dc, fused /late VFOs)"; got = r.flags; want = w.flags; }
+        char msg[320];
         if (field) {
-            char msg[320];
             snprintf(msg, sizeof(msg), "%s: record %d (for stream %d): %s is 0x%llx, this bank needs 0x%llx; nothing was loaded", who, k,
                      (int)streams[k], field, got, want);
             set_error(msg);
             return SDRB_E_INVALID;
         }
+        // the two scalars every later call computes from: table indices (blocks_done * block) and the DC recursion
+        const long long max_done = SDRB_STATE_MAX_BLOCKS_DONE(b->plan->h.block);
+        if (r.blocks_done < 0 || r.blocks_done > max_done) {
+            snprintf(msg, sizeof(msg), "%s: record %d (for stream %d): blocks_done is %lld, this bank needs 0..%lld; nothing was loaded",
+                     who, k, (int)streams[k], r.blocks_done, max_done);
+            set_error(msg);
+            return SDRB_E_INVALID;
+        }
+        const float dc[2] = {r.dc_state.x, r.dc_state.y};
+        for (int a = 0; a < 2; a++)
+            if (!(fabsf(dc[a]) <= SDRB_STATE_MAX_DC)) {           // also refuses NaN
+                snprintf(msg, sizeof(msg), "%s: record %d (for stream %d): dc_state %c is %.9g, this bank needs a finite value in "
+                         "[-%g, %g]; nothing was loaded", who, k, (int)streams[k], a ? 'Q' : 'I', (double)dc[a],
+                         (double)SDRB_STATE_MAX_DC, (double)SDRB_STATE_MAX_DC);
+                set_error(msg);
+                return SDRB_E_INVALID;
+            }
     }
     return SDRB_OK;
 }

@@ -3,7 +3,9 @@ bank whose plan computes the same samples, so the fingerprint covers everything 
 nothing that cannot (topics, addresses)."""
 import glob
 import os
+import re
 
+import numpy as np
 import pytest
 
 from conftest import plan_path
@@ -72,3 +74,40 @@ def test_fingerprint_null_arguments():
     L = B.lib()
     assert L.sdrb_plan_fingerprint(None, None) == -1
     assert L.sdrb_bank_state_bytes(None) == 0
+
+
+def header_bounds(root):
+    """The record bounds as include/sdrb200.h states them: (samples behind SDRB_STATE_MAX_BLOCKS_DONE, SDRB_STATE_MAX_DC)."""
+    with open(os.path.join(root, "include", "sdrb200.h")) as f:
+        h = f.read()
+    shift = re.search(r"#define SDRB_STATE_MAX_BLOCKS_DONE\(block\) \(\(int64_t\)\(\(\(int64_t\)1 << (\d+)\) / \(int64_t\)\(block\)\)\)", h)
+    dc = re.search(r"#define SDRB_STATE_MAX_DC ([0-9.]+)f", h)
+    assert shift and dc
+    return 1 << int(shift.group(1)), float(dc.group(1))
+
+
+def test_counter_bound_leaves_headroom(root):
+    samples, _ = header_bounds(root)
+    assert samples == 2**62 and samples / 1536000 / (365.25 * 86400) > 95000      # years of signal at 1.536 MS/s
+    for p in all_plans(root):
+        block = B.Plan(p).block
+        top = samples // block
+        assert top * block <= 2**62 < (top + 1) * block
+        # a receiver loaded at the bound still has 2^62 samples before (blocks_done + b) * block overflows
+        assert (top + 2**62 // block) * block < 2**63
+
+
+def test_dc_recursion_stays_inside_the_record_bound(root):
+    """avept = avept * (1 - 1e-6) + 1e-6 * (x - 127) in float32 (sdrj.cpp:277-283), started at 0, on full-scale input: it
+    rises monotonically to the fixed point of its rounding, +-124.2353, inside SDRB_STATE_MAX_DC = 128. The recursion is
+    monotone in its input, so no byte sequence takes it further out than all 255 or all 0."""
+    from oracle import oracle as O
+    _, bound = header_bounds(root)
+    n = 4_000_000                                            # 4 time constants; the state stops moving after about 3.5
+    for v, sign in ((255, 1.0), (0, -1.0)):
+        t = O.dc_trace(np.full(2 * n, v, np.uint8), every=1)
+        for arm in (t.real, t.imag):
+            assert np.all(np.isfinite(arm)) and np.all(sign * arm >= 0)
+            peak = float(np.abs(arm).max())
+            assert arm[-1] == arm[-n // 8] and abs(peak - 124.2353) < 1e-4, (v, peak)   # settled at its rounding fixed point
+            assert peak <= bound
