@@ -216,6 +216,36 @@ int sdrb_bank_process_device(sdrb_bank *bank, const uint8_t *d_iq, size_t iq_str
  * is still ordered on `stream`. */
 int sdrb_bank_process_device_ex(sdrb_bank *bank, const uint8_t *d_iq, size_t iq_stride, int n_blocks,
                                 int16_t *d_pcm, float *d_tap, void *cuda_stream, void *input_ready_event);
+/*
+ * Stream-list calls: n_blocks callbacks for the listed receivers only; every other receiver of the
+ * bank is not touched. For live receivers that deliver callbacks at their own pace: process whoever
+ * has a callback ready, without waiting for the others and without feeding them filler.
+ *   streams  host array of n distinct stream indices in [0, n_streams), any order, 1 <= n <= n_streams;
+ *            the caller may reuse it as soon as the call returns. A bad list (or a NULL pointer)
+ *            returns SDRB_E_INVALID, names the entry in sdrb_last_error() and changes nothing.
+ * Device call: the layout, n_blocks, iq_stride, alignment and input_ready_event of
+ * sdrb_bank_process_device_ex. Stream s reads d_iq + s*iq_stride and writes PCM (tap) row s; rows of
+ * unlisted streams are never read in d_iq and never written in d_pcm or d_tap.
+ * Host call (synchronous; waits for asynchronous host calls first): h_iq[k] holds the
+ * n_blocks*block*2 bytes of stream streams[k] (pinned or pageable); h_pcm and h_tap (optional) are
+ * compact, [n][n_blocks][pcm_per_block], record k belonging to streams[k].
+ * State: listed receivers advance by n_blocks; the carried state of an unlisted receiver stays as it
+ * was, byte for byte (sdrb_bank_save_state of it gives the same record before and after). Calls are
+ * ordered like the other process calls. The inspection entry points (copy/read_main, _sub,
+ * _forward, _input, copy_dc_trace) are defined for the listed streams of the last call only, and
+ * sdrb_bank_spectrum_feed feeds only their displays.
+ * Exactness: everything except the sub-VFO cascade's products -- main outputs, forwarder bytes, the DC
+ * trace and its modes, blocks_done -- is bit-identical to the receiver run alone. Audio is within
+ * +-1 LSB of it: the sub-VFO cascade chooses its table-anchored or exact mixing path per group of up
+ * to eight streams, from the NCO phase of every stream in the group, and the two paths round
+ * differently. When every stream listed in a call is at the same callback count, audio is bit for
+ * bit too.
+ */
+int sdrb_bank_process_streams_device(sdrb_bank *bank, const int32_t *streams, int n,
+                                     const uint8_t *d_iq, size_t iq_stride, int n_blocks,
+                                     int16_t *d_pcm, float *d_tap, void *cuda_stream, void *input_ready_event);
+int sdrb_bank_process_streams_host(sdrb_bank *bank, const int32_t *streams, int n,
+                                   const uint8_t *const *h_iq, int n_blocks, int16_t *h_pcm, float *h_tap);
 /* Copy out the main VFO outputs (vfo::decimate[decimateCount], vfo.h:39) of the last
  * process call: cf32 [n_streams][n_blocks*block_out] on the device. */
 int sdrb_bank_copy_main(sdrb_bank *bank, int main_idx, int n_blocks, float *d_out_cf32, void *cuda_stream);
@@ -393,6 +423,11 @@ int sdrb_publisher_pool_open(const char *address, int bind, int n_sockets, sdrb_
 int sdrb_publisher_pool_sockets(const sdrb_publisher_pool *pool);
 int sdrb_publisher_pool_address(const sdrb_publisher_pool *pool, int k, char *buf, size_t len);
 int sdrb_publisher_pool_send_call(sdrb_publisher_pool *pool, const sdrb_plan *plan, const int16_t *h_pcm, int n_streams, int n_blocks);
+/* The compact [n][n_blocks][pcm_per_block] result of sdrb_bank_process_streams_host: record k is receiver streams[k], sent on
+ * socket streams[k] % n_sockets like in send_call. NULL pointers, n or n_blocks < 1, and negative or repeated stream indices
+ * return SDRB_E_INVALID and send nothing. */
+int sdrb_publisher_pool_send_streams(sdrb_publisher_pool *pool, const sdrb_plan *plan, const int16_t *h_pcm,
+                                     const int32_t *streams, int n, int n_blocks);
 void sdrb_publisher_pool_close(sdrb_publisher_pool *pool);
 
 /* ---- ingest front ends, host side (the library opens no socket and no dongle) ---- */

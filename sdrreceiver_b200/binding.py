@@ -92,6 +92,8 @@ def lib():
         "sdrb_bank_write_state": (i, [vp, vp, i, vp]),
         "sdrb_bank_process_device": (i, [vp, vp, sz, i, vp, vp, vp]),
         "sdrb_bank_process_device_ex": (i, [vp, vp, sz, i, vp, vp, vp, vp]),
+        "sdrb_bank_process_streams_device": (i, [vp, vp, i, vp, sz, i, vp, vp, vp, vp]),
+        "sdrb_bank_process_streams_host": (i, [vp, vp, i, vp, i, vp, vp]),
         "sdrb_bank_copy_main": (i, [vp, i, i, vp, vp]),
         "sdrb_bank_copy_dc_trace": (i, [vp, i, vp, vp, vp]),
         "sdrb_bank_copy_forward": (i, [vp, i, i, vp, vp]),
@@ -153,6 +155,7 @@ def lib():
         "sdrb_publisher_pool_sockets": (i, [vp]),
         "sdrb_publisher_pool_address": (i, [vp, i, C.c_char_p, C.c_size_t]),
         "sdrb_publisher_pool_send_call": (i, [vp, vp, vp, i, i]),
+        "sdrb_publisher_pool_send_streams": (i, [vp, vp, vp, vp, i, i]),
         "sdrb_publisher_pool_close": (None, [vp]),
         "sdrb_last_error": (C.c_char_p, []),
         "sdrb_version": (C.c_char_p, []),
@@ -316,6 +319,40 @@ class Bank:
         call overlap the previous call (sdrb_bank_process_device_ex)."""
         _check(lib().sdrb_bank_process_device_ex(self.h, d_iq_ptr, iq_stride, n_blocks, d_pcm_ptr, d_tap_ptr,
                                                  cuda_stream, input_ready_event), "sdrb_bank_process_device_ex")
+
+    def process_streams_device(self, streams, d_iq_ptr, iq_stride, n_blocks, d_pcm_ptr, d_tap_ptr=None, cuda_stream=None,
+                               input_ready_event=None):
+        """n_blocks callbacks for the listed streams only, in the layout of process_device: stream s reads
+        d_iq + s*iq_stride and writes PCM row s; every other stream is left as it was (sdrb_bank_process_streams_device)."""
+        s, sp = self._streams(streams)
+        _check(lib().sdrb_bank_process_streams_device(self.h, sp, s.size, d_iq_ptr, iq_stride, n_blocks, d_pcm_ptr, d_tap_ptr,
+                                                      cuda_stream, input_ready_event), "sdrb_bank_process_streams_device")
+
+    def process_streams_host(self, streams, rows, n_blocks, want_tap=False):
+        """rows[k]: the uint8 input of stream streams[k] (n_blocks*block*2 bytes: a numpy array, or an int host address) ->
+        compact (pcm int16 [len(streams), n_blocks, pcm_per_block], tap) with record k for streams[k]
+        (sdrb_bank_process_streams_host)."""
+        s, sp = self._streams(streams)
+        if len(rows) != s.size:
+            raise SdrbError("process_streams_host: %d rows for %d streams" % (len(rows), s.size))
+        need = n_blocks * self.plan.block * 2
+        keep, ptrs = [], (C.c_void_p * s.size)()
+        for k, r in enumerate(rows):
+            if isinstance(r, int):
+                ptrs[k] = r
+                continue
+            a = np.ascontiguousarray(r, dtype=np.uint8).reshape(-1)
+            if a.size < need:
+                raise SdrbError("process_streams_host: row %d has %d bytes, needs %d" % (k, a.size, need))
+            keep.append(a)
+            ptrs[k] = a.ctypes.data
+        pcm = np.zeros((s.size, n_blocks, self.plan.pcm_per_block), dtype=np.int16)
+        tap = np.zeros(pcm.shape, dtype=np.float32) if want_tap else None
+        _check(lib().sdrb_bank_process_streams_host(self.h, sp, s.size, C.cast(ptrs, C.c_void_p), n_blocks,
+                                                    pcm.ctypes.data_as(C.c_void_p),
+                                                    tap.ctypes.data_as(C.c_void_p) if want_tap else None),
+               "sdrb_bank_process_streams_host")
+        return pcm, tap
 
     def copy_main(self, main_idx, n_blocks, d_out_ptr, cuda_stream=None):
         _check(lib().sdrb_bank_copy_main(self.h, main_idx, n_blocks, d_out_ptr, cuda_stream), "sdrb_bank_copy_main")

@@ -209,17 +209,17 @@ static int v2_pick_threads(int halo, const char *env) {
     return best;
 }
 
-template <int NT>
+template <int NT, bool MAP = false>
 static void launch_k1_v2(const K1V2Params &q, bool dc, int ns, int block, cudaStream_t st, bool bulk = false) {
     const int tiles = (block + k1v2_adv<NT>() - 1) / k1v2_adv<NT>();
     const dim3 grid((unsigned)ns, (unsigned)((tiles + K1_TPC - 1) / K1_TPC), 1u);
     if (NT == 64 && bulk) {          // the bulk-copy (TMA) prefetch exists for the default CTA size; SDRB_K1_BULK=0 turns it off
-        if (dc) k1_v2<true, 64, true><<<grid, 64, k1v2_smem_bulk<64>(), st>>>(q);
-        else k1_v2<false, 64, true><<<grid, 64, k1v2_smem_bulk<64>(), st>>>(q);
+        if (dc) k1_v2<true, 64, true, MAP><<<grid, 64, k1v2_smem_bulk<64>(), st>>>(q);
+        else k1_v2<false, 64, true, MAP><<<grid, 64, k1v2_smem_bulk<64>(), st>>>(q);
         return;
     }
-    if (dc) k1_v2<true, NT><<<grid, NT, k1v2_smem<NT>(), st>>>(q);
-    else k1_v2<false, NT><<<grid, NT, k1v2_smem<NT>(), st>>>(q);
+    if (dc) k1_v2<true, NT, false, MAP><<<grid, NT, k1v2_smem<NT>(), st>>>(q);
+    else k1_v2<false, NT, false, MAP><<<grid, NT, k1v2_smem<NT>(), st>>>(q);
 }
 
 struct SubGroup {           // sub VFOs of one main VFO (at most V2_MAX_VFO) -> one k2a_v2 launch
@@ -278,6 +278,10 @@ struct sdrb_bank {
     int *qtab_buf(int par) const { return (int *)dc_qtab.p + (size_t)par * 512 * (size_t)n_streams; }
     DcAnchor *anchor_buf(int par) const { return (DcAnchor *)dc_anchor.p + (size_t)par * 2 * (size_t)n_streams; }
     uint2 *table_buf(int par) const { return (uint2 *)dc_table.p + (size_t)par * 2 * (size_t)n_streams * (size_t)(dc_stride + DC_HALO_BLKS); }
+    // stream-list calls: the device copy of the call's list, per call parity like the tables above -- the DC pre-pass of call n+1
+    // reads its list while the filters of call n still read theirs
+    DevBuf stream_list;
+    int *list_buf(int par) const { return (int *)stream_list.p + (size_t)par * (size_t)n_streams; }
     // descriptors
     K1Params k1{};          // cf32-input variant (vfo::process entry)
     K1V2Params k1v2{};
@@ -326,6 +330,7 @@ struct sdrb_bank {
     const uint8_t *last_iq = nullptr; size_t last_iq_stride = 0;
     const float2 *last_cf = nullptr; size_t last_cf_stride = 0;
     int last_blocks = 0, last_par = 0;
+    const int *last_map = nullptr; int last_n = 0;   // a stream-list call: its device list and length (inspection covers those streams)
     // host staging for process_host
     DevBuf d_iq, d_pcm, d_tap, d_cf, d_fwd;
     cudaStream_t s_copy_in = nullptr, s_compute = nullptr, s_copy_out = nullptr;
@@ -358,7 +363,7 @@ extern "C" void sdrb_bank_destroy(sdrb_bank *b) {
     cudaDeviceSynchronize();                                 // asynchronous host calls may still be in flight
     DevBuf *all[] = {&b->luts, &b->taps, &b->blocks_done, &b->dc_state, &b->raw_tail, &b->cf_tail, &b->dc_anchor, &b->dc_stats, &b->dc_table, &b->dc_qtab,
                      &b->main_out, &b->zbuf, &b->dbuf, &b->cascdev, &b->rfdev, &b->latedev, &b->usbdev, &b->carry,
-                     &b->main_tails, &b->sub_tails, &b->state_items, &b->state_streams, &b->d_state,
+                     &b->main_tails, &b->sub_tails, &b->state_items, &b->state_streams, &b->d_state, &b->stream_list,
                      &b->d_iq, &b->d_pcm, &b->d_tap, &b->d_cf, &b->d_fwd, &b->k3_rrel};
     for (DevBuf *d : all) d->release();
     if (b->ev_state) cudaEventDestroy(b->ev_state);
@@ -455,6 +460,7 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
     b->dc_stride = max_blocks * (h.block / DC_BLK);
     BANK_TRY(b->dc_anchor.alloc(2 * sizeof(DcAnchor) * 2 * (size_t)n_streams));
     BANK_TRY(b->dc_qtab.alloc(2 * sizeof(int) * 512 * (size_t)n_streams));
+    BANK_TRY(b->stream_list.alloc(2 * sizeof(int) * (size_t)n_streams));
     BANK_TRY(b->dc_stats.alloc(h.correct_dc ? sizeof(DcStats) * 2 * (size_t)n_streams * (size_t)b->dc_stride + 1024 : 16));
     BANK_TRY(b->dc_table.alloc(h.correct_dc ? 2 * sizeof(uint2) * 2 * (size_t)n_streams * (size_t)(b->dc_stride + DC_HALO_BLKS) : 64));
     // the halo entries a state record saves exist before any u8 call writes them (a bank fed only cf32 input): start them at zero
@@ -751,6 +757,9 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
         BANK_CU(cudaFuncSetAttribute(k2a_v3<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         BANK_CU(cudaFuncSetAttribute(k2a_v3<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         BANK_CU(cudaFuncSetAttribute(k2a_v3<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        BANK_CU((cudaFuncSetAttribute(k2a_v3<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)));
+        BANK_CU((cudaFuncSetAttribute(k2a_v3<3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)));
+        BANK_CU((cudaFuncSetAttribute(k2a_v3<5, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)));
     }
     if (!latedev.empty()) BANK_CU(cudaMemcpy(b->latedev.p, latedev.data(), sizeof(LateDev) * latedev.size(), cudaMemcpyHostToDevice));
     if (!usbdev.empty()) BANK_CU(cudaMemcpy(b->usbdev.p, usbdev.data(), sizeof(UsbDev) * usbdev.size(), cudaMemcpyHostToDevice));
@@ -776,8 +785,29 @@ extern "C" int sdrb_bank_create(const sdrb_plan *plan, int device, int n_streams
     b->uv_eo_rows = 34 + b->uv_np_max / 32;
     b->uv_warp_floats = std::max(UV_IN_FLOATS, 2 * b->uv_eo_rows * UV_ROW);
     b->uv_smem = sizeof(float) * (2 * (size_t)(64 + b->uv_np_max) + (size_t)UV_WARPS * b->uv_warp_floats);
-    BANK_CU(cudaFuncSetAttribute(k2b_v2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->uv_smem));
-    BANK_CU(cudaFuncSetAttribute(k0_dc_walk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DCW_SMEM));
+    BANK_CU(cudaFuncSetAttribute(k2b_v2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->uv_smem));
+    BANK_CU(cudaFuncSetAttribute(k0_dc_walk<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DCW_SMEM));
+    // the stream-list instantiations (MAP = true) of the kernels above and below
+    BANK_CU(cudaFuncSetAttribute(k2b_v2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->uv_smem));
+    BANK_CU(cudaFuncSetAttribute(k0_dc_walk<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DCW_SMEM));
+    BANK_CU((cudaFuncSetAttribute(k2_late_v2<5, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lv_smem<5>())));
+    BANK_CU((cudaFuncSetAttribute(k2_late_v2<6, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lv_smem<6>())));
+    BANK_CU((cudaFuncSetAttribute(k2_late_v2<5, 10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lv_smem<5>())));
+    BANK_CU((cudaFuncSetAttribute(k2_late_v2<6, 13, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lv_smem<6>())));
+    BANK_CU((cudaFuncSetAttribute(k2a_v2<64, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<64>::SMEM)));
+    BANK_CU((cudaFuncSetAttribute(k2a_v2<96, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<96>::SMEM)));
+    BANK_CU((cudaFuncSetAttribute(k2a_v2<128, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<128>::SMEM)));
+    BANK_CU((cudaFuncSetAttribute(k2a_v2<64, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<64>::SMEM)));
+    BANK_CU((cudaFuncSetAttribute(k2a_v2<96, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<96>::SMEM)));
+    BANK_CU((cudaFuncSetAttribute(k2a_v2<128, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V2L<128>::SMEM)));
+    BANK_CU((cudaFuncSetAttribute(k1_v2<true, 64, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1v2_smem<64>())));
+    BANK_CU((cudaFuncSetAttribute(k1_v2<false, 64, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1v2_smem<64>())));
+    BANK_CU((cudaFuncSetAttribute(k1_v2<true, 96, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1v2_smem<96>())));
+    BANK_CU((cudaFuncSetAttribute(k1_v2<false, 96, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1v2_smem<96>())));
+    BANK_CU((cudaFuncSetAttribute(k1_v2<true, 128, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1v2_smem<128>())));
+    BANK_CU((cudaFuncSetAttribute(k1_v2<false, 128, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1v2_smem<128>())));
+    BANK_CU((cudaFuncSetAttribute(k1_v2<true, 64, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1v2_smem_bulk<64>())));
+    BANK_CU((cudaFuncSetAttribute(k1_v2<false, 64, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1v2_smem_bulk<64>())));
     BANK_CU((cudaFuncSetAttribute(k2_late_v2<5, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lv_smem<5>())));
     BANK_CU((cudaFuncSetAttribute(k2_late_v2<6, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lv_smem<6>())));
     BANK_CU((cudaFuncSetAttribute(k2_late_v2<5, 10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lv_smem<5>())));
@@ -872,6 +902,9 @@ struct CallCtx {
     int n_blocks = 0;
     int16_t *d_pcm = nullptr; float *d_tap = nullptr;
     int par = 0;                                            // which dc_anchor / dc_table buffer this call owns
+    // stream-list calls: the caller's list (host) and its device copy; the launch helpers then get s0 = 0 and ns = its length
+    const int32_t *h_map = nullptr; int n_map = 0;
+    const int *map = nullptr;
 };
 
 // DC recursion of callback cb for streams [s0, s0+ns) on the side stream `sd`: (anchor once per
@@ -884,22 +917,37 @@ static int enqueue_dc_cb(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaStr
     if (ready) CU_TRY(cudaStreamWaitEvent(sd, ready, 0));
     if (cb == 0) {
         TimedScope t(b, sd, 0);
-        k0_dc_anchor<<<(unsigned)((2 * ns + 127) / 128), 128, 0, sd>>>((const float2 *)b->dc_state.p,
-                                                                      b->anchor_buf(c.par), ns, s0);
-        k0_dc_qtab<<<(unsigned)(2 * ns), 256, 0, sd>>>(b->anchor_buf(c.par), b->qtab_buf(c.par), s0);
+        const dim3 ga((unsigned)((2 * ns + 127) / 128));
+        if (c.map) {
+            k0_dc_anchor<true><<<ga, 128, 0, sd>>>((const float2 *)b->dc_state.p, b->anchor_buf(c.par), ns, s0, c.map);
+            k0_dc_qtab<true><<<(unsigned)(2 * ns), 256, 0, sd>>>(b->anchor_buf(c.par), b->qtab_buf(c.par), s0, c.map);
+        } else {
+            k0_dc_anchor<<<ga, 128, 0, sd>>>((const float2 *)b->dc_state.p, b->anchor_buf(c.par), ns, s0);
+            k0_dc_qtab<<<(unsigned)(2 * ns), 256, 0, sd>>>(b->anchor_buf(c.par), b->qtab_buf(c.par), s0);
+        }
         (*nl) += 2;
     }
     {
         TimedScope t(b, sd, 0);
-        k0_dc_blocks<<<dim3((unsigned)((per_cb + 127) / 128), (unsigned)ns), 128, 0, sd>>>(
-            c.d_iq, c.iq_stride, b->anchor_buf(c.par), b->qtab_buf(c.par), (DcStats *)b->dc_stats.p, b->dc_stride, cb * per_cb,
-            per_cb, s0);
+        const dim3 gb((unsigned)((per_cb + 127) / 128), (unsigned)ns);
+        if (c.map)
+            k0_dc_blocks<true><<<gb, 128, 0, sd>>>(c.d_iq, c.iq_stride, b->anchor_buf(c.par), b->qtab_buf(c.par), (DcStats *)b->dc_stats.p,
+                                                   b->dc_stride, cb * per_cb, per_cb, s0, c.map);
+        else
+            k0_dc_blocks<<<gb, 128, 0, sd>>>(c.d_iq, c.iq_stride, b->anchor_buf(c.par), b->qtab_buf(c.par), (DcStats *)b->dc_stats.p,
+                                             b->dc_stride, cb * per_cb, per_cb, s0);
     }
     {
         TimedScope t(b, sd, 0);
-        k0_dc_walk<<<(unsigned)ns, 64, DCW_SMEM, sd>>>(c.d_iq, c.iq_stride, (const DcStats *)b->dc_stats.p, b->dc_stride,
-                                                      b->anchor_buf(c.par), b->qtab_buf(c.par), (float2 *)b->dc_state.p, b->table_buf(c.par),
-                                                      b->dc_stride + DC_HALO_BLKS, cb * per_cb, per_cb, s0);
+        if (c.map)
+            k0_dc_walk<true><<<(unsigned)ns, 64, DCW_SMEM, sd>>>(c.d_iq, c.iq_stride, (const DcStats *)b->dc_stats.p, b->dc_stride,
+                                                                b->anchor_buf(c.par), b->qtab_buf(c.par), (float2 *)b->dc_state.p,
+                                                                b->table_buf(c.par), b->dc_stride + DC_HALO_BLKS, cb * per_cb, per_cb, s0,
+                                                                c.map);
+        else
+            k0_dc_walk<<<(unsigned)ns, 64, DCW_SMEM, sd>>>(c.d_iq, c.iq_stride, (const DcStats *)b->dc_stats.p, b->dc_stride,
+                                                          b->anchor_buf(c.par), b->qtab_buf(c.par), (float2 *)b->dc_state.p, b->table_buf(c.par),
+                                                          b->dc_stride + DC_HALO_BLKS, cb * per_cb, per_cb, s0);
     }
     (*nl) += 2;
     CU_TRY(cudaEventRecord(done, sd));
@@ -921,8 +969,13 @@ static int enqueue_ingest_cb(sdrb_bank *b, const CallCtx &c, int s0, int ns, cud
         K1V2Params q = b->k1v2;
         q.iq = c.d_iq; q.iq_stride = c.iq_stride; q.stream0 = s0; q.b0 = cb;
         q.dc_table = b->table_buf(c.par); q.dc_anchor = b->anchor_buf(c.par);
+        q.map = c.map;
         TimedScope t(b, st, 1);
-        if (b->k1_threads == 64) launch_k1_v2<64>(q, h.correct_dc, ns, h.block, st, b->k1_bulk);
+        if (c.map) {
+            if (b->k1_threads == 64) launch_k1_v2<64, true>(q, h.correct_dc, ns, h.block, st, b->k1_bulk);
+            else if (b->k1_threads == 96) launch_k1_v2<96, true>(q, h.correct_dc, ns, h.block, st);
+            else launch_k1_v2<128, true>(q, h.correct_dc, ns, h.block, st);
+        } else if (b->k1_threads == 64) launch_k1_v2<64>(q, h.correct_dc, ns, h.block, st, b->k1_bulk);
         else if (b->k1_threads == 96) launch_k1_v2<96>(q, h.correct_dc, ns, h.block, st);
         else launch_k1_v2<128>(q, h.correct_dc, ns, h.block, st);
     }
@@ -959,7 +1012,7 @@ static int k3_slots(K kernel, int threads, size_t smem) {
 // (the rotation table is per CTA, a ring per warp): take the CTA size with the most resident warps (25E's 15 two-stage VFOs: 6 warps,
 // 12 per SM).
 template <int MAXS>
-static void launch_k3(sdrb_bank *b, size_t gi, int ns, int ncb, cudaStream_t st) {
+static void launch_k3(sdrb_bank *b, size_t gi, int ns, int ncb, cudaStream_t st, bool map) {
     const SubGroup &g = b->groups[gi];
     K3Params &kp = b->k3[gi];
     int &slots = b->k3_slots[gi], &cw = b->k3_cw[gi];
@@ -978,17 +1031,20 @@ static void launch_k3(sdrb_bank *b, size_t gi, int ns, int ncb, cudaStream_t st)
     dim3 grid;
     k3_geometry(g, kp, ns, ncb, cw, slots, &grid);
     TimedScope t(b, st, 2);
-    k2a_v3<MAXS><<<grid, cw * 32, k3_cta_smem_bytes(g.count, cw, rows), st>>>(kp);
+    if (map) k2a_v3<MAXS, true><<<grid, cw * 32, k3_cta_smem_bytes(g.count, cw, rows), st>>>(kp);
+    else k2a_v3<MAXS><<<grid, cw * 32, k3_cta_smem_bytes(g.count, cw, rows), st>>>(kp);
 }
 
 // The half-band stages of the deep main VFOs (subs = false, timed with the ingest class) or sub VFOs (timed with the cascades)
 // that their mixing kernel does not run, for callbacks cb0 .. cb0+ncb-1: one k_hb_tail launch, nothing for a plan without them.
-static int enqueue_tails(sdrb_bank *b, bool subs, int s0, int ns, cudaStream_t st, int cb0, int ncb, int *nl) {
+static int enqueue_tails(sdrb_bank *b, const CallCtx &c, bool subs, int s0, int ns, cudaStream_t st, int cb0, int ncb, int *nl) {
     const int n = subs ? b->n_sub_tails : b->n_main_tails, tiles = subs ? b->sub_tail_tiles : b->main_tail_tiles;
     if (n == 0) return SDRB_OK;
     TimedScope t(b, st, subs ? 2 : 1);
-    k_hb_tail<<<dim3((unsigned)ns, (unsigned)(n * tiles), (unsigned)ncb), TAIL_NT, V2L<TAIL_NT>::SMEM, st>>>(
-        (const TailDev *)(subs ? b->sub_tails.p : b->main_tails.p), tiles, s0, cb0);
+    const dim3 grid((unsigned)ns, (unsigned)(n * tiles), (unsigned)ncb);
+    const TailDev *devs = (const TailDev *)(subs ? b->sub_tails.p : b->main_tails.p);
+    if (c.map) k_hb_tail<true><<<grid, TAIL_NT, V2L<TAIL_NT>::SMEM, st>>>(devs, tiles, s0, cb0, c.map);
+    else k_hb_tail<<<grid, TAIL_NT, V2L<TAIL_NT>::SMEM, st>>>(devs, tiles, s0, cb0);
     (*nl)++;
     return SDRB_OK;
 }
@@ -999,19 +1055,27 @@ static int enqueue_subs(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaStre
         const size_t gi = (size_t)(&g - b->groups.data());
         if (g.v3) {
             K3Params &kp = b->k3[gi];
-            kp.stream0 = s0; kp.stream_end = s0 + ns; kp.b0 = cb0;
+            kp.stream0 = s0; kp.stream_end = s0 + ns; kp.b0 = cb0; kp.map = c.map;
             if (b->k3_slots.size() <= gi) { b->k3_slots.resize(gi + 1, -1); b->k3_cw.resize(gi + 1, 0); }
-            if (g.v3_maxs == 2) launch_k3<2>(b, gi, ns, ncb, st);
-            else if (g.v3_maxs == 3) launch_k3<3>(b, gi, ns, ncb, st);
-            else launch_k3<5>(b, gi, ns, ncb, st);
+            if (g.v3_maxs == 2) launch_k3<2>(b, gi, ns, ncb, st, c.map != nullptr);
+            else if (g.v3_maxs == 3) launch_k3<3>(b, gi, ns, ncb, st, c.map != nullptr);
+            else launch_k3<5>(b, gi, ns, ncb, st, c.map != nullptr);
             (*nl)++;
             continue;
         }
         K2V2Params &kp = b->k2v2[gi];
-        kp.stream0 = s0; kp.b0 = cb0;
+        kp.stream0 = s0; kp.b0 = cb0; kp.map = c.map;
         TimedScope t(b, st, 2);
         const dim3 grid((unsigned)ns, (unsigned)g.tiles, (unsigned)ncb);
-        if (g.ragged) {
+        if (c.map) {
+            if (g.ragged) {
+                if (g.threads == 64) k2a_v2<64, true, true><<<grid, 64, V2L<64>::SMEM, st>>>(kp);
+                else if (g.threads == 96) k2a_v2<96, true, true><<<grid, 96, V2L<96>::SMEM, st>>>(kp);
+                else k2a_v2<128, true, true><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
+            } else if (g.threads == 64) k2a_v2<64, false, true><<<grid, 64, V2L<64>::SMEM, st>>>(kp);
+            else if (g.threads == 96) k2a_v2<96, false, true><<<grid, 96, V2L<96>::SMEM, st>>>(kp);
+            else k2a_v2<128, false, true><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
+        } else if (g.ragged) {
             if (g.threads == 64) k2a_v2<64, true><<<grid, 64, V2L<64>::SMEM, st>>>(kp);
             else if (g.threads == 96) k2a_v2<96, true><<<grid, 96, V2L<96>::SMEM, st>>>(kp);
             else k2a_v2<128, true><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
@@ -1020,7 +1084,7 @@ static int enqueue_subs(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaStre
         else k2a_v2<128><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
         (*nl)++;
     }
-    return enqueue_tails(b, true, s0, ns, st, cb0, ncb, nl);
+    return enqueue_tails(b, c, true, s0, ns, st, cb0, ncb, nl);
 }
 
 // /late FIR and USB audio of callbacks cb0 .. cb0+ncb-1. `out_done` (optional) is recorded at the end.
@@ -1033,14 +1097,20 @@ static int enqueue_audio(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaStr
             const dim3 grid((unsigned)ns, (unsigned)b->n_late, (unsigned)((ncb * b->max_late_samples + LV_TILE - 1) / LV_TILE));
             // late_taps_per_phase: the reference's 49-tap /5 and 73-tap /6 filters get their tap loops at compile time
             const LateDev *ld = (const LateDev *)b->latedev.p;
-            if (b->late_factor == 5 && b->late_taps_per_phase == 10) k2_late_v2<5, 10><<<grid, LV_THREADS, lv_smem<5>(), st>>>(ld, cb0, ncb, s0);
+            if (c.map) {
+                if (b->late_factor == 5 && b->late_taps_per_phase == 10) k2_late_v2<5, 10, true><<<grid, LV_THREADS, lv_smem<5>(), st>>>(ld, cb0, ncb, s0, c.map);
+                else if (b->late_factor == 5) k2_late_v2<5, 0, true><<<grid, LV_THREADS, lv_smem<5>(), st>>>(ld, cb0, ncb, s0, c.map);
+                else if (b->late_taps_per_phase == 13) k2_late_v2<6, 13, true><<<grid, LV_THREADS, lv_smem<6>(), st>>>(ld, cb0, ncb, s0, c.map);
+                else k2_late_v2<6, 0, true><<<grid, LV_THREADS, lv_smem<6>(), st>>>(ld, cb0, ncb, s0, c.map);
+            } else if (b->late_factor == 5 && b->late_taps_per_phase == 10) k2_late_v2<5, 10><<<grid, LV_THREADS, lv_smem<5>(), st>>>(ld, cb0, ncb, s0);
             else if (b->late_factor == 5) k2_late_v2<5, 0><<<grid, LV_THREADS, lv_smem<5>(), st>>>(ld, cb0, ncb, s0);
             else if (b->late_taps_per_phase == 13) k2_late_v2<6, 13><<<grid, LV_THREADS, lv_smem<6>(), st>>>(ld, cb0, ncb, s0);
             else k2_late_v2<6, 0><<<grid, LV_THREADS, lv_smem<6>(), st>>>(ld, cb0, ncb, s0);
         } else {
             const int tiles = (ncb * b->max_late_samples + LATE_TILE - 1) / LATE_TILE;
-            k2_late_fir<<<dim3((unsigned)ns, (unsigned)b->n_late, (unsigned)tiles), LATE_TILE, 0, st>>>(
-                (const LateDev *)b->latedev.p, cb0, ncb, s0);
+            const dim3 grid((unsigned)ns, (unsigned)b->n_late, (unsigned)tiles);
+            if (c.map) k2_late_fir<true><<<grid, LATE_TILE, 0, st>>>((const LateDev *)b->latedev.p, cb0, ncb, s0, c.map);
+            else k2_late_fir<<<grid, LATE_TILE, 0, st>>>((const LateDev *)b->latedev.p, cb0, ncb, s0);
         }
         (*nl)++;
     }
@@ -1049,7 +1119,7 @@ static int enqueue_audio(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaStr
         up.devs = (const UsbDev *)b->usbdev.p; up.pcm = c.d_pcm; up.tap = c.d_tap;
         up.n_blocks = c.n_blocks; up.cb0 = cb0; up.ncb = ncb; up.stream0 = s0; up.stream_end = s0 + ns;
         up.pcm_per_block = h.pcm_per_block; up.warp_floats = b->uv_warp_floats; up.eo_rows = b->uv_eo_rows;
-        up.np_max = b->uv_np_max;
+        up.np_max = b->uv_np_max; up.map = c.map;
         int max_tiles = 0;
         for (size_t k = 0; k < b->uv_vfo_out.size() && k < (size_t)SDRB_MAX_SUB; k++) {
             const int tile_out = UV_USB - b->uv_vfo_np[k];
@@ -1058,8 +1128,9 @@ static int enqueue_audio(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaStr
             max_tiles = std::max(max_tiles, tiles);
         }
         TimedScope t(b, st, 4);
-        k2b_v2<<<dim3((unsigned)((ns + UV_WARPS - 1) / UV_WARPS), (unsigned)b->n_usb, (unsigned)max_tiles), UV_WARPS * 32,
-                 b->uv_smem, st>>>(up);
+        const dim3 grid((unsigned)((ns + UV_WARPS - 1) / UV_WARPS), (unsigned)b->n_usb, (unsigned)max_tiles);
+        if (c.map) k2b_v2<true><<<grid, UV_WARPS * 32, b->uv_smem, st>>>(up);
+        else k2b_v2<<<grid, UV_WARPS * 32, b->uv_smem, st>>>(up);
         (*nl)++;
     }
     if (out_done) CU_TRY(cudaEventRecord(out_done, st));
@@ -1072,7 +1143,7 @@ static int enqueue_main_cb(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaS
                            cudaEvent_t out_done, int *nl) {
     int rc;
     if ((rc = enqueue_ingest_cb(b, c, s0, ns, st, cb, wait, nl)) != SDRB_OK) return rc;
-    if ((rc = enqueue_tails(b, false, s0, ns, st, cb, 1, nl)) != SDRB_OK) return rc;
+    if ((rc = enqueue_tails(b, c, false, s0, ns, st, cb, 1, nl)) != SDRB_OK) return rc;
     if ((rc = enqueue_subs(b, c, s0, ns, st, cb, 1, nl)) != SDRB_OK) return rc;
     return enqueue_audio(b, c, s0, ns, st, cb, 1, out_done, nl);
 }
@@ -1081,33 +1152,64 @@ static int enqueue_main_cb(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaS
 static int enqueue_carry(sdrb_bank *b, const CallCtx &c, int s0, int ns, cudaStream_t st, int *nl) {
     const HostPlan &h = b->plan->h;
     const bool dc = h.correct_dc && !c.d_cf;
+    if (dc && c.map) {
+        // Every stream's DC halo moves from the buffer this call read (par) to the one the next call reads (par ^ 1); k3_carry then
+        // overwrites it for the listed streams. Without this an unlisted stream would find in its next call the halo of the call
+        // before its last one. Entries 0 .. DC_HALO_BLKS-1 of a stream are never written by the DC walk, so this does not race with
+        // a next call's DC pre-pass that already runs on table_buf(par ^ 1).
+        const size_t pitch = (size_t)(b->dc_stride + DC_HALO_BLKS) * 2 * sizeof(uint2);
+        CU_TRY(cudaMemcpy2DAsync(b->table_buf(c.par ^ 1), pitch, b->table_buf(c.par), pitch, 2 * DC_HALO_BLKS * sizeof(uint2),
+                                 (size_t)b->n_streams, cudaMemcpyDeviceToDevice, st));
+    }
     TimedScope t(b, st, 5);
-    k3_carry<<<dim3((unsigned)ns, (unsigned)(b->n_carry + 1)), 128, 0, st>>>(
-        (const CarryItem *)b->carry.p, b->n_carry, c.n_blocks, c.d_iq, c.iq_stride, h.block, (uint8_t *)b->raw_tail.p,
-        (long long *)b->blocks_done.p, dc ? b->table_buf(c.par) : nullptr, b->table_buf(c.par ^ 1), b->anchor_buf(c.par),
-        b->dc_stride + DC_HALO_BLKS, c.n_blocks * (h.block / DC_BLK), s0, c.d_cf, c.cf_stride, (float2 *)b->cf_tail.p);
+    const dim3 grid((unsigned)ns, (unsigned)(b->n_carry + 1));
+    if (c.map)
+        k3_carry<true><<<grid, 128, 0, st>>>(
+            (const CarryItem *)b->carry.p, b->n_carry, c.n_blocks, c.d_iq, c.iq_stride, h.block, (uint8_t *)b->raw_tail.p,
+            (long long *)b->blocks_done.p, dc ? b->table_buf(c.par) : nullptr, b->table_buf(c.par ^ 1), b->anchor_buf(c.par),
+            b->dc_stride + DC_HALO_BLKS, c.n_blocks * (h.block / DC_BLK), s0, c.d_cf, c.cf_stride, (float2 *)b->cf_tail.p, c.map);
+    else
+        k3_carry<<<grid, 128, 0, st>>>(
+            (const CarryItem *)b->carry.p, b->n_carry, c.n_blocks, c.d_iq, c.iq_stride, h.block, (uint8_t *)b->raw_tail.p,
+            (long long *)b->blocks_done.p, dc ? b->table_buf(c.par) : nullptr, b->table_buf(c.par ^ 1), b->anchor_buf(c.par),
+            b->dc_stride + DC_HALO_BLKS, c.n_blocks * (h.block / DC_BLK), s0, c.d_cf, c.cf_stride, (float2 *)b->cf_tail.p);
     (*nl)++;
     CU_TRY(cudaGetLastError());
     return SDRB_OK;
 }
 
-// Whole call for all streams of the bank on one stream (device-resident entry points): the DC walk
-// of callback cb+1 runs on the side stream while callback cb is filtered.
+// Whole call for all streams of the bank, or for the streams c.h_map lists, on one stream (device-resident entry points): the DC
+// walk of callback cb+1 runs on the side stream while callback cb is filtered.
 // `input_ready` (optional cudaEvent_t): the input of this call is valid once that event has fired.
 // The DC pre-pass then waits only for it (and for the call before the previous one, whose table
 // buffer it reuses) instead of for everything queued on `st` -- it overlaps the previous call.
 static int enqueue_all(sdrb_bank *b, CallCtx &c, cudaStream_t st, int *launches, cudaEvent_t input_ready = nullptr) {
     const HostPlan &h = b->plan->h;
     const bool dc = h.correct_dc && !c.d_cf;
-    const int ns = b->n_streams;
+    const int ns = c.h_map ? c.n_map : b->n_streams;
     int rc;
     c.par = b->dc_par;
     b->last_iq = c.d_iq; b->last_iq_stride = c.iq_stride; b->last_cf = c.d_cf; b->last_cf_stride = c.cf_stride;
     b->last_blocks = c.n_blocks; b->last_par = c.par;
+    b->last_map = c.h_map ? b->list_buf(c.par) : nullptr; b->last_n = ns;
     if (b->state_pending) {             // a save or load since the last call: the DC pre-pass and the filters come after it
         CU_TRY(cudaStreamWaitEvent(st, b->ev_state, 0));
         if (dc) CU_TRY(cudaStreamWaitEvent(b->s_dc[0], b->ev_state, 0));
         b->state_pending = false;
+    }
+    if (c.h_map) {
+        // the list goes where the call's first kernel runs; the call two before this one, which read the same buffer, must be over
+        cudaStream_t first = dc ? b->s_dc[0] : st;
+        if (dc && b->ev_end_valid[c.par]) CU_TRY(cudaStreamWaitEvent(first, b->ev_end[c.par], 0));
+        // without a DC pre-pass the first kernel reads d_iq on `st`: it waits for input_ready there (a DC plan's side stream does below)
+        if (!dc && input_ready) CU_TRY(cudaStreamWaitEvent(st, input_ready, 0));
+        const std::vector<int> list(c.h_map, c.h_map + ns);  // pageable: staged before cudaMemcpyAsync returns, the caller may reuse it
+        CU_TRY(cudaMemcpyAsync(b->list_buf(c.par), list.data(), sizeof(int) * (size_t)ns, cudaMemcpyHostToDevice, first));
+        c.map = b->list_buf(c.par);
+        if (dc) {                       // the filters on `st` read the list too
+            CU_TRY(cudaEventRecord(b->ev_entry[1], first));
+            CU_TRY(cudaStreamWaitEvent(st, b->ev_entry[1], 0));
+        }
     }
     if (dc) {
         cudaStream_t sd = b->s_dc[0];
@@ -1137,7 +1239,7 @@ static int enqueue_all(sdrb_bank *b, CallCtx &c, cudaStream_t st, int *launches,
         // (their warm-up tiles amortise), and the DC walk of the next call has the whole cascade/audio phase to hide in
         for (int cb = 0; cb < c.n_blocks; cb++)
             if ((rc = enqueue_ingest_cb(b, c, 0, ns, st, cb, dc ? b->ev_dc[0][(size_t)cb] : nullptr, launches)) != SDRB_OK) return rc;
-        if ((rc = enqueue_tails(b, false, 0, ns, st, 0, c.n_blocks, launches)) != SDRB_OK) return rc;
+        if ((rc = enqueue_tails(b, c, false, 0, ns, st, 0, c.n_blocks, launches)) != SDRB_OK) return rc;
         if ((rc = enqueue_subs(b, c, 0, ns, st, 0, c.n_blocks, launches)) != SDRB_OK) return rc;
         if ((rc = enqueue_audio(b, c, 0, ns, st, 0, c.n_blocks, nullptr, launches)) != SDRB_OK) return rc;
     }
@@ -1208,6 +1310,20 @@ static int check_process_args(sdrb_bank *b, const void *iq, size_t iq_stride, in
     return SDRB_OK;
 }
 
+// A list of n distinct streams of the bank (state records, stream-list calls) and the buffer that goes with it.
+static int check_stream_list(const sdrb_bank *b, const int32_t *streams, int n, const void *data, const char *who) {
+    if (!b || !streams || !data) { set_error(std::string(who) + ": NULL argument"); return SDRB_E_INVALID; }
+    if (n <= 0 || n > b->n_streams) { set_error(std::string(who) + ": n must be 1..n_streams"); return SDRB_E_INVALID; }
+    std::vector<char> seen((size_t)b->n_streams, 0);
+    for (int k = 0; k < n; k++) {
+        const int s = streams[k];
+        const char *bad = (s < 0 || s >= b->n_streams) ? "is outside 0..n_streams-1" : (seen[(size_t)s] ? "is listed twice" : nullptr);
+        if (bad) { set_error(std::string(who) + ": streams[" + std::to_string(k) + "] = " + std::to_string(s) + " " + bad); return SDRB_E_INVALID; }
+        seen[(size_t)s] = 1;
+    }
+    return SDRB_OK;
+}
+
 extern "C" int sdrb_bank_process_device_ex(sdrb_bank *b, const uint8_t *d_iq, size_t iq_stride, int n_blocks,
                                            int16_t *d_pcm, float *d_tap, void *cuda_stream, void *input_ready_event) {
     int rc = check_process_args(b, d_iq, iq_stride, n_blocks, d_pcm);
@@ -1223,6 +1339,19 @@ extern "C" int sdrb_bank_process_device_ex(sdrb_bank *b, const uint8_t *d_iq, si
 extern "C" int sdrb_bank_process_device(sdrb_bank *b, const uint8_t *d_iq, size_t iq_stride, int n_blocks,
                                         int16_t *d_pcm, float *d_tap, void *cuda_stream) {
     return sdrb_bank_process_device_ex(b, d_iq, iq_stride, n_blocks, d_pcm, d_tap, cuda_stream, nullptr);
+}
+
+extern "C" int sdrb_bank_process_streams_device(sdrb_bank *b, const int32_t *streams, int n, const uint8_t *d_iq, size_t iq_stride,
+                                                int n_blocks, int16_t *d_pcm, float *d_tap, void *cuda_stream, void *input_ready_event) {
+    int rc = check_stream_list(b, streams, n, d_iq, "sdrb_bank_process_streams_device");
+    if (rc != SDRB_OK || (rc = check_process_args(b, d_iq, iq_stride, n_blocks, d_pcm)) != SDRB_OK) return rc;
+    CU_TRY(cudaSetDevice(b->device));
+    if ((rc = host_drain(b)) != SDRB_OK) return rc;
+    b->last_launches = 0;
+    CallCtx c;
+    c.d_iq = d_iq; c.iq_stride = iq_stride; c.n_blocks = n_blocks; c.d_pcm = d_pcm; c.d_tap = d_tap;
+    c.h_map = streams; c.n_map = n;
+    return enqueue_all(b, c, (cudaStream_t)cuda_stream, &b->last_launches, (cudaEvent_t)input_ready_event);
 }
 
 extern "C" int sdrb_bank_copy_main(sdrb_bank *b, int main_idx, int n_blocks, float *d_out, void *cuda_stream) {
@@ -1300,9 +1429,14 @@ static int input_launch(sdrb_bank *b, int cb, int n, float2 *d_out, cudaStream_t
         return SDRB_OK;
     }
     const bool dc = h.correct_dc != 0;
-    k_input_samples<<<dim3((unsigned)((n / DC_BLK + 63) / 64), (unsigned)b->n_streams), 64, 0, st>>>(
-        b->last_iq, b->last_iq_stride, (size_t)cb * h.block, n, dc ? b->table_buf(b->last_par) : nullptr, b->anchor_buf(b->last_par),
-        b->dc_stride + DC_HALO_BLKS, cb * (h.block / DC_BLK), d_out);
+    const dim3 grid((unsigned)((n / DC_BLK + 63) / 64), (unsigned)(b->last_map ? b->last_n : b->n_streams));
+    if (b->last_map)                    // a stream-list call: the rows of its streams
+        k_input_samples<true><<<grid, 64, 0, st>>>(b->last_iq, b->last_iq_stride, (size_t)cb * h.block, n,
+                                                   dc ? b->table_buf(b->last_par) : nullptr, b->anchor_buf(b->last_par),
+                                                   b->dc_stride + DC_HALO_BLKS, cb * (h.block / DC_BLK), d_out, b->last_map);
+    else
+        k_input_samples<<<grid, 64, 0, st>>>(b->last_iq, b->last_iq_stride, (size_t)cb * h.block, n, dc ? b->table_buf(b->last_par) : nullptr,
+                                             b->anchor_buf(b->last_par), b->dc_stride + DC_HALO_BLKS, cb * (h.block / DC_BLK), d_out);
     CU_TRY(cudaGetLastError());
     return SDRB_OK;
 }
@@ -1336,9 +1470,13 @@ static int ensure_sub_z(sdrb_bank *b, int sub_idx, cudaStream_t st) {
     kp.in_stride = (long long)b->main_stride; kp.out_stride = (long long)b->z_stride;
     kp.count = 1; kp.lut_len = (int)s.lut.size(); kp.block_in = s.block_in; kp.HT = 0; kp.stream0 = 0; kp.b0 = 0;
     kp.blk_off = -b->last_blocks;
+    kp.map = b->last_map;
     const int tiles = (s.block_in + 128 * V2_CHUNK - 1) / (128 * V2_CHUNK);
-    const dim3 grid((unsigned)b->n_streams, (unsigned)tiles, (unsigned)b->last_blocks);
-    if (s.block_in % V2_CHUNK != 0) k2a_v2<128, true><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
+    const dim3 grid((unsigned)(b->last_map ? b->last_n : b->n_streams), (unsigned)tiles, (unsigned)b->last_blocks);
+    if (b->last_map) {                  // after a stream-list call only its streams have the counters the replay subtracts from
+        if (s.block_in % V2_CHUNK != 0) k2a_v2<128, true, true><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
+        else k2a_v2<128, false, true><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
+    } else if (s.block_in % V2_CHUNK != 0) k2a_v2<128, true><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
     else k2a_v2<128><<<grid, 128, V2L<128>::SMEM, st>>>(kp);
     CU_TRY(cudaGetLastError());
     return SDRB_OK;
@@ -1436,6 +1574,20 @@ extern "C" int sdrb_bank_host_wait_until(sdrb_bank *b, int max_in_flight) {
     return SDRB_OK;
 }
 
+// Device staging of the host entry points: one input row of max_blocks callbacks and one PCM (and tap) record per stream.
+static int host_staging(sdrb_bank *b, bool tap) {
+    const HostPlan &h = b->plan->h;
+    int rc;
+    if (!b->d_iq.p) {
+        rc = b->d_iq.alloc((size_t)b->max_blocks * h.block * 2 * (size_t)b->n_streams); if (rc) return rc;
+        rc = b->d_pcm.alloc((size_t)b->max_blocks * h.pcm_per_block * sizeof(int16_t) * (size_t)b->n_streams); if (rc) return rc;
+    }
+    if (tap && !b->d_tap.p) {
+        rc = b->d_tap.alloc((size_t)b->max_blocks * h.pcm_per_block * sizeof(float) * (size_t)b->n_streams); if (rc) return rc;
+    }
+    return SDRB_OK;
+}
+
 // Enqueues one host call. Consecutive calls may be in flight together (the staging buffers are shared,
 // so per chunk: the copy-in of call n+1 waits until call n no longer reads that region, the filters of
 // call n+1 wait until call n's copy-out of that region is done).
@@ -1451,13 +1603,7 @@ static int host_enqueue(sdrb_bank *b, const uint8_t *h_iq, size_t iq_stride, int
     const size_t in_row = (size_t)n_blocks * h.block * 2;
     const size_t rec = (size_t)n_blocks * h.pcm_per_block;
     const size_t in_max = (size_t)b->max_blocks * h.block * 2;
-    if (!b->d_iq.p) {
-        rc = b->d_iq.alloc(in_max * (size_t)b->n_streams); if (rc) return rc;
-        rc = b->d_pcm.alloc((size_t)b->max_blocks * h.pcm_per_block * sizeof(int16_t) * (size_t)b->n_streams); if (rc) return rc;
-    }
-    if (h_tap && !b->d_tap.p) {
-        rc = b->d_tap.alloc((size_t)b->max_blocks * h.pcm_per_block * sizeof(float) * (size_t)b->n_streams); if (rc) return rc;
-    }
+    if ((rc = host_staging(b, h_tap != nullptr)) != SDRB_OK) return rc;
     // Chunks = (callback, stream group), callback-major: copy-in, kernels and copy-out of different
     // chunks overlap on three streams (+ one DC side stream per group); a chunk's kernels start when
     // its copy has landed. Callback-major order gives every group's sequential DC walk the time of
@@ -1518,7 +1664,7 @@ static int host_enqueue(sdrb_bank *b, const uint8_t *h_iq, size_t iq_stride, int
     c.d_pcm = (int16_t *)b->d_pcm.p; c.d_tap = h_tap ? (float *)b->d_tap.p : nullptr;
     c.par = b->dc_par;
     b->last_iq = c.d_iq; b->last_iq_stride = c.iq_stride; b->last_cf = nullptr; b->last_cf_stride = 0;
-    b->last_blocks = n_blocks; b->last_par = c.par;
+    b->last_blocks = n_blocks; b->last_par = c.par; b->last_map = nullptr;
     b->dc_par ^= 1;                                       // host calls order themselves with per-chunk events
     b->ev_end_valid[0] = b->ev_end_valid[1] = false;
     for (int cb = 0; cb < n_blocks; cb++)
@@ -1582,6 +1728,41 @@ extern "C" int sdrb_bank_process_host(sdrb_bank *b, const uint8_t *h_iq, size_t 
     return host_drain(b);
 }
 
+// The stream-list call from host memory: each listed row into the staging row of its stream, the device-resident call on the
+// compute stream, each record back into its compact place. Synchronous.
+extern "C" int sdrb_bank_process_streams_host(sdrb_bank *b, const int32_t *streams, int n, const uint8_t *const *h_iq, int n_blocks,
+                                              int16_t *h_pcm, float *h_tap) {
+    static const char *who = "sdrb_bank_process_streams_host";
+    int rc = check_stream_list(b, streams, n, h_iq, who);
+    if (rc != SDRB_OK) return rc;
+    if (!h_pcm) { set_error(std::string(who) + ": NULL argument"); return SDRB_E_INVALID; }
+    if (n_blocks <= 0 || n_blocks > b->max_blocks) { set_error(std::string(who) + ": n_blocks outside 1..max_blocks"); return SDRB_E_INVALID; }
+    for (int k = 0; k < n; k++)
+        if (!h_iq[k]) { set_error(std::string(who) + ": h_iq[" + std::to_string(k) + "] is NULL"); return SDRB_E_INVALID; }
+    CU_TRY(cudaSetDevice(b->device));
+    if ((rc = host_drain(b)) != SDRB_OK || (rc = host_staging(b, h_tap != nullptr)) != SDRB_OK) return rc;
+    const HostPlan &h = b->plan->h;
+    const size_t in_max = (size_t)b->max_blocks * h.block * 2, row = (size_t)n_blocks * h.block * 2;
+    const size_t rec = (size_t)n_blocks * h.pcm_per_block;
+    cudaStream_t st = b->s_compute;
+    if (b->device_tail_pending) CU_TRY(cudaStreamWaitEvent(st, b->ev_device_tail, 0));   // the staging rows and the state it updates
+    for (int k = 0; k < n; k++)
+        CU_TRY(cudaMemcpyAsync((uint8_t *)b->d_iq.p + (size_t)streams[k] * in_max, h_iq[k], row, cudaMemcpyHostToDevice, st));
+    b->last_launches = 0;
+    CallCtx c;
+    c.d_iq = (const uint8_t *)b->d_iq.p; c.iq_stride = in_max; c.n_blocks = n_blocks;
+    c.d_pcm = (int16_t *)b->d_pcm.p; c.d_tap = h_tap ? (float *)b->d_tap.p : nullptr;
+    c.h_map = streams; c.n_map = n;
+    if ((rc = enqueue_all(b, c, st, &b->last_launches)) != SDRB_OK) return rc;
+    for (int k = 0; k < n; k++) {
+        const size_t at = (size_t)streams[k] * rec;
+        CU_TRY(cudaMemcpyAsync(h_pcm + (size_t)k * rec, (int16_t *)b->d_pcm.p + at, rec * sizeof(int16_t), cudaMemcpyDeviceToHost, st));
+        if (h_tap) CU_TRY(cudaMemcpyAsync(h_tap + (size_t)k * rec, (float *)b->d_tap.p + at, rec * sizeof(float), cudaMemcpyDeviceToHost, st));
+    }
+    CU_TRY(cudaStreamSynchronize(st));
+    return SDRB_OK;
+}
+
 extern "C" int sdrb_bank_process_cf32_host(sdrb_bank *b, const float *h_in, size_t stride_samples, int n_blocks,
                                            int16_t *h_pcm, float *h_tap) {
     if (!b || !h_in || !h_pcm || n_blocks <= 0 || n_blocks > b->max_blocks ||
@@ -1633,19 +1814,6 @@ extern "C" int sdrb_bank_last_launches(const sdrb_bank *b) { return b ? b->last_
 
 // ---- receiver state records (layout: include/sdrb200.h, kernels.cuh k_state_io) ----
 extern "C" size_t sdrb_bank_state_bytes(const sdrb_bank *b) { return b ? b->state_bytes : 0; }
-
-static int check_state_args(const sdrb_bank *b, const int32_t *streams, int n, const void *records, const char *who) {
-    if (!b || !streams || !records) { set_error(std::string(who) + ": NULL argument"); return SDRB_E_INVALID; }
-    if (n <= 0 || n > b->n_streams) { set_error(std::string(who) + ": n must be 1..n_streams"); return SDRB_E_INVALID; }
-    std::vector<char> seen((size_t)b->n_streams, 0);
-    for (int k = 0; k < n; k++) {
-        const int s = streams[k];
-        const char *bad = (s < 0 || s >= b->n_streams) ? "is outside 0..n_streams-1" : (seen[(size_t)s] ? "is listed twice" : nullptr);
-        if (bad) { set_error(std::string(who) + ": streams[" + std::to_string(k) + "] = " + std::to_string(s) + " " + bad); return SDRB_E_INVALID; }
-        seen[(size_t)s] = 1;
-    }
-    return SDRB_OK;
-}
 
 // Every header of a batch against this bank, before anything is written: a load is all or nothing.
 static int check_state_headers(const sdrb_bank *b, const int32_t *streams, int n, const unsigned char *h, size_t pitch, const char *who) {
@@ -1717,7 +1885,7 @@ static int state_enqueue(sdrb_bank *b, const int32_t *streams, int n, void *d_re
 }
 
 extern "C" int sdrb_bank_save_state(sdrb_bank *b, const int32_t *streams, int n, void *d_records, void *cuda_stream) {
-    int rc = check_state_args(b, streams, n, d_records, "sdrb_bank_save_state");
+    int rc = check_stream_list(b, streams, n, d_records, "sdrb_bank_save_state");
     if (rc != SDRB_OK) return rc;
     CU_TRY(cudaSetDevice(b->device));
     if ((rc = host_drain(b)) != SDRB_OK) return rc;
@@ -1725,7 +1893,7 @@ extern "C" int sdrb_bank_save_state(sdrb_bank *b, const int32_t *streams, int n,
 }
 
 extern "C" int sdrb_bank_load_state(sdrb_bank *b, const int32_t *streams, int n, const void *d_records, void *cuda_stream) {
-    int rc = check_state_args(b, streams, n, d_records, "sdrb_bank_load_state");
+    int rc = check_stream_list(b, streams, n, d_records, "sdrb_bank_load_state");
     if (rc != SDRB_OK) return rc;
     CU_TRY(cudaSetDevice(b->device));
     if ((rc = host_drain(b)) != SDRB_OK) return rc;
@@ -1746,7 +1914,7 @@ static int state_staging(sdrb_bank *b, int n) {
 }
 
 extern "C" int sdrb_bank_read_state(sdrb_bank *b, const int32_t *streams, int n, void *h_records) {
-    int rc = check_state_args(b, streams, n, h_records, "sdrb_bank_read_state");
+    int rc = check_stream_list(b, streams, n, h_records, "sdrb_bank_read_state");
     if (rc != SDRB_OK) return rc;
     CU_TRY(cudaSetDevice(b->device));
     if ((rc = host_drain(b)) != SDRB_OK || (rc = state_staging(b, n)) != SDRB_OK) return rc;
@@ -1758,7 +1926,7 @@ extern "C" int sdrb_bank_read_state(sdrb_bank *b, const int32_t *streams, int n,
 }
 
 extern "C" int sdrb_bank_write_state(sdrb_bank *b, const int32_t *streams, int n, const void *h_records) {
-    int rc = check_state_args(b, streams, n, h_records, "sdrb_bank_write_state");
+    int rc = check_stream_list(b, streams, n, h_records, "sdrb_bank_write_state");
     if (rc != SDRB_OK) return rc;
     if ((rc = check_state_headers(b, streams, n, (const unsigned char *)h_records, b->state_bytes, "sdrb_bank_write_state")) != SDRB_OK)
         return rc;
@@ -2048,12 +2216,30 @@ extern "C" int sdrb_spectrum_create(int device, int n_displays, int nfft, sdrb_s
         (rc = sp->smooth.alloc((size_t)n_displays * (FFT_N - 10) * sizeof(double))) || (rc = sp->stats.alloc((size_t)n_displays * 2 * sizeof(double)))) {
         sdrb_spectrum_destroy(sp); return rc;
     }
-    if (cudaFuncSetAttribute(k_spectrum_feed, cudaFuncAttributeMaxDynamicSharedMemorySize, FFT_N * (int)sizeof(float2)) != cudaSuccess) {
+    if (cudaFuncSetAttribute(k_spectrum_feed<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FFT_N * (int)sizeof(float2)) != cudaSuccess ||
+        cudaFuncSetAttribute(k_spectrum_feed<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FFT_N * (int)sizeof(float2)) != cudaSuccess) {
         set_error("sdrb_spectrum_create: cannot reserve 64 KB of shared memory"); sdrb_spectrum_destroy(sp); return SDRB_E_CUDA;
     }
     rc = sdrb_spectrum_reset(sp, -1);
     if (rc != SDRB_OK) { sdrb_spectrum_destroy(sp); return rc; }
     *out = sp;
+    return SDRB_OK;
+}
+
+// k_spectrum_feed for every display, or (map != nullptr) for the n displays a device list names
+static int spectrum_feed_launch(sdrb_spectrum *sp, const float *d_in, size_t in_stride, int len, float *d_fft_out, cudaStream_t st,
+                                const int *map, int n) {
+    FftTables T;
+    { const int trc = fft_tables(sp->device, &T); if (trc != SDRB_OK) return trc; }
+    if (map)
+        k_spectrum_feed<true><<<(unsigned)n, FFT_THREADS, FFT_N * sizeof(float2), st>>>(
+            (const float2 *)d_in, (long long)in_stride, len, (float2 *)sp->inr.p, (double *)sp->pwr.p, (double *)sp->smooth.p,
+            (double *)sp->stats.p, (float2 *)d_fft_out, T, map);
+    else
+        k_spectrum_feed<<<(unsigned)sp->n, FFT_THREADS, FFT_N * sizeof(float2), st>>>(
+            (const float2 *)d_in, (long long)in_stride, len, (float2 *)sp->inr.p, (double *)sp->pwr.p, (double *)sp->smooth.p,
+            (double *)sp->stats.p, (float2 *)d_fft_out, T);
+    CU_TRY(cudaGetLastError());
     return SDRB_OK;
 }
 
@@ -2063,13 +2249,7 @@ extern "C" int sdrb_spectrum_feed_device(sdrb_spectrum *sp, const float *d_in, s
         set_error("sdrb_spectrum_feed_device: bad argument"); return SDRB_E_INVALID;
     }
     CU_TRY(cudaSetDevice(sp->device));
-    FftTables T;
-    { const int trc = fft_tables(sp->device, &T); if (trc != SDRB_OK) return trc; }
-    k_spectrum_feed<<<(unsigned)sp->n, FFT_THREADS, FFT_N * sizeof(float2), (cudaStream_t)cuda_stream>>>(
-        (const float2 *)d_in, (long long)in_stride, len, (float2 *)sp->inr.p, (double *)sp->pwr.p, (double *)sp->smooth.p,
-        (double *)sp->stats.p, (float2 *)d_fft_out, T);
-    CU_TRY(cudaGetLastError());
-    return SDRB_OK;
+    return spectrum_feed_launch(sp, d_in, in_stride, len, d_fft_out, (cudaStream_t)cuda_stream, nullptr, 0);
 }
 
 // fftHandlerSlot for every receiver of a bank at once, straight from the bank's device buffers:
@@ -2090,12 +2270,13 @@ extern "C" int sdrb_bank_spectrum_feed(sdrb_bank *b, sdrb_spectrum *sp, int sour
         int rc = input_launch(b, cb, n, (float2 *)sp->scratch.p, st);
         if (rc != SDRB_OK) return rc;
         // a callback shorter than the FFT (none of the supported rates) would leave the tail stale, like the reference
-        return sdrb_spectrum_feed_device(sp, (const float *)sp->scratch.p, (size_t)n, n, d_fft_out, cuda_stream);
+        return spectrum_feed_launch(sp, (const float *)sp->scratch.p, (size_t)n, n, (float *)d_fft_out, st, b->last_map, b->last_n);
     }
     const SubVfo &s = b->plan->h.subs[(size_t)source];
     { const int zrc = ensure_sub_z(b, source, st); if (zrc != SDRB_OK) return zrc; }
     const float2 *z = (const float2 *)b->zbuf.p + b->sub_z_off[(size_t)source] + b->sub_z_hist[(size_t)source] + (size_t)cb * s.block_z;
-    return sdrb_spectrum_feed_device(sp, (const float *)z, b->z_stride, s.block_z, d_fft_out, cuda_stream);
+    // after a stream-list call the displays of its streams only: the others keep pwr, inr and stats
+    return spectrum_feed_launch(sp, (const float *)z, b->z_stride, s.block_z, (float *)d_fft_out, st, b->last_map, b->last_n);
 }
 
 extern "C" int sdrb_spectrum_feed_host(sdrb_spectrum *sp, const float *h_in, size_t in_stride, int len) {

@@ -46,6 +46,11 @@ constexpr int LATE_TILE = 256;
 constexpr int MAX_FIR_TAPS = 512;
 
 constexpr int DC_HALO_BLKS = RAW_TAIL / DC_BLK;     // table entries kept from the previous call
+
+// Bank stream of grid index i. MAP = false: streams s0 .. s0+n-1 of the bank (every full-bank and stream-group launch); MAP = true:
+// the stream-list calls, where map is the call's device copy of the caller's list and i a list position.
+template <bool MAP>
+__device__ __forceinline__ int map_stream(const int *__restrict__ map, int s0, int i) { return MAP ? __ldg(map + i) : s0 + i; }
 #define DC_A (1.0f - 0.000001f)         /* sdrj.cpp:281, evaluated in float like the reference */
 #define DC_C 0.000001f
 #define DC_MAGIC 12582912.0f            /* 1.5 * 2^23: (y + M) - M rounds y to nearest-even integer */
@@ -258,11 +263,12 @@ __device__ __forceinline__ float dc_incr(const DcAnchor &A, float x) {
     return __fadd_rn(__fadd_rn(y, DC_MAGIC), -DC_MAGIC);
 }
 
+template <bool MAP = false>
 __global__ void __launch_bounds__(128) k0_dc_anchor(const float2 *__restrict__ dc_state, DcAnchor *__restrict__ anchors,
-                                                     int n_streams, int stream0) {
+                                                     int n_streams, int stream0, const int *__restrict__ map = nullptr) {
     const int idx = blockIdx.x * 128 + threadIdx.x;
     if (idx >= 2 * n_streams) return;
-    const int stream = stream0 + (idx >> 1), arm = idx & 1;
+    const int stream = map_stream<MAP>(map, stream0, idx >> 1), arm = idx & 1;
     const float2 st = dc_state[stream];
     const float s0 = arm ? st.y : st.x;
     DcAnchor A;
@@ -318,19 +324,23 @@ __global__ void __launch_bounds__(128) k0_dc_anchor(const float2 *__restrict__ d
 // Q needs no tie handling: a half-way fl(c*x)/ulp, whose rounding in the real sum would depend on the state's parity, occurs
 // only for |state| < 2^-6, where the anchor is never ok (tests/test_dc_model.py::test_no_rounding_tie_is_reachable checks
 // every byte against every anchor a uint8 input can produce).
-__global__ void __launch_bounds__(256) k0_dc_qtab(const DcAnchor *__restrict__ anchors, int *__restrict__ qtab, int stream0) {
-    const int sa = 2 * stream0 + blockIdx.x;                       // (stream, arm)
+template <bool MAP = false>
+__global__ void __launch_bounds__(256) k0_dc_qtab(const DcAnchor *__restrict__ anchors, int *__restrict__ qtab, int stream0,
+                                                  const int *__restrict__ map = nullptr) {
+    const int sa = MAP ? 2 * map_stream<MAP>(map, 0, blockIdx.x >> 1) + (blockIdx.x & 1) : 2 * stream0 + blockIdx.x;   // (stream, arm)
     const DcAnchor A = anchors[sa];
     int d = 0;
     if (A.ok) d = (int)dc_incr(A, (float)((int)threadIdx.x - 127)) - A.r0;
     qtab[(size_t)sa * 256 + threadIdx.x] = d;
 }
 
+template <bool MAP = false>
 __global__ void __launch_bounds__(128) k0_dc_blocks(const uint8_t *__restrict__ iq, size_t iq_stride,
                                                      const DcAnchor *__restrict__ anchors, const int *__restrict__ qtab,
-                                                     DcStats *__restrict__ stats, int stats_stride, int blk0, int n_blk, int stream0) {
+                                                     DcStats *__restrict__ stats, int stats_stride, int blk0, int n_blk, int stream0,
+                                                     const int *__restrict__ map = nullptr) {
     __shared__ int sq[2][257];                                     // +1: the two arms start in different banks
-    const int stream = stream0 + blockIdx.y;
+    const int stream = map_stream<MAP>(map, stream0, blockIdx.y);
     for (int e = threadIdx.x; e < 512; e += 128) sq[e >> 8][e & 255] = qtab[(size_t)stream * 512 + e];
     __syncthreads();
     const int blk = blk0 + blockIdx.x * 128 + threadIdx.x;
@@ -500,14 +510,15 @@ __device__ __forceinline__ bool dc_solve_run(const unsigned char *raw, int arm, 
     return true;
 }
 
+template <bool MAP = false>
 __global__ void __launch_bounds__(64) k0_dc_walk(const uint8_t *__restrict__ iq, size_t iq_stride,
                                                   const DcStats *__restrict__ stats, int stats_stride,
                                                   const DcAnchor *__restrict__ anchors, const int *__restrict__ qtab,
                                                   float2 *__restrict__ dc_state,
                                                   uint2 *__restrict__ table, int table_stride, int blk0, int n_blk,
-                                                  int stream0) {
+                                                  int stream0, const int *__restrict__ map = nullptr) {
     extern __shared__ __align__(16) unsigned char dcw_smem[];
-    const int stream = stream0 + blockIdx.x;
+    const int stream = map_stream<MAP>(map, stream0, blockIdx.x);
     const int arm = threadIdx.x >> 5, lane = threadIdx.x & 31;
     uint4 *ring = reinterpret_cast<uint4 *>(dcw_smem) + (size_t)arm * DCW_RING * DCW_SLOT16;
     float *sq = reinterpret_cast<float *>(dcw_smem + (size_t)2 * DCW_RING * DCW_SLOT16 * 16) + arm * DC_BLK;
@@ -781,11 +792,13 @@ __global__ void __launch_bounds__(K1_THREADS, 2) k1_ingest_main(const K1Params p
 // (fir_decI/Q FIRUpdateAndProcess on the first sample of each group of `late`, FIRUpdate
 // on the others: vfo.cpp:346-384; newest sample excluded: dsp.cpp:59-71).
 // ------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(LATE_TILE) k2_late_fir(const LateDev *__restrict__ devs, int cb0, int ncb, int stream0) {
+template <bool MAP = false>
+__global__ void __launch_bounds__(LATE_TILE) k2_late_fir(const LateDev *__restrict__ devs, int cb0, int ncb, int stream0,
+                                                         const int *__restrict__ map = nullptr) {
     __shared__ float2 sz[LATE_TILE * 6 + MAX_FIR_TAPS];
     __shared__ float st[MAX_FIR_TAPS];
     const LateDev &D = devs[blockIdx.y];
-    const int stream = stream0 + blockIdx.x;
+    const int stream = map_stream<MAP>(map, stream0, blockIdx.x);
     const int n_total = (cb0 + ncb) * D.samples_out;               // outputs exist up to here
     const int m0 = cb0 * D.samples_out + blockIdx.z * LATE_TILE;
     if (m0 >= n_total) return;
@@ -817,6 +830,7 @@ __global__ void __launch_bounds__(LATE_TILE) k2_late_fir(const LateDev *__restri
 // K3: carry. Copies the trailing `hist` bytes of what this call produced to the front of
 // each buffer (main outputs, z, d) and keeps the last RAW_TAIL raw samples.
 // ------------------------------------------------------------------------------------
+template <bool MAP = false>
 __global__ void __launch_bounds__(128) k3_carry(const CarryItem *__restrict__ items, int n_items, int n_blocks,
                                                  const uint8_t *__restrict__ iq, size_t iq_stride, int block,
                                                  uint8_t *__restrict__ tail, long long *__restrict__ blocks_done,
@@ -824,8 +838,8 @@ __global__ void __launch_bounds__(128) k3_carry(const CarryItem *__restrict__ it
                                                  const DcAnchor *__restrict__ dc_anchor,
                                                  int dc_table_stride, int n_dcblk, int stream0,
                                                  const float2 *__restrict__ cf_in, size_t cf_stride,
-                                                 float2 *__restrict__ cf_tail) {
-    const int stream = stream0 + blockIdx.x;
+                                                 float2 *__restrict__ cf_tail, const int *__restrict__ map = nullptr) {
+    const int stream = map_stream<MAP>(map, stream0, blockIdx.x);
     const int item = blockIdx.y;
     if (item < n_items) {
         const CarryItem it = items[item];

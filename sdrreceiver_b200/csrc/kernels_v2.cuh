@@ -335,17 +335,18 @@ struct K2V2Params {
     long long in_stride, out_stride;
     int count, lut_len, block_in, HT, stream0, b0;
     int blk_off, pad;               // added to the callback counter: -n for a replay of the last call's callbacks after the carry
+    const int *map;                 // MAP instantiations: grid x indexes this list of bank streams
 };
 
 // RAGGED: callbacks that are not a whole number of 32-sample chunks (a 30 000- or 3 600-sample parent): loads stop at the end of
 // the callback, stores at the end of each VFO's callback (cascade_loop).
-template <int NT, bool RAGGED = false>
+template <int NT, bool RAGGED = false, bool MAP = false>
 __global__ void __launch_bounds__(NT, v2_minb<NT>()) k2a_v2(const __grid_constant__ K2V2Params p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2 *sm = reinterpret_cast<float2 *>(smem_raw);
     int *sBase = reinterpret_cast<int *>(sm + V2L<NT>::SEND);
 
-    const int stream = p.stream0 + blockIdx.x;
+    const int stream = map_stream<MAP>(p.map, p.stream0, blockIdx.x);
     const int tile = blockIdx.y, b = p.b0 + blockIdx.z;
     const int t = threadIdx.x;
     const int B = p.block_in, L = p.lut_len;
@@ -395,13 +396,15 @@ struct TailDev {
     int in_hist, out_hist, block_in, S, HT, tiles;   // HT halo threads per tile, tiles per callback
 };
 
-__global__ void __launch_bounds__(TAIL_NT) k_hb_tail(const TailDev *__restrict__ devs, int max_tiles, int stream0, int b0) {
+template <bool MAP = false>
+__global__ void __launch_bounds__(TAIL_NT) k_hb_tail(const TailDev *__restrict__ devs, int max_tiles, int stream0, int b0,
+                                                     const int *__restrict__ map = nullptr) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2 *sm = reinterpret_cast<float2 *>(smem_raw);
     const TailDev D = devs[blockIdx.y / max_tiles];
     const int tile = blockIdx.y % max_tiles;
     if (tile >= D.tiles) return;                              // uniform per CTA: a shorter channel of the launch
-    const int stream = stream0 + blockIdx.x, b = b0 + blockIdx.z;
+    const int stream = map_stream<MAP>(map, stream0, blockIdx.x), b = b0 + blockIdx.z;
     const int t = threadIdx.x;
     const int B = D.block_in, S = D.S;
     const int v0 = tile * ((TAIL_NT - D.HT) * V2_CHUNK) - D.HT * V2_CHUNK + t * V2_CHUNK;
@@ -492,6 +495,7 @@ struct K1V2Params {
     int dc_stride, block, lut_len, n_main, stream0, b0;
     CascVfo vfos[SDRB_MAX_MAIN];    // the main VFOs
     RfTab rf[SDRB_MAX_MAIN];
+    const int *map;                 // MAP instantiations: grid x indexes this list of bank streams
 };
 
 __device__ __forceinline__ float dc_decode(uint2 e, const DcAnchor &A) {
@@ -502,13 +506,16 @@ __device__ __forceinline__ float dc_decode(uint2 e, const DcAnchor &A) {
 // correct_dc_bias, DC-corrected input -- for the first n samples of one callback. It is what the
 // "Main" spectrum shows (sdrj.cpp:296-303). One thread per 128-sample DC block: it starts from the
 // block-start state of the walk (bit-exact) and repeats the reference's float steps (no FMA), so
-// the result is bit-identical to the reference. table == nullptr: conversion only.
+// the result is bit-identical to the reference. table == nullptr: conversion only. MAP: grid y indexes the streams of a
+// stream-list call; rows of out are bank streams either way.
+template <bool MAP = false>
 __global__ void __launch_bounds__(64) k_input_samples(const uint8_t *__restrict__ iq, size_t iq_stride, size_t first, int n,
                                                       const uint2 *__restrict__ table, const DcAnchor *__restrict__ anchor,
-                                                      int table_stride, int blk0, float2 *__restrict__ out) {
+                                                      int table_stride, int blk0, float2 *__restrict__ out,
+                                                      const int *__restrict__ map = nullptr) {
     const int j = blockIdx.x * 64 + threadIdx.x;                 // DC block inside the request
     if (j * DC_BLK >= n) return;
-    const int stream = blockIdx.y;
+    const int stream = map_stream<MAP>(map, 0, blockIdx.y);
     const uint8_t *src = iq + (size_t)stream * iq_stride + (first + (size_t)j * DC_BLK) * 2;
     float2 *dst = out + (size_t)stream * n + (size_t)j * DC_BLK;
     float sI = 0.f, sQ = 0.f;
@@ -554,13 +561,13 @@ template <int NT> constexpr size_t k1v2_smem_bulk() { return V2L<NT>::SMEM + 2 *
 constexpr int K1_PF_BYTES = 112;                          // per thread: 6 x 16 raw bytes + 2 x 8 table bytes
 template <int NT> constexpr size_t k1v2_smem() { return V2L<NT>::SMEM + (size_t)NT * K1_PF_BYTES; }
 
-template <bool DC, int NT, bool BULK = false>
+template <bool DC, int NT, bool BULK = false, bool MAP = false>
 __global__ void __launch_bounds__(NT, v2_minb<NT>()) k1_v2(const __grid_constant__ K1V2Params p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2 *sm = reinterpret_cast<float2 *>(smem_raw);
     int *sBase = reinterpret_cast<int *>(sm + V2L<NT>::SEND);
 
-    const int stream = p.stream0 + blockIdx.x;
+    const int stream = map_stream<MAP>(p.map, p.stream0, blockIdx.x);
     const int b = p.b0 + blockIdx.z;
     const int t = threadIdx.x;
     const int B = p.block, L = p.lut_len;
@@ -772,6 +779,7 @@ struct K2bV2Params {
     int eo_rows;                            // rows of each of E and O
     int np_max;                             // longest (padded) low-pass of the plan
     unsigned short tiles[SDRB_MAX_SUB];     // tiles per callback of each USB VFO: CTAs beyond it leave without touching memory
+    const int *map;                         // MAP: warp i of the grid runs bank stream map[i], stream0 is 0 and stream_end the list length
 };
 
 __device__ __forceinline__ constexpr int uv_off(int x) { return (x >> 4) * UV_ROW + (x & 15) * 2; }   // pair index -> float offset
@@ -820,6 +828,7 @@ __device__ __noinline__ void uv_store_ragged(const float *v, int k0, int tile_ou
 #ifndef UV_MINB
 #define UV_MINB 4
 #endif
+template <bool MAP = false>
 __global__ void __launch_bounds__(UV_WARPS * 32, UV_MINB) k2b_v2(const __grid_constant__ K2bV2Params p) {
     extern __shared__ __align__(16) float uv_smem[];
     if (blockIdx.z >= p.tiles[blockIdx.y]) return;          // grid.z is the longest VFO's tile count
@@ -830,8 +839,9 @@ __global__ void __launch_bounds__(UV_WARPS * 32, UV_MINB) k2b_v2(const __grid_co
     const int n_lo = p.cb0 * D.samples_out, n_total = (p.cb0 + p.ncb) * D.samples_out;
     const int n0 = n_lo + blockIdx.z * tile_out;
     if (n0 >= n_total) return;
-    const int stream = p.stream0 + blockIdx.x * UV_WARPS + warp;
-    const bool live = stream < p.stream_end;
+    const int li = p.stream0 + blockIdx.x * UV_WARPS + warp;   // the stream, or (MAP) its list position
+    const bool live = li < p.stream_end;
+    const int stream = MAP ? map_stream<MAP>(p.map, 0, live ? li : 0) : li;
     // ---- the tile's input, z-local q = 0..1152 (re rows: q - 66, im rows: q - 1): lane l owns q = 32 it + l.
     // All 37 loads of the lane are issued before the coefficient staging and the barrier, so the tile costs
     // one HBM/L2 latency, overlapped with the descriptor-dependent coefficient loads.
@@ -987,8 +997,9 @@ template <int L> constexpr size_t lv_smem() {
 #ifndef LV_MINB
 #define LV_MINB 4
 #endif
-template <int L, int AT>
-__global__ void __launch_bounds__(LV_THREADS, LV_MINB) k2_late_v2(const LateDev *__restrict__ devs, int cb0, int ncb, int stream0) {
+template <int L, int AT, bool MAP = false>
+__global__ void __launch_bounds__(LV_THREADS, LV_MINB) k2_late_v2(const LateDev *__restrict__ devs, int cb0, int ncb, int stream0,
+                                                                  const int *__restrict__ map = nullptr) {
     extern __shared__ __align__(16) unsigned char lv_raw[];
     constexpr int SEG = L * LV_R;                           // samples per thread segment
     float2 *sz = reinterpret_cast<float2 *>(lv_raw);
@@ -998,7 +1009,7 @@ __global__ void __launch_bounds__(LV_THREADS, LV_MINB) k2_late_v2(const LateDev 
     const int n_total = (cb0 + ncb) * D.samples_out;               // outputs exist up to here
     const int m0 = cb0 * D.samples_out + blockIdx.z * LV_TILE;
     if (m0 >= n_total) return;
-    const int stream = stream0 + blockIdx.x;
+    const int stream = map_stream<MAP>(map, stream0, blockIdx.x);
     const int t = threadIdx.x;
     const int N = D.ntaps;
     const int A = AT > 0 ? AT : (N + L - 1) / L;            // taps per phase (10 for 49/5, 13 for 73/6)

@@ -68,6 +68,9 @@ struct K3Params {
     const long long *blocks_done;
     long long in_stride, out_stride;
     int hist_in, count, lut_len, block_in, n_tiles, tiles_per_span, stream0, stream_end, b0, nsw;
+    // k2a_v3<MAXS, true>: warp-local stream s of stream group sg is bank stream map[sg * nsw + s]; stream0 is 0 and stream_end is
+    // the list length
+    const int *map;
 };
 
 // Host side: the folded taps and the rotation table of one VFO. w = angle of the float rotation the Oscillator
@@ -220,27 +223,37 @@ K3_HD void k3_prefetch_l1(const void *p) {
 #endif
 }
 
-// One warp's work: streams sbase .. sbase+nsw-1, tiles of span `span` of callback b.
+// One warp's work: streams sbase .. sbase+nsw-1 (MAP: list entries sg*nsw .. sg*nsw+nsw-1 of p.map), tiles of span `span` of
+// callback b.
 //   ring    32 rows of K3_ROW float2, private to the warp
 //   sdst    32 pointers, private to the warp
 //   srrel   the CTA's copy of p.rrel;  stab: slot table (v << 8 | 16-byte chunk), n_slots entries per stream
+//   sK      32 entries, private to the warp: 0..nsw-1 hold each stream's table index and start flag, and with MAP entries 16.. the
+//           bank index of each stream (every row offset below is then taken from stream 0, not from the warp's first stream)
 // The warp plays both roles in turn (role A, warp barrier, role B). The lanes load their windows from global memory, the lines
 // prefetched into L1 one tile ahead.
-template <int MAXS, class Env>
+template <int MAXS, bool MAP = false, class Env>
 K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 *ring, float2 **sdst, float2 *sF, int2 *sK,
                    const float2 *srrel, const unsigned short *stab, int n_slots) {
     const int lane = env.lane;
     const int nv = p.count, nsw = p.nsw, B = p.block_in, L = p.lut_len;
-    const int sbase = p.stream0 + sg * nsw;
+    const int sbase = MAP ? 0 : p.stream0 + sg * nsw;
+    const int lbase = MAP ? sg * nsw : sbase;              // list position of the warp's first stream, checked against stream_end
+    int *sS = reinterpret_cast<int *>(sK + 16);
+    auto srow = [&](int s) { return MAP ? sS[s] : s; };    // row of warp-local stream s, counted from stream sbase
     const int t_begin = span * p.tiles_per_span;
     const int t_end = (t_begin + p.tiles_per_span < p.n_tiles) ? t_begin + p.tiles_per_span : p.n_tiles;
     if (t_begin >= t_end) return;
 
     // ---- role B of this lane: row = lane = sB * nv + vB ----
     const int sB = lane / nv, vB = lane - sB * nv;
-    const bool rowB = sB < nsw && (sbase + sB) < p.stream_end;
+    const bool rowB = sB < nsw && (lbase + sB) < p.stream_end;
     const int SB = p.v[rowB ? vB : 0].S;
-    float2 *outB = p.v[rowB ? vB : 0].out + (size_t)(sbase + (rowB ? sB : 0)) * (size_t)p.out_stride + p.v[rowB ? vB : 0].hist +
+    if (MAP) {
+        if (lane < nsw) sS[lane] = lbase + lane < p.stream_end ? p.map[lbase + lane] : p.map[lbase];
+        env.sync();
+    }
+    float2 *outB = p.v[rowB ? vB : 0].out + (size_t)(sbase + srow(rowB ? sB : 0)) * (size_t)p.out_stride + p.v[rowB ? vB : 0].hist +
                    (size_t)b * (size_t)p.v[rowB ? vB : 0].block_out;
     K3Hist H;
 #pragma unroll
@@ -252,8 +265,8 @@ K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 
     // per stream of the warp: table index of callback coordinate 0 and "this callback starts the stream" (oscillator.cpp:26-30)
     if (lane < nsw) {
         int kb = 0, zero = 0;
-        if (sbase + lane < p.stream_end) {
-            const long long blk = k3_ldg(p.blocks_done + sbase + lane) + b;
+        if (lbase + lane < p.stream_end) {
+            const long long blk = k3_ldg(p.blocks_done + sbase + srow(lane)) + b;
             kb = (int)((blk * (long long)B) % L);
             zero = blk == 0;
         }
@@ -269,7 +282,7 @@ K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 
     int fpar = 0;
     const float2 *in0 = p.in + (size_t)sbase * (size_t)p.in_stride + p.hist_in + (long long)b * B;         // sample 0 of stream sbase
     int n_str = 0;
-    for (int s = 0; s < nsw && sbase + s < p.stream_end; ++s) n_str++;
+    for (int s = 0; s < nsw && lbase + s < p.stream_end; ++s) n_str++;
     const float2 *in_pf = in0 + K3_TILE - 16 + 16 * lane;                                                  // this lane's line of the next tile
     const float2 *in_ln = in0 + 4 * lane;                                                                  // this lane's chunk of a tile
     // Output copy, common case (at most 32 sixteen-byte chunks per stream and tile): this lane's chunk is the same for every
@@ -297,19 +310,23 @@ K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 
         // hoisted above the barrier, staged input -- none of them moves the kernel's time.
         if (t + 1 < t_end && lane < 10) {
             const float2 *pf = in_pf + c0;
-            for (int s = 0; s < n_str; ++s, pf += p.in_stride) k3_prefetch_l1(pf);
+            if (MAP) {
+                for (int s = 0; s < n_str; ++s) k3_prefetch_l1(pf + (size_t)sS[s] * (size_t)p.in_stride);
+            } else {
+                for (int s = 0; s < n_str; ++s, pf += p.in_stride) k3_prefetch_l1(pf);
+            }
         }
         // =============================== role A ===============================
         for (int s0 = 0; s0 < nsw; s0 += 2) {
-            const int strA = sbase + s0, strB = sbase + s0 + 1;
+            const int strA = lbase + s0, strB = lbase + s0 + 1;
             const bool hasA = strA < p.stream_end, hasB = (s0 + 1 < nsw) && strB < p.stream_end;
             const int2 baseA = sK[s0], baseB = sK[hasB ? s0 + 1 : s0];
             const int kaA = wrapL(baseA.x + c0), kaB = wrapL(baseB.x + c0);      // table index of sample c0
             const bool fastA = c0 != 0 && kaA >= K3_LUT_STEADY + 16 && kaA + K3_TILE + 8 <= L;
             const bool fastB = c0 != 0 && kaB >= K3_LUT_STEADY + 16 && kaB + K3_TILE + 8 <= L;
             // sample c0 + 4l of the two streams
-            const float2 *inA = in_ln + (size_t)s0 * (size_t)p.in_stride + c0;
-            const float2 *inB = in_ln + (size_t)(hasB ? s0 + 1 : s0) * (size_t)p.in_stride + c0;
+            const float2 *inA = in_ln + (size_t)srow(s0) * (size_t)p.in_stride + c0;
+            const float2 *inB = in_ln + (size_t)srow(hasB ? s0 + 1 : s0) * (size_t)p.in_stride + c0;
             if (env.all(fastA && fastB)) {              // a vote: the compiler then knows the branch (and the VFO loop in it) is warp-uniform
                 // ---- sums and differences, once for all VFOs ----
                 // x[i] = sample c0 + 4l - 10 + i; outputs m' = 0, 1 have centres i = 5, 7
@@ -492,9 +509,9 @@ K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 
                 env.sync();
                 if (lane < n_slots) {
                     const long long adv = ((long long)t * K3_OUT1) >> cp_shift;      // out1 index 64 t -> index of the VFO's own output
-                    for (int s = 0; s < nsw && sbase + s < p.stream_end; ++s) {
+                    for (int s = 0; s < nsw && lbase + s < p.stream_end; ++s) {
                         const float4 v = *reinterpret_cast<const float4 *>(ring + s * nv * K3_ROW + cp_src);
-                        k3_store_global16(cp_dst + (size_t)s * (size_t)p.out_stride + adv, v);
+                        k3_store_global16(cp_dst + (size_t)srow(s) * (size_t)p.out_stride + adv, v);
                     }
                 }
             } else {
@@ -507,7 +524,7 @@ K3_HD void k3_unit(Env &env, const K3Params &p, int sg, int span, int b, float2 
                 // 2-stage kernel's time (profiles/r02_experiments.md section 1). The stores are st.global: a generic store would keep the
                 // compiler from moving the next shared loads above it.
                 for (int s = 0; s < nsw; ++s) {
-                    if (sbase + s >= p.stream_end) break;
+                    if (lbase + s >= p.stream_end) break;
                     for (int slot0 = lane; slot0 < n_slots; slot0 += 128) {
                         int e[4];
                         float4 v[4];
@@ -541,10 +558,11 @@ struct K3DevEnv {
 constexpr int K3_WARPS = 2;                                 // default warps per CTA; the kernel works with any CTA size (independent warps that
                                                             // only share the read-only tables)
 
-// grid: x = ceil(stream groups / warps per CTA), y = spans, z = callbacks
+// grid: x = ceil(stream groups / warps per CTA), y = spans, z = callbacks. MAP: the stream groups are groups of consecutive entries
+// of p.map (stream-list calls)
 // Register cap: 168 for 2 and 3 stages (three warps per scheduler = 12 per SM). At 168 the 5-stage cascade spills a history array; at 200
 // it holds two warps per scheduler = 8 per SM (the register file is per scheduler: 16384 registers), without spills.
-template <int MAXS>
+template <int MAXS, bool MAP = false>
 __global__ void __maxnreg__(MAXS == 5 ? 200 : 168) k2a_v3(const __grid_constant__ K3Params p) {
     extern __shared__ __align__(16) unsigned char k3_smem[];
     float2 *srrel = reinterpret_cast<float2 *>(k3_smem);
@@ -566,9 +584,9 @@ __global__ void __maxnreg__(MAXS == 5 ? 200 : 168) k2a_v3(const __grid_constant_
     float2 *sF = reinterpret_cast<float2 *>(sdst + 32);
     int2 *sK = reinterpret_cast<int2 *>(sF + 64);
     const int sg = blockIdx.x * (int)(blockDim.x >> 5) + warp;
-    if (p.stream0 + sg * p.nsw >= p.stream_end) return;
+    if ((MAP ? 0 : p.stream0) + sg * p.nsw >= p.stream_end) return;
     K3DevEnv env{lane};
-    k3_unit<MAXS>(env, p, sg, (int)blockIdx.y, p.b0 + (int)blockIdx.z, ring, sdst, sF, sK, srrel, stab, n_slots);
+    k3_unit<MAXS, MAP>(env, p, sg, (int)blockIdx.y, p.b0 + (int)blockIdx.z, ring, sdst, sF, sK, srrel, stab, n_slots);
 }
 #endif
 

@@ -234,13 +234,16 @@ __global__ void __launch_bounds__(FFT_THREADS) prim_fft8192(const float2 *__rest
 //   X       = FFT(inr)                                         (kiss_fft, unscaled)
 //   pwr[b]  = pwr[b]*0.95 + 0.05*10*log10(max(1e5*|X[i]|/N, 1)),  b = (i + N/2) mod N
 //   smooth[i] = (pwr[i] + ... + pwr[i+4])/5, i < N-10;  stats = {max(pwr) (at least avg+10), avg(pwr)}
+// MAP: CTA i feeds display map[i] only (the streams of a stream-list call); the other displays are not touched.
+template <bool MAP = false>
 __global__ void __launch_bounds__(FFT_THREADS) k_spectrum_feed(const float2 *__restrict__ data, long long data_stride, int len,
                                                                float2 *__restrict__ inr, double *__restrict__ pwr,
                                                                double *__restrict__ smooth, double *__restrict__ stats,
-                                                               float2 *__restrict__ fft_out, FftTables T) {
+                                                               float2 *__restrict__ fft_out, FftTables T,
+                                                               const int *__restrict__ map = nullptr) {
     extern __shared__ float2 s[];
     __shared__ double red_max[FFT_THREADS / 32], red_sum[FFT_THREADS / 32];
-    const int d = blockIdx.x;
+    const int d = map_stream<MAP>(map, 0, blockIdx.x);
     const float2 *x = data + (size_t)d * data_stride;
     float2 *keep = inr + (size_t)d * FFT_N;
     double *P = pwr + (size_t)d * FFT_N;

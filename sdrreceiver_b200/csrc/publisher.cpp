@@ -12,6 +12,7 @@
 #include <cstdlib>
 #include <mutex>
 #include <string>
+#include <set>
 #include <thread>
 #include <vector>
 
@@ -167,6 +168,7 @@ struct sdrb_publisher_pool {
     // the job of the current generation
     const sdrb_plan *plan = nullptr;
     const int16_t *pcm = nullptr;
+    const int32_t *streams = nullptr;   // send_streams: record i belongs to receiver streams[i] (send_call: to receiver i)
     int n_streams = 0, n_blocks = 0;
     std::string error;
 };
@@ -189,20 +191,22 @@ std::string pool_address(const char *address, int k) {
 void pool_worker(sdrb_publisher_pool *pool, int k) {
     unsigned long long seen = 0;
     for (;;) {
-        const sdrb_plan *plan; const int16_t *pcm; int ns, nb;
+        const sdrb_plan *plan; const int16_t *pcm; const int32_t *list; int ns, nb;
         {
             std::unique_lock<std::mutex> lk(pool->mu);
             pool->cv_go.wait(lk, [&] { return pool->quit || pool->gen != seen; });
             if (pool->quit) return;
             seen = pool->gen;
-            plan = pool->plan; pcm = pool->pcm; ns = pool->n_streams; nb = pool->n_blocks;
+            plan = pool->plan; pcm = pool->pcm; list = pool->streams; ns = pool->n_streams; nb = pool->n_blocks;
         }
         int rc = SDRB_OK;
         const size_t rec = (size_t)plan->h.pcm_per_block;
         const int n = (int)pool->pubs.size();
-        for (int s = k; s < ns && rc == SDRB_OK; s += n)
+        for (int i = list ? 0 : k; i < ns && rc == SDRB_OK; i += list ? 1 : n) {
+            if (list && list[i] % n != k) continue;
             for (int cb = 0; cb < nb && rc == SDRB_OK; ++cb)
-                rc = sdrb_publisher_send_block(pool->pubs[(size_t)k], plan, pcm + ((size_t)s * nb + cb) * rec);
+                rc = sdrb_publisher_send_block(pool->pubs[(size_t)k], plan, pcm + ((size_t)i * nb + cb) * rec);
+        }
         {
             std::lock_guard<std::mutex> lk(pool->mu);
             if (rc != SDRB_OK) { pool->failed = rc; pool->error = sdrb_last_error(); }
@@ -240,11 +244,11 @@ extern "C" int sdrb_publisher_pool_address(const sdrb_publisher_pool *pool, int 
     return SDRB_OK;
 }
 
-extern "C" int sdrb_publisher_pool_send_call(sdrb_publisher_pool *pool, const sdrb_plan *plan, const int16_t *h_pcm, int n_streams, int n_blocks) {
-    if (!pool || !plan || (!h_pcm && n_streams > 0 && n_blocks > 0)) { sdrb::set_error("sdrb_publisher_pool_send_call: NULL argument"); return SDRB_E_INVALID; }
-    if (n_streams <= 0 || n_blocks <= 0) return SDRB_OK;
+// One job for every sender thread; returns when all of them are done.
+static int pool_run(sdrb_publisher_pool *pool, const sdrb_plan *plan, const int16_t *h_pcm, const int32_t *streams, int n_streams,
+                    int n_blocks) {
     std::unique_lock<std::mutex> lk(pool->mu);
-    pool->plan = plan; pool->pcm = h_pcm; pool->n_streams = n_streams; pool->n_blocks = n_blocks;
+    pool->plan = plan; pool->pcm = h_pcm; pool->streams = streams; pool->n_streams = n_streams; pool->n_blocks = n_blocks;
     pool->pending = (int)pool->workers.size();
     pool->failed = 0;
     ++pool->gen;
@@ -252,6 +256,28 @@ extern "C" int sdrb_publisher_pool_send_call(sdrb_publisher_pool *pool, const sd
     pool->cv_done.wait(lk, [&] { return pool->pending == 0; });
     if (pool->failed) { sdrb::set_error(pool->error); return pool->failed; }
     return SDRB_OK;
+}
+
+extern "C" int sdrb_publisher_pool_send_call(sdrb_publisher_pool *pool, const sdrb_plan *plan, const int16_t *h_pcm, int n_streams, int n_blocks) {
+    if (!pool || !plan || (!h_pcm && n_streams > 0 && n_blocks > 0)) { sdrb::set_error("sdrb_publisher_pool_send_call: NULL argument"); return SDRB_E_INVALID; }
+    if (n_streams <= 0 || n_blocks <= 0) return SDRB_OK;
+    return pool_run(pool, plan, h_pcm, nullptr, n_streams, n_blocks);
+}
+
+extern "C" int sdrb_publisher_pool_send_streams(sdrb_publisher_pool *pool, const sdrb_plan *plan, const int16_t *h_pcm,
+                                                const int32_t *streams, int n, int n_blocks) {
+    static const char *who = "sdrb_publisher_pool_send_streams";
+    if (!pool || !plan || !h_pcm || !streams) { sdrb::set_error(std::string(who) + ": NULL argument"); return SDRB_E_INVALID; }
+    if (n <= 0 || n_blocks <= 0) { sdrb::set_error(std::string(who) + ": n and n_blocks must be positive"); return SDRB_E_INVALID; }
+    std::set<int32_t> seen;
+    for (int k = 0; k < n; k++) {
+        const char *bad = streams[k] < 0 ? "is negative" : (!seen.insert(streams[k]).second ? "is listed twice" : nullptr);
+        if (bad) {
+            sdrb::set_error(std::string(who) + ": streams[" + std::to_string(k) + "] = " + std::to_string(streams[k]) + " " + bad);
+            return SDRB_E_INVALID;
+        }
+    }
+    return pool_run(pool, plan, h_pcm, streams, n, n_blocks);
 }
 
 extern "C" void sdrb_publisher_pool_close(sdrb_publisher_pool *pool) {
